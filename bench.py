@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Tacotron synthesis forward path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path -- embeddings -> encoder CBHG ->
 attention decoder loop -> post-net CBHG -> linear dense -- over one synthetic
@@ -37,6 +37,10 @@ Extra keys of the line (informational, none of them changes `value`):
 The forward and the vocoder replay CUDA graphs after their second identical call (taco_set_cuda_graphs).
 
 `--impl reference` times that CPU restatement alone (rank 0 only).
+`--dump-outputs DIR` writes, after the timed steps, what the last step returned for rank 0's first batch as DIR/<name>.npy
+(float32 / float64, 46 MB): mel_outputs and alignments whole, linear_outputs_sampled at the seeded frame indices
+linear_outputs_frames, and steps.  Inputs and weights are seeded, so two builds (or the two --impl arms, which run the
+same batch) can be compared output for output.
 N > 1: launched under torchrun, one rank per GPU, each rank runs its own batch
 of 32 utterances (weak scaling, no collective on the data path).
 """
@@ -60,6 +64,7 @@ if ROOT not in sys.path:
 METRIC = "mel_frames_per_s"
 UNIT = "frames/s"
 BATCH, T_IN, MAX_ITERS, R, ID_NUM = 32, 100, 200, 5, 60
+DUMP_LINEAR_FRAMES, DUMP_MAX_BYTES = 250, 64 * 10**6   # --dump-outputs: 46 MB at config 3
 
 
 def bind_to_gpu_numa_node(torch, local: int):
@@ -195,7 +200,26 @@ def cpu_restatement_seconds(n_threads: int, batch: int = BATCH):
     out = O.tacotron_forward(w, hp, ids, lengths, identities=spk, id_num=ID_NUM)
     dt = time.perf_counter() - t0
     frames = out["mel_outputs"].shape[0] * out["mel_outputs"].shape[1]
-    return dt, frames
+    return dt, frames, out
+
+
+def dump_arrays(mel, linear, alignments, steps):
+    """What a caller of the timed path receives from one step, as host float arrays (torch tensors on any device in):
+    mel [N, T, 80] and alignments [N, T_in, steps] whole, linear [N, T, 1025] (131 MB at config 3) at DUMP_LINEAR_FRAMES
+    frame indices drawn with a fixed seed (stored as linear_outputs_frames), and the decoder step count."""
+    frames = np.sort(np.random.default_rng(0).choice(linear.shape[1], min(DUMP_LINEAR_FRAMES, linear.shape[1]), replace=False))
+    arrays = {"mel_outputs": mel.cpu().numpy(), "alignments": alignments.cpu().numpy(),
+              "linear_outputs_sampled": linear.cpu().numpy()[:, frames], "linear_outputs_frames": frames.astype(np.float64),
+              "steps": np.float64(steps)}
+    arrays = {k: np.ascontiguousarray(v, np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    return arrays
+
+
+def write_dump(path: str, arrays) -> None:
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def run_reference(args):
@@ -206,9 +230,11 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     times, frames = [], 0
     for i in range(args.warmup + args.steps):
-        dt, frames = cpu_restatement_seconds(cores)
+        dt, frames, out = cpu_restatement_seconds(cores)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, dump_arrays(out["mel_outputs"], out["linear_outputs"], out["alignments"], out["steps"]))
     ms = 1e3 * float(np.mean(times))
     value = frames / (ms / 1e3)
     line = {
@@ -292,7 +318,8 @@ def run_ours(args):
                 l["stream"].wait_event(start)
                 st = 0
                 for _ in range(k):
-                    st = step(l)[3]
+                    l["last"] = step(l)
+                    st = l["last"][3]
                 ev = torch.cuda.Event(enable_timing=True)
                 ev.record()
                 ends.append(ev)
@@ -331,6 +358,8 @@ def run_ours(args):
     t_wall0 = time.time()
     ms_total, steps_taken = timed(dev_lanes, args.steps)
     launches = sum(l["eng"].launch_count() for l in lanes) - launches0
+    # lane 0 always takes part and recomputes its one batch every step; the legs below overwrite its output buffers
+    dump = dump_arrays(*lanes[0]["last"]) if args.dump_outputs and rank == 0 else None
     ms_per_step = ms_total / args.steps
     frames_per_step = BATCH * steps_taken * R * world
     value = frames_per_step / (ms_per_step / 1e3)
@@ -591,7 +620,7 @@ def run_ours(args):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu:
         cores = os.cpu_count() or 1
-        dt, frames = cpu_restatement_seconds(cores)
+        dt, frames, _ = cpu_restatement_seconds(cores)
         cpu = {"value": frames / dt, "unit": UNIT, "cores": cores, "kind": "port", "seconds": dt,
                "sample": "one full batch (32 utterances x 1000 frames), torch-CPU fp32 restatement of the reference "
                          "TF graph (TensorFlow 1.x cannot be installed here)"}
@@ -609,6 +638,8 @@ def run_ours(args):
         }
         line.update(extra)
         emit(line)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     for l in lanes:
         l["eng"].close()
     if dist is not None:
@@ -630,6 +661,8 @@ def main():
     ap.add_argument("--no-throughput-mode", action="store_true", help="skip the informational 4-cluster decoder legs")
     ap.add_argument("--no-configs", action="store_true", help="skip the legs for BASELINE configs 1, 2, 4, 5 and the synthesize-shaped e2e")
     ap.add_argument("--quick-configs", action="store_true", help="fewer runs in those legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last step returned (rank 0, first batch) as DIR/<name>.npy")
     args = ap.parse_args()
     # stdout carries exactly ONE JSON line.  Libraries write there too (NCCL prints its version banner on stdout when
     # NCCL_DEBUG is set): file descriptor 1 is pointed at stderr for the whole run and the line goes to the saved one.
