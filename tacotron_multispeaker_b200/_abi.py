@@ -24,6 +24,7 @@ BN_MOVING, BN_BATCH = 0, 1
 ACT_NONE, ACT_RELU, ACT_SIGMOID, ACT_TANH = 0, 1, 2, 3
 CBHG_ENCODER, CBHG_POST = 0, 1
 GEMM_FFMA, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
+EPI_PLAIN, EPI_HIGHWAY = 0, 1
 
 # Every symbol include/taco_b200.h declares (tests check the library exports all of them).
 SYMBOLS = [
@@ -35,6 +36,7 @@ SYMBOLS = [
     "taco_bigru", "taco_conv1d", "taco_maxpool_affine", "taco_bn_batch_stats",
     "taco_set_gemm_mode", "taco_launch_count", "taco_decoder_geometry", "taco_set_decoder_clusters", "taco_set_profiling", "taco_last_stage_ms", "taco_set_cuda_graphs",
     "taco_wav_length", "taco_griffin_lim",
+    "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit",
 ]
 
 
@@ -52,6 +54,31 @@ class TacoAudioParams(C.Structure):
         ("frame_length_ms", C.c_double), ("frame_shift_ms", C.c_double), ("preemphasis", C.c_double),
         ("min_level_db", C.c_double), ("ref_level_db", C.c_double), ("power", C.c_double),
     ]
+
+
+class TacoGemmDesc(C.Structure):
+    """``taco_gemm_desc``: one dense / conv GEMM with its epilogue (pointers as integers)."""
+    _fields_ = [
+        ("x", C.c_void_p), ("x_bs", C.c_int64), ("ldx", C.c_int32),
+        ("x_hi", C.c_void_p), ("x_lo", C.c_void_p),
+        ("N", C.c_int32), ("T", C.c_int32), ("Cin", C.c_int32), ("taps", C.c_int32), ("bank", C.c_int32),
+        ("Cout", C.c_int32),
+        ("w_host", C.c_void_p), ("w2_host", C.c_void_p), ("bias_host", C.c_void_p), ("bias2_host", C.c_void_p),
+        ("scale_host", C.c_void_p), ("shift_host", C.c_void_p),
+        ("res", C.c_void_p), ("res_bs", C.c_int64), ("ldres", C.c_int32),
+        ("act", C.c_int32), ("epi", C.c_int32),
+        ("out", C.c_void_p), ("out_bs", C.c_int64), ("ldo", C.c_int32), ("col_off", C.c_int32),
+        ("out_hi", C.c_void_p), ("out_lo", C.c_void_p), ("out_cp", C.c_int32),
+    ]
+
+
+class TacoGemmPlan(C.Structure):
+    """``taco_gemm_plan``: the launch shape of a tensor-core GEMM."""
+    _fields_ = [(n, C.c_int32) for n in ("valid", "tiles", "ctas", "persistent", "long_k", "stages", "epi_warps",
+                                         "acc_cols", "vec_epi", "variant", "smem_bytes")]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
 
 
 class TacoError(RuntimeError):
@@ -113,10 +140,20 @@ def load() -> C.CDLL:
     lib.taco_wav_length.argtypes = [C.POINTER(TacoAudioParams), i]
     lib.taco_wav_length.restype = i64
     lib.taco_griffin_lim.argtypes = [H, C.POINTER(TacoAudioParams), fp, i, i, i64, fp, vp]
+    lib.taco_umma_plan.argtypes = [C.POINTER(TacoGemmDesc), i, C.POINTER(TacoGemmPlan)]
+    lib.taco_gemm_unit.argtypes = [H, C.POINTER(TacoGemmDesc), C.POINTER(TacoGemmPlan), vp]
+    lib.taco_highway4_unit.argtypes = [H, fp, i64, i, vp, vp, vp, vp, fp, vp, vp, vp]
     for name in SYMBOLS:
         getattr(lib, name)  # AttributeError here = header and library out of sync
     _lib = lib
     return lib
+
+
+def umma_plan(desc: TacoGemmDesc, sms: int = 148) -> dict:
+    """``taco_umma_plan``: how the tensor-core kernel would run ``desc`` on ``sms`` SMs (host only, no device)."""
+    plan = TacoGemmPlan()
+    load().taco_umma_plan(C.byref(desc), int(sms), C.byref(plan))
+    return plan.as_dict()
 
 
 def check(lib, handle, rc: int) -> None:

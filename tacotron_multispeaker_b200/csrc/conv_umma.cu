@@ -25,6 +25,7 @@
 #include <cuda_bf16.h>
 
 #include <stdlib.h>
+#include <string.h>
 
 #include <mutex>
 #include <unordered_map>
@@ -531,7 +532,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
 // highwaynet x 4 on [rows, 128]: y = relu(x W_H + b_H) T + x (1 - T), T = sigmoid(x W_T + b_T), four times.  As four
 // conv_umma launches (+ four hi/lo split passes) the 16 MB activation made eight HBM / L2 round trips and every launch paid its
 // own pipeline fill (25.7 us each for 2.1 GF).  Here a CTA owns 128 rows for all layers: the activation lives in the epilogue
-// threads' REGISTERS (one row x 64 channels per thread, two threads per row), is re-written as bf16 hi / lo operand tiles in
+// threads' REGISTERS (one row x 32 channels per thread, four threads per row), is re-written as bf16 hi / lo operand tiles in
 // shared memory (128-byte swizzle, K-major: what TMA would have produced) for the next layer's tcgen05.mma, and only the weights
 // (128 KB per layer, hi + lo, L2 resident) stream in by TMA -- prefetched during the previous layer's epilogue.
 struct Hw4Args {
@@ -679,6 +680,10 @@ highway4_kernel(const __grid_constant__ CUtensorMap tmB, const Hw4Args p) {
             x[ch * 16 + i + 1] = fmaf(T1, H1 - x[ch * 16 + i + 1], x[ch * 16 + i + 1]);
           }
         }
+        // The half-1 MMAs read both A k-blocks too and are not covered by acc_full(0): the hf = 0 warps wait for their commit
+        // before overwriting k-block 0 (for the next layer, or the next tile at the top of the loop).  The gate math above has
+        // already overlapped them.
+        if (hf == 0) mbar_wait(acc_full(1), n & 1);
         if (l + 1 < p.layers) write_operands(x);                      // next layer's A operand (also releases the accumulator)
       }
       // results: fp32 rows (and, for the GEMM that follows, their bf16 hi / lo split)
@@ -855,9 +860,77 @@ bool get_map_b(CUtensorMap* m, const void* base, int Kld, int rows) {
 int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 }  // namespace
 
-cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st) {
+// Launch shapes (developer switches read once: TACO_UMMA_PERSISTENT = 0 / 1 forces, TACO_UMMA_EW, TACO_UMMA_STAGES_MAX, TACO_UMMA_CTAS):
+//  * long K (>= 24 k-blocks: the 3 x 1024 -> 256 projection, the conv banks): bound by loads and MMAs.  Persistent CTAs, one per
+//    SM, three 64 KB stages, two TMEM accumulators (the epilogue of tile i overlaps the main loop of tile i+1), 4 epilogue warps.
+//  * short K with more than two tiles per SM (the 1025-wide linear output, highway layers at full length): bound by the
+//    epilogue.  Persistent as well, but with EIGHT epilogue warps and two stages.
+//  * few tiles: one tile per CTA, eight epilogue warps, a shallow ring so that two CTAs share an SM.
+// Reads only the shape, the flags and whether each pointer is null or 16-byte aligned: no device access.
+taco_gemm_plan umma_plan(const ConvUmma& c, int sms) {
+  taco_gemm_plan q;
+  memset(&q, 0, sizeof(q));
+  if (c.N <= 0 || c.T <= 0 || c.Cp <= 0 || c.Cp % BK || c.Kld % BK || c.taps <= 0 || c.Cout <= 0 || sms <= 0) return q;
+  const int ny = (c.Cout + BN - 1) / BN;
+  const long long ntiles = (long long)c.N * ((c.T + BM - 1) / BM) * ny * (c.bank > 1 ? c.bank : 1);
+  if (ntiles > 0x7fffffffLL) return q;
+  q.tiles = (int)ntiles;
+  static const int force = env_int("TACO_UMMA_PERSISTENT", -1), ew_force = env_int("TACO_UMMA_EW", 0);
+  static const int stage_cap = env_int("TACO_UMMA_STAGES_MAX", 0), cta_cap = env_int("TACO_UMMA_CTAS", 0);
+  static const int stage_force = env_int("TACO_UMMA_STAGES", 0);
+  const int nkb_max = c.taps * (c.Cp / BK);
+  const bool long_k = nkb_max >= 24;
+  const bool persistent = force >= 0 ? force != 0 : (long_k || q.tiles > 2 * sms);
+  q.long_k = long_k; q.persistent = persistent;
+  q.epi_warps = ew_force == 4 || ew_force == 8 ? ew_force : (long_k ? 4 : 8);
+  if (persistent) q.stages = long_k ? MAX_STAGES : 2;
+  else q.stages = nkb_max >= 3 ? 2 : 1;
+  if (stage_force >= 1 && !long_k) q.stages = stage_force > MAX_STAGES ? MAX_STAGES : stage_force;
+  if (stage_cap >= 1 && q.stages > stage_cap) q.stages = stage_cap;
+  while (smem_bytes(q.stages, q.epi_warps) > 227u * 1024u && q.stages > 1) --q.stages;
+  int nctas = persistent ? (cta_cap > 0 ? cta_cap : sms) : q.tiles;
+  if (nctas > q.tiles) nctas = q.tiles;
+  q.ctas = nctas;
+  q.acc_cols = nctas < q.tiles ? 256 : 128;
+  const int chn = c.epi == EPI_HIGHWAY ? 2 : 1;
+  auto al4 = [](long long v) { return (v & 3) == 0; };
+  q.vec_epi = (al4(c.ldo) && al4(c.col_off) && al4(c.out_bs) && al4(c.Cout / chn) && (c.Cout % (4 * chn) == 0) &&
+               (c.out == nullptr || (reinterpret_cast<uintptr_t>(c.out) & 15) == 0) &&
+               (c.res == nullptr || (al4(c.ldres) && al4(c.res_bs) && (reinterpret_cast<uintptr_t>(c.res) & 15) == 0)) &&
+               (c.bias == nullptr || (reinterpret_cast<uintptr_t>(c.bias) & 15) == 0) &&
+               (c.scale == nullptr || ((reinterpret_cast<uintptr_t>(c.scale) & 15) == 0 && (reinterpret_cast<uintptr_t>(c.shift) & 15) == 0)))
+                  ? 1 : 0;
+  q.smem_bytes = (int)smem_bytes(q.stages, q.epi_warps);
+  // epilogue variant: the combinations the forward uses are compiled in, anything else takes the run-time variant 0
+  if (c.epi == EPI_HIGHWAY) q.variant = 5;
+  else if (c.act == 0 && !c.scale && !c.res) q.variant = 1;
+  else if (c.act == 1 && !c.scale && !c.res) q.variant = 2;
+  else if (c.act == 1 && c.scale && !c.res) q.variant = 3;
+  else if (c.act == 0 && c.scale && c.res) q.variant = 4;
+  // refusals
+  if (c.epi == EPI_HIGHWAY && (c.bias == nullptr || c.res == nullptr)) return q;
+  if (c.out_hi != nullptr && (c.out_lo == nullptr || !q.vec_epi || c.epi != EPI_PLAIN || c.bank > 1 || c.col_off != 0 || (c.out_cp & 63) ||
+                              c.out_cp < c.Cout || c.out_cp > ny * BN))
+    return q;
+  if (c.out == nullptr && c.out_hi == nullptr) return q;
+  if ((c.scale == nullptr) != (c.shift == nullptr)) return q;
+  q.valid = 1;
+  return q;
+}
+
+cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st, taco_gemm_plan* plan_out) {
   if (c.N <= 0 || c.T <= 0) return cudaSuccess;
-  if (c.Cp % BK || c.Kld % BK) return cudaErrorInvalidValue;
+  static int n_sm[64] = {0};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (n_sm[dev & 63] == 0) {
+    int v = 0;
+    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) v = 148;
+    n_sm[dev & 63] = v;
+  }
+  const taco_gemm_plan q = umma_plan(c, n_sm[dev & 63]);
+  if (plan_out) *plan_out = q;
+  if (!q.valid) return cudaErrorInvalidValue;
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
   const bool split = c.nsplit > 1;
   if (!get_map_a(&ma_hi, c.a_hi, c.Cp, c.T, c.N) || !get_map_b(&mb_hi, c.b_hi, c.Kld, c.b_rows) ||
@@ -870,62 +943,9 @@ cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st) {
   p.out_hi = c.out_hi; p.out_lo = c.out_lo; p.out_cp = c.out_cp;
   p.nx = c.N * ((c.T + BM - 1) / BM);
   p.ny = (c.Cout + BN - 1) / BN;
-  const long long ntiles = (long long)p.nx * p.ny * (c.bank > 1 ? c.bank : 1);
-  if (ntiles > 0x7fffffffLL) return cudaErrorInvalidValue;
-  p.ntiles = (int)ntiles;
-  static int n_sm[64] = {0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (n_sm[dev & 63] == 0) {
-    int v = 0;
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) v = 148;
-    n_sm[dev & 63] = v;
-  }
-  const int sms = n_sm[dev & 63];
-  // Launch shapes (developer switches read once: TACO_UMMA_PERSISTENT = 0 / 1 forces, TACO_UMMA_EW, TACO_UMMA_STAGES_MAX, TACO_UMMA_CTAS):
-  //  * long K (>= 24 k-blocks: the 3 x 1024 -> 256 projection, the conv banks): bound by loads and MMAs.  Persistent CTAs, one per
-  //    SM, three 64 KB stages, two TMEM accumulators (the epilogue of tile i overlaps the main loop of tile i+1), 4 epilogue warps.
-  //  * short K with more than two tiles per SM (the 1025-wide linear output, highway layers at full length): bound by the
-  //    epilogue.  Persistent as well, but with EIGHT epilogue warps and two stages.
-  //  * few tiles: one tile per CTA, eight epilogue warps, a shallow ring so that two CTAs share an SM.
-  static const int force = env_int("TACO_UMMA_PERSISTENT", -1), ew_force = env_int("TACO_UMMA_EW", 0);
-  static const int stage_cap = env_int("TACO_UMMA_STAGES_MAX", 0), cta_cap = env_int("TACO_UMMA_CTAS", 0);
-  const int nkb_max = c.taps * (c.Cp / BK);
-  const bool long_k = nkb_max >= 24;
-  const bool persistent = force >= 0 ? force != 0 : (long_k || p.ntiles > 2 * sms);
-  p.epi_warps = ew_force == 4 || ew_force == 8 ? ew_force : (long_k ? 4 : 8);
-  static const int stage_force = env_int("TACO_UMMA_STAGES", 0);
-  if (persistent) p.stages = long_k ? MAX_STAGES : 2;
-  else p.stages = nkb_max >= 3 ? 2 : 1;
-  if (stage_force >= 1 && !long_k) p.stages = stage_force > MAX_STAGES ? MAX_STAGES : stage_force;
-  if (stage_cap >= 1 && p.stages > stage_cap) p.stages = stage_cap;
-  while (smem_bytes(p.stages, p.epi_warps) > 227u * 1024u && p.stages > 1) --p.stages;
-  int nctas = persistent ? (cta_cap > 0 ? cta_cap : sms) : p.ntiles;
-  if (nctas > p.ntiles) nctas = p.ntiles;
-  p.acc_cols = nctas < p.ntiles ? 256 : 128;
-  dim3 grid(nctas, 1, 1);
-  const int chn = c.epi == EPI_HIGHWAY ? 2 : 1;
-  auto al4 = [](long long v) { return (v & 3) == 0; };
-  p.vec_epi = (al4(c.ldo) && al4(c.col_off) && al4(c.out_bs) && al4(c.Cout / chn) && (c.Cout % (4 * chn) == 0) &&
-               (c.out == nullptr || (reinterpret_cast<uintptr_t>(c.out) & 15) == 0) &&
-               (c.res == nullptr || (al4(c.ldres) && al4(c.res_bs) && (reinterpret_cast<uintptr_t>(c.res) & 15) == 0)) &&
-               (c.bias == nullptr || (reinterpret_cast<uintptr_t>(c.bias) & 15) == 0) &&
-               (c.scale == nullptr || ((reinterpret_cast<uintptr_t>(c.scale) & 15) == 0 && (reinterpret_cast<uintptr_t>(c.shift) & 15) == 0)))
-                  ? 1 : 0;
-  if (c.epi == EPI_HIGHWAY && (c.bias == nullptr || c.res == nullptr)) return cudaErrorInvalidValue;
-  if (c.out_hi != nullptr && (c.out_lo == nullptr || !p.vec_epi || c.epi != EPI_PLAIN || c.bank > 1 || c.col_off != 0 || (c.out_cp & 63) ||
-                              c.out_cp < c.Cout || c.out_cp > p.ny * BN))
-    return cudaErrorInvalidValue;
-  if (c.out == nullptr && c.out_hi == nullptr) return cudaErrorInvalidValue;
-  if ((c.scale == nullptr) != (c.shift == nullptr)) return cudaErrorInvalidValue;
-  const uint32_t smem = smem_bytes(p.stages, p.epi_warps);
-  // epilogue variant: the combinations the forward uses are compiled in, anything else takes the run-time variant 0
-  int ev = 0;
-  if (c.epi == EPI_HIGHWAY) ev = 5;
-  else if (c.act == 0 && !c.scale && !c.res) ev = 1;
-  else if (c.act == 1 && !c.scale && !c.res) ev = 2;
-  else if (c.act == 1 && c.scale && !c.res) ev = 3;
-  else if (c.act == 0 && c.scale && c.res) ev = 4;
+  p.ntiles = q.tiles;
+  p.epi_warps = q.epi_warps; p.stages = q.stages; p.acc_cols = q.acc_cols; p.vec_epi = q.vec_epi;
+  dim3 grid(q.ctas, 1, 1);
   using KernelFn = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const UmmaArgs);
   static const KernelFn kernels[2][6] = {
       {conv_umma_kernel<3, 0>, conv_umma_kernel<3, 1>, conv_umma_kernel<3, 2>, conv_umma_kernel<3, 3>, conv_umma_kernel<3, 4>, conv_umma_kernel<3, 5>},
@@ -941,7 +961,7 @@ cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st) {
     attr_set = true;
   }
   const int nthreads = 64 + 32 * p.epi_warps;
-  kernels[split ? 0 : 1][ev]<<<grid, nthreads, smem, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
+  kernels[split ? 0 : 1][q.variant]<<<grid, nthreads, (uint32_t)q.smem_bytes, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
   return cudaGetLastError();
 }
 

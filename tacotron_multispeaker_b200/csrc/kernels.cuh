@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/taco_b200.h"
 #include "decoder_cw.h"
 
 namespace taco {
@@ -52,7 +53,9 @@ struct ConvUmma {
   // channels Cout .. out_cp-1 written as zeros (out_cp % 64 == 0); plain epilogue, 16-byte aligned rows, no bank, col_off 0
   void* out_hi = nullptr; void* out_lo = nullptr; int out_cp = 0;
 };
-cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st);
+// The launch shape of a ConvUmma on `sms` SMs (include/taco_b200.h, taco_gemm_plan); valid == 0: the launch is refused.
+taco_gemm_plan umma_plan(const ConvUmma& c, int sms);
+cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st, taco_gemm_plan* plan_out = nullptr);
 // The highway layers of a CBHG (reference modules.py:63-64, 79-89) in one launch: x, out [rows][128] fp32 dense; w_hi = the layers'
 // W^T hi / lo matrices [layer][hi|lo][256][128] bf16 (contiguous, columns interleaved (H_c, T_c)); bias[l] = [256] interleaved.
 // out_hi / out_lo (nullable): bf16 hi / lo copy of the result for the GEMM that follows.

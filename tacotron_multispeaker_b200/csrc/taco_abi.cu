@@ -146,6 +146,11 @@ int fail(taco_handle* h, int code, const std::string& msg) {
   if (h) h->err = msg;
   return code;
 }
+// The GEMM operand split (split_bf16_kernel), the FFMA conv and the decoder read activations with 16-byte vector loads at
+// x + n*x_bs + t*ldx + c: the stage entry points refuse pointers and strides that would misalign them.
+bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+bool rows16(const void* p, int64_t x_bs, int64_t ldx) { return al16(p) && x_bs % 4 == 0 && ldx % 4 == 0; }
+
 #define CUDA_OK(h, expr)                                                                   \
   do {                                                                                     \
     cudaError_t _e = (expr);                                                               \
@@ -250,6 +255,34 @@ size_t put_vec(Arena& A, const float* src, int n) {
   return off;
 }
 
+// One highway layer (modules.py:79-89) as ONE GEMM: W_H, W_T [128][128] -> [128][256] with columns interleaved (H_c, T_c),
+// biases likewise [256] (the epilogues and highway4_kernel read the gate pair of channel c from columns 2c, 2c + 1).
+void put_highway(Arena& A, const float* wh, const float* bh, const float* wt, const float* bt, size_t& w_off, size_t& b_off) {
+  w_off = A.alloc(128 * 256);
+  b_off = A.alloc(256);
+  for (int r = 0; r < 128; ++r)
+    for (int c = 0; c < 128; ++c) {
+      A.buf[w_off + (size_t)r * 256 + 2 * c] = wh[(size_t)r * 128 + c];
+      A.buf[w_off + (size_t)r * 256 + 2 * c + 1] = wt[(size_t)r * 128 + c];
+    }
+  for (int c = 0; c < 128; ++c) {
+    A.buf[b_off + 2 * c] = bh[c];
+    A.buf[b_off + 2 * c + 1] = bt[c];
+  }
+}
+
+// W^T of a GEMM as bf16 hi / lo [b_rows][Kld] at hi (lo follows), from the fp32 weights at base + w_off[0] ([taps*Cin][ldw]);
+// a bank reads conv ci ([(ci+1)*Cin][ldw]) at base + w_off[ci] into rows ci*Cout ...
+void pack_gemmw(const GemmW& g, const float* base, const size_t* w_off, uint16_t* hi, cudaStream_t st) {
+  uint16_t* lo = hi + (size_t)g.b_rows * g.Kld;
+  if (g.bank > 1) {
+    for (int ci = 0; ci < g.bank; ++ci)
+      launch_pack_wt(base + w_off[ci], g.ldw, ci + 1, g.Cin, g.Cout, g.Cp, g.Kld, ci * g.Cout, hi, lo, st);
+  } else {
+    launch_pack_wt(base + w_off[0], g.ldw, g.taps, g.Cin, g.Cout, g.Cp, g.Kld, 0, hi, lo, st);
+  }
+}
+
 // conv1d() of the reference: kernel/bias + BN.  Emits weights, bias and the four
 // BN-derived vectors at given column offset of pre-allocated vectors.
 bool pack_bn(taco_handle* h, const std::string& scope, int C, float* scale, float* shift, float* gamma,
@@ -314,23 +347,13 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
     D.dense_w = put_matrix(A, w->data.data(), P2, 128, 128);
     D.dense_b = put_vec(A, b->data.data(), 128);
   }
-  for (int i = 0; i < 4; ++i) {   // highway: interleave columns (H_c, T_c)
+  for (int i = 0; i < 4; ++i) {
     const std::string hs = s + "/highway_" + std::to_string(i + 1);
     GETV(wh, hs + "/H/kernel", 128, 128);
     GETV(bh, hs + "/H/bias", 128);
     GETV(wt, hs + "/T/kernel", 128, 128);
     GETV(bt, hs + "/T/bias", 128);
-    D.hw_w[i] = A.alloc(128 * 256);
-    D.hw_b[i] = A.alloc(256);
-    for (int r = 0; r < 128; ++r)
-      for (int c = 0; c < 128; ++c) {
-        A.buf[D.hw_w[i] + (size_t)r * 256 + 2 * c] = wh->data[(size_t)r * 128 + c];
-        A.buf[D.hw_w[i] + (size_t)r * 256 + 2 * c + 1] = wt->data[(size_t)r * 128 + c];
-      }
-    for (int c = 0; c < 128; ++c) {
-      A.buf[D.hw_b[i] + 2 * c] = bh->data[c];
-      A.buf[D.hw_b[i] + 2 * c + 1] = bt->data[c];
-    }
+    put_highway(A, wh->data.data(), bh->data.data(), wt->data.data(), bt->data.data(), D.hw_w[i], D.hw_b[i]);
   }
   // BiGRU: gates/kernel [256,256] rows = [x(128); h(128)], candidate/kernel [256,128] likewise.
   D.gru_wx = A.alloc(128 * 768); D.gru_bx = A.alloc(768);
@@ -873,6 +896,20 @@ int do_postnet(taco_handle* h, Bump& ws, const float* mel, int N, int T, int bn_
   return check_launch(h, "postnet");
 }
 
+// The ConvUmma of a unit GEMM with its parameters at the given device pointers (the caller fills in the weight operand and,
+// unless d is presplit, the A operand).  For a bank, taps = bank: the heaviest conv and the width of the weight rows.
+ConvUmma unit_umma(const taco_gemm_desc& d, const float* bias, const float* scale, const float* shift) {
+  ConvUmma u;
+  const bool bank = d.bank > 1;
+  u.a_hi = d.x_hi; u.a_lo = d.x_lo; u.N = d.N; u.T = d.T; u.Cp = (d.Cin + 63) & ~63; u.Cin = d.Cin;
+  u.taps = bank ? d.bank : d.taps; u.bank = bank ? d.bank : 1; u.Cout = d.Cout; u.nsplit = 3;
+  u.b_hi = nullptr; u.b_lo = nullptr; u.b_rows = bank ? d.bank * d.Cout : d.Cout; u.Kld = u.taps * u.Cp;
+  u.bias = bias; u.scale = scale; u.shift = shift; u.res = d.res; u.res_bs = d.res_bs; u.ldres = d.ldres;
+  u.out = d.out; u.out_bs = d.out_bs; u.ldo = d.ldo; u.col_off = d.col_off; u.act = d.act; u.epi = d.epi;
+  u.out_hi = d.out_hi; u.out_lo = d.out_lo; u.out_cp = d.out_cp;
+  return u;
+}
+
 }  // namespace
 
 // =============================== C ABI ========================================
@@ -1045,15 +1082,8 @@ int taco_finalize_weights(taco_handle* h) {
     CUDA_OK(h, cudaMalloc(&h->dB, sizeof(uint16_t) * nb));
     CUDA_OK(h, cudaMemset(h->dB, 0, sizeof(uint16_t) * nb));
     for (GemmW* g : gs) {
-      uint16_t* hi = h->dB + g->bt;
-      uint16_t* lo = hi + (size_t)g->b_rows * g->Kld;
-      if (g->bank > 1) {
-        const CbhgDev& D = (g == &h->enc.g_bank) ? h->enc : h->post;
-        for (int ci = 0; ci < g->bank; ++ci)
-          launch_pack_wt(h->dW + D.bank_w[ci], 128, ci + 1, g->Cin, g->Cout, g->Cp, g->Kld, ci * g->Cout, hi, lo, 0);
-      } else {
-        launch_pack_wt(h->dW + g->w, g->ldw, g->taps, g->Cin, g->Cout, g->Cp, g->Kld, 0, hi, lo, 0);
-      }
+      const CbhgDev& D = (g == &h->enc.g_bank) ? h->enc : h->post;
+      pack_gemmw(*g, h->dW, g->bank > 1 ? D.bank_w.data() : &g->w, h->dB + g->bt, 0);
     }
     CUDA_OK(h, cudaDeviceSynchronize());
     const char* gm = getenv("TACO_GEMM");
@@ -1133,6 +1163,7 @@ int taco_decode(taco_handle* h, const float* memory, int N, int T_in, const floa
                 int teacher_force, float* dec_out, float* align_out, int32_t* steps_out_host, void* stream) {
   REQUIRE_READY(h);
   if (!memory || !dec_out || N <= 0 || T_in <= 0) return fail(h, TACO_ERR_INVALID, "bad argument");
+  if (!al16(memory)) return fail(h, TACO_ERR_INVALID, "memory must be 16-byte aligned");
   int rc = ensure_ws(h, sizeof(float) * (size_t)N * T_in * 512 + 65536);
   if (rc) return rc;
   Bump ws(h->ws, h->ws_bytes);
@@ -1146,6 +1177,8 @@ int taco_cbhg(taco_handle* h, int which, const float* x, const int32_t* lengths,
   if (!x || !out || N <= 0 || T <= 0) return fail(h, TACO_ERR_INVALID, "bad argument");
   const CbhgDev& D = which == TACO_CBHG_ENCODER ? h->enc : h->post;
   if (x_batch_stride == 0) x_batch_stride = (int64_t)T * D.Cin;
+  if (!rows16(x, x_batch_stride, D.Cin))
+    return fail(h, TACO_ERR_INVALID, "x must be 16-byte aligned, with a batch stride and a width that are multiples of 4 floats");
   int rc = ensure_ws(h, sizeof(float) * cbhg_ws_floats(D.K, D.P1, D.P2, (int64_t)N * T) + 65536);
   if (rc) return rc;
   Bump ws(h->ws, h->ws_bytes);
@@ -1160,6 +1193,8 @@ int taco_postnet(taco_handle* h, const float* mel, int N, int T, int bn_mode, in
   REQUIRE_READY(h);
   if (!mel || !linear_out || N <= 0 || T <= 0) return fail(h, TACO_ERR_INVALID, "bad argument");
   if (mel_batch_stride == 0) mel_batch_stride = (int64_t)T * h->hp.num_mels;
+  if (!rows16(mel, mel_batch_stride, h->hp.num_mels))
+    return fail(h, TACO_ERR_INVALID, "mel must be 16-byte aligned, with a batch stride and a width that are multiples of 4 floats");
   if (linear_batch_stride == 0) linear_batch_stride = (int64_t)T * h->hp.num_freq;
   int rc = ensure_ws(h, postnet_ws_bytes(h, N, T));
   if (rc) return rc;
@@ -1172,6 +1207,7 @@ int taco_bigru(taco_handle* h, int which, const float* x, const int32_t* lengths
                void* stream) {
   REQUIRE_READY(h);
   if (!x || !out || N <= 0 || T <= 0) return fail(h, TACO_ERR_INVALID, "bad argument");
+  if (!al16(x)) return fail(h, TACO_ERR_INVALID, "x must be 16-byte aligned");
   const CbhgDev& D = which == TACO_CBHG_ENCODER ? h->enc : h->post;
   int rc = ensure_ws(h, sizeof(float) * (size_t)N * T * 1024 + 65536);
   if (rc) return rc;
@@ -1192,6 +1228,7 @@ int taco_conv1d(taco_handle* h, const float* x, int N, int T, int Cin, const flo
   CUDA_OK(h, cudaSetDevice(h->device));
   if (!x || !kernel || !out || N <= 0 || T <= 0 || Cin <= 0 || Cin % 4 || k <= 0 || Cout <= 0)
     return fail(h, TACO_ERR_INVALID, "bad argument (Cin must be a multiple of 4)");
+  if (!al16(x) || !al16(kernel)) return fail(h, TACO_ERR_INVALID, "x and kernel must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   Ctx c{h, st};
   if (h->gemm_mode != 0) {   // tensor-core path: pack W^T hi/lo and split x on the device, then one UMMA launch
@@ -1233,7 +1270,6 @@ int taco_conv1d(taco_handle* h, const float* x, int N, int T, int Cin, const flo
   return check_launch(h, "conv1d");
 }
 
-// Post-net again on the true length after an early stop (the all-zero frame case): rare, synchronous.
 // ---- unit entry points for the two helper kernels of the CBHG that have no stage of their own --------------------------------
 int taco_maxpool_affine(taco_handle* h, const float* x, int N, int T, int C, const float* scale, const float* shift, float* out,
                         void* stream) {
@@ -1258,6 +1294,127 @@ int taco_bn_batch_stats(taco_handle* h, const float* x, int N, int T, int C, con
   return check_launch(h, "bn_batch_stats");
 }
 
+// ---- the GEMM and the fused highway kernel alone ------------------------------------------------------------------------------
+int taco_umma_plan(const taco_gemm_desc* d, int sms, taco_gemm_plan* plan) {
+  if (!plan) return TACO_ERR_INVALID;
+  memset(plan, 0, sizeof(*plan));
+  if (!d) return TACO_ERR_INVALID;
+  alignas(16) static const float param[4] = {0.f, 0.f, 0.f, 0.f};   // stands for the parameters the library stores aligned
+  *plan = umma_plan(unit_umma(*d, d->bias_host ? param : nullptr, d->scale_host ? param : nullptr, d->shift_host ? param : nullptr), sms);
+  return plan->valid ? TACO_OK : TACO_ERR_INVALID;
+}
+
+int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (plan) memset(plan, 0, sizeof(*plan));
+  if (!d || d->N <= 0 || d->T <= 0 || d->Cin <= 0 || d->Cout <= 0 || d->bank < 1 || (d->bank == 1 && d->taps < 1) || !d->w_host ||
+      (d->epi != TACO_EPI_PLAIN && d->epi != TACO_EPI_HIGHWAY) || ((d->scale_host == nullptr) != (d->shift_host == nullptr)))
+    return fail(h, TACO_ERR_INVALID, "bad argument");
+  const bool hw = d->epi == TACO_EPI_HIGHWAY, bank = d->bank > 1, presplit = d->x_hi != nullptr;
+  if (hw && (d->Cin != 128 || d->Cout != 256 || bank || d->taps != 1 || !d->w2_host || !d->bias_host || !d->bias2_host || !d->res ||
+             d->scale_host))
+    return fail(h, TACO_ERR_INVALID, "highway: 128 -> 256 interleaved (H, T) columns, one tap, W_T, b_H, b_T and the carry input");
+  if (presplit ? d->x_lo == nullptr : (d->x == nullptr || !rows16(d->x, d->x_bs, d->ldx)))
+    return fail(h, TACO_ERR_INVALID, "x: 16-byte aligned rows with strides that are multiples of 4 floats, or both halves of a split operand");
+  const int gm = h->gemm_mode;
+  if (gm == 0 && (presplit || d->out_hi != nullptr || d->out == nullptr))
+    return fail(h, TACO_ERR_INVALID, "gemm mode 0 (FFMA) reads and writes fp32 only");
+  const int taps = bank ? d->bank : d->taps, nparam = bank ? d->bank * d->Cout : d->Cout;
+  GemmW g = make_gemmw(0, hw ? 256 : (d->Cout + 3) & ~3, taps, d->Cin, d->Cout, d->bank);
+  // parameters: staged on the host as taco_finalize_weights stages them, then one copy to the device
+  Arena A;
+  std::vector<size_t> w_off(bank ? d->bank : 1);
+  size_t b_off = 0, sc_off = 0, sh_off = 0;
+  if (hw) {
+    put_highway(A, d->w_host, d->bias_host, d->w2_host, d->bias2_host, w_off[0], b_off);
+  } else if (bank) {
+    size_t src = 0;
+    for (int ci = 0; ci < d->bank; ++ci) {
+      w_off[ci] = put_matrix(A, d->w_host + src, (ci + 1) * d->Cin, d->Cout, g.ldw);
+      src += (size_t)(ci + 1) * d->Cin * d->Cout;
+    }
+  } else {
+    w_off[0] = put_matrix(A, d->w_host, taps * d->Cin, d->Cout, g.ldw);
+  }
+  if (!hw && d->bias_host) b_off = put_vec(A, d->bias_host, nparam);
+  if (d->scale_host) { sc_off = put_vec(A, d->scale_host, nparam); sh_off = put_vec(A, d->shift_host, nparam); }
+  const size_t nbt = gm ? (size_t)2 * g.b_rows * g.Kld : 0, na = gm && !presplit ? (size_t)2 * d->N * d->T * g.Cp : 0;
+  int rc = ensure_ws(h, sizeof(float) * A.buf.size() + sizeof(uint16_t) * (nbt + na) + 65536);
+  if (rc) return rc;
+  Bump ws(h->ws, h->ws_bytes);
+  float* dP = ws.take<float>(A.buf.size());
+  uint16_t* bt = ws.take<uint16_t>(nbt);
+  BfScratch sc;
+  if (na) sc = take_bf(ws, (int64_t)d->N * d->T, g.Cp);
+  if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (gemm unit)");
+  cudaStream_t st = (cudaStream_t)stream;
+  CUDA_OK(h, cudaMemcpyAsync(dP, A.buf.data(), sizeof(float) * A.buf.size(), cudaMemcpyHostToDevice, st));
+  const float* bias = d->bias_host ? dP + b_off : nullptr;
+  const float* scale = d->scale_host ? dP + sc_off : nullptr;
+  const float* shift = d->scale_host ? dP + sh_off : nullptr;
+  Ctx c{h, st};
+  if (gm == 0) {   // the fp32 FFMA kernel, one launch per conv as run_cbhg does for a bank
+    for (int ci = 0; ci < (bank ? d->bank : 1); ++ci) {
+      const int o = ci * d->Cout;
+      conv(c, d->x, d->x_bs, d->ldx, d->N, d->T, d->Cin, bank ? ci + 1 : taps, dP + w_off[ci], g.ldw, bias ? bias + o : nullptr,
+           scale ? scale + o : nullptr, shift ? shift + o : nullptr, d->res, d->res_bs, d->ldres, d->out, d->out_bs, d->ldo,
+           d->col_off + o, d->Cout, d->act, d->epi);
+    }
+    return check_launch(h, "gemm unit");
+  }
+  pack_gemmw(g, dP, w_off.data(), bt, st);
+  ConvUmma u = unit_umma(*d, bias, scale, shift);
+  if (!presplit) {
+    launch_split_bf16(d->x, d->x_bs, d->ldx, d->N, d->T, d->Cin, g.Cp, sc.hi, sc.lo, st);
+    u.a_hi = sc.hi; u.a_lo = sc.lo;
+  }
+  u.b_hi = bt; u.b_lo = bt + (size_t)g.b_rows * g.Kld; u.nsplit = gm == 2 ? 1 : 3;
+  taco_gemm_plan q;
+  cudaError_t e = launch_conv_umma(u, st, &q);
+  if (plan) *plan = q;
+  if (e != cudaSuccess)
+    return fail(h, q.valid ? TACO_ERR_CUDA : TACO_ERR_INVALID, std::string("conv_umma launch: ") + cudaGetErrorString(e));
+  h->launches += (bank ? d->bank : 1) + (presplit ? 1 : 2);
+  return check_launch(h, "gemm unit");
+}
+
+int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers, const float* w_h_host, const float* b_h_host,
+                       const float* w_t_host, const float* b_t_host, float* out, void* out_hi, void* out_lo, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (!x || rows <= 0 || rows > 0x7fffffffLL || layers < 1 || layers > 4 || !w_h_host || !b_h_host || !w_t_host || !b_t_host ||
+      (out == nullptr && out_hi == nullptr) || ((out_hi == nullptr) != (out_lo == nullptr)))
+    return fail(h, TACO_ERR_INVALID, "bad argument");
+  if (!al16(x) || !al16(out) || !al16(out_hi) || !al16(out_lo)) return fail(h, TACO_ERR_INVALID, "x and the outputs must be 16-byte aligned");
+  if (h->gemm_mode == 0) return fail(h, TACO_ERR_UNSUPPORTED, "the fused highway kernel runs on the tensor cores only (gemm mode 1 or 2)");
+  Arena A;
+  size_t w_off[4], b_off[4];
+  for (int l = 0; l < layers; ++l)
+    put_highway(A, w_h_host + (size_t)l * 128 * 128, b_h_host + (size_t)l * 128, w_t_host + (size_t)l * 128 * 128,
+                b_t_host + (size_t)l * 128, w_off[l], b_off[l]);
+  const GemmW g = make_gemmw(0, 256, 1, 128, 256);
+  const size_t per_layer = (size_t)2 * g.b_rows * g.Kld;   // [hi|lo][256][128]: the layout launch_highway4 reads, layer after layer
+  int rc = ensure_ws(h, sizeof(float) * A.buf.size() + sizeof(uint16_t) * per_layer * layers + 65536);
+  if (rc) return rc;
+  Bump ws(h->ws, h->ws_bytes);
+  float* dP = ws.take<float>(A.buf.size());
+  uint16_t* bt = ws.take<uint16_t>(per_layer * layers);
+  if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (highway4 unit)");
+  cudaStream_t st = (cudaStream_t)stream;
+  CUDA_OK(h, cudaMemcpyAsync(dP, A.buf.data(), sizeof(float) * A.buf.size(), cudaMemcpyHostToDevice, st));
+  const float* hb[4] = {nullptr, nullptr, nullptr, nullptr};
+  for (int l = 0; l < layers; ++l) {
+    pack_gemmw(g, dP, &w_off[l], bt + per_layer * l, st);
+    hb[l] = dP + b_off[l];
+  }
+  cudaError_t e = launch_highway4(x, out, out_hi, out_lo, bt, hb, layers, rows, h->gemm_mode == 2 ? 1 : 3, st);
+  if (e != cudaSuccess) return fail(h, TACO_ERR_CUDA, std::string("highway4 launch: ") + cudaGetErrorString(e));
+  h->launches += layers + 1;
+  return check_launch(h, "highway4 unit");
+}
+
+// Post-net again on the true length after an early stop (the all-zero frame case): rare, synchronous.
 static int redo_postnet(taco_handle* h, int N, int T_in, int max_steps, int steps, int bn_mode, const float* mel,
                         float* linear_out, cudaStream_t st) {
   const taco_hparams& hp = h->hp;

@@ -233,6 +233,49 @@ class Engine:
         self._ck(self.lib.taco_bn_batch_stats(self._h, _ptr(x), N, T, Cc, _ptr(gamma), _ptr(beta), _ptr(scale), _ptr(shift), self.stream))
         return scale, shift
 
+    def gemm_unit(self, N, T, Cin, Cout, w, *, x=None, x_bs=None, ldx=None, x_split=None, taps=1, bank=1, w2=None,
+                  bias=None, bias2=None, scale=None, shift=None, res=None, res_bs=None, ldres=None, act=_abi.ACT_NONE,
+                  epi=_abi.EPI_PLAIN, out=None, out_bs=None, ldo=None, col_off=0, out_split=None, out_cp=0):
+        """``taco_gemm_unit`` in the current gemm mode.  ``x`` / ``res`` / ``out`` are device tensors addressed through the
+        given strides (defaults: dense [N, T, C]); ``x_split`` / ``out_split`` are (hi, lo) bf16 operand tensors.  Weights
+        and per-channel parameters are host arrays in the reference layouts.  Returns the plan the launch used (a dict)."""
+        keep = []
+
+        def host(a):
+            if a is None:
+                return None
+            a = np.ascontiguousarray(a, dtype=np.float32)
+            keep.append(a)
+            return a.ctypes.data
+
+        def dev(t):
+            return None if t is None else t.data_ptr()
+
+        d = _abi.TacoGemmDesc()
+        d.x, d.x_bs, d.ldx = dev(x), T * Cin if x_bs is None else x_bs, Cin if ldx is None else ldx
+        d.x_hi, d.x_lo = (dev(x_split[0]), dev(x_split[1])) if x_split is not None else (None, None)
+        d.N, d.T, d.Cin, d.taps, d.bank, d.Cout = N, T, Cin, taps, bank, Cout
+        d.w_host, d.w2_host, d.bias_host, d.bias2_host = host(w), host(w2), host(bias), host(bias2)
+        d.scale_host, d.shift_host = host(scale), host(shift)
+        ch = Cout // 2 if epi == _abi.EPI_HIGHWAY else Cout
+        d.res, d.res_bs, d.ldres = dev(res), T * ch if res_bs is None else res_bs, ch if ldres is None else ldres
+        d.act, d.epi = act, epi
+        width = ch * max(bank, 1)
+        d.out, d.out_bs, d.ldo, d.col_off = dev(out), T * width if out_bs is None else out_bs, width if ldo is None else ldo, col_off
+        d.out_hi, d.out_lo = (dev(out_split[0]), dev(out_split[1])) if out_split is not None else (None, None)
+        d.out_cp = out_cp
+        plan = _abi.TacoGemmPlan()
+        self._ck(self.lib.taco_gemm_unit(self._h, C.byref(d), C.byref(plan), self.stream))
+        return plan.as_dict()
+
+    def highway4_unit(self, x, w_h, b_h, w_t, b_t, out=None, out_split=None):
+        """``taco_highway4_unit``: len(w_h) highway layers on x [rows, 128] (device) with host weights [layers, 128, 128] and
+        biases [layers, 128]; writes ``out`` [rows, 128] and / or the bf16 (hi, lo) copy ``out_split``."""
+        w_h, b_h, w_t, b_t = (np.ascontiguousarray(a, dtype=np.float32) for a in (w_h, b_h, w_t, b_t))
+        hi, lo = out_split if out_split is not None else (None, None)
+        self._ck(self.lib.taco_highway4_unit(self._h, _ptr(x), x.shape[0], w_h.shape[0], w_h.ctypes.data, b_h.ctypes.data,
+                                             w_t.ctypes.data, b_t.ctypes.data, _ptr(out), _ptr(hi), _ptr(lo), self.stream))
+
     # ---- vocoder (the step after the path) ----
     def audio_params(self, griffin_lim_iters: Optional[int] = None) -> "_abi.TacoAudioParams":
         hp = self.hp
