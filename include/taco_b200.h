@@ -260,6 +260,22 @@ int64_t taco_wav_length(const taco_audio_params* ap, int T);
 int taco_griffin_lim(taco_handle* h, const taco_audio_params* ap, const float* linear, int N, int T,
                      int64_t linear_batch_stride, float* wav_out, void* stream);
 
+/* ---- analysis: waveform -> normalised spectrogram targets ------------------ */
+/* Frames util/audio.py spectrogram / melspectrogram give an utterance of L samples: 1 + L / hop
+ * (librosa.stft with center=True).  < 0 on bad arguments.  No device needed. */
+int64_t taco_spectrogram_frames(const taco_audio_params* ap, int64_t L);
+/* util/audio.py spectrogram(y) and melspectrogram(y) for a batch, in the [T, F] layout the model consumes (the
+ * reference returns [F, T]): preemphasis (before padding) -> librosa 0.5.1 stft(n_fft 2048, hop, win, center=True,
+ * reflect padding, periodic Hann centred in the frame) -> |D| -> 20 log10(max(1e-5, .)) - ref_level_db -> _normalize,
+ * and the same on the mel filter bank librosa.filters.mel(sample_rate, 2048, num_mels) applied to |D|.
+ * wav [N, L] dense; lengths_host [N] (HOST, each in [1, L]) or NULL (all L).  linear_out [N, T_out, num_freq] and
+ * mel_out [N, T_out, num_mels], either may be NULL; rows t >= 1 + lengths[n] / hop are written as 0.0 (the targets'
+ * padding).  Needs no weights.  TACO_ERR_INVALID: a length outside [1, L], or T_out < the longest utterance's frames.
+ * TACO_ERR_UNSUPPORTED: num_freq != 1025, win > 2048, or N * T_out * 1025 >= 2^31.  Uses ap->preemphasis,
+ * min_level_db and ref_level_db; griffin_lim_iters and power are not read. */
+int taco_spectrogram(taco_handle* h, const taco_audio_params* ap, const float* wav, const int32_t* lengths_host, int N,
+                     int64_t L, int T_out, float* linear_out, float* mel_out, void* stream);
+
 /* ---- arithmetic mode of the dense layers ----------------------------------- */
 /* The reference computes in fp32.  0 = fp32 FFMA kernels; 1 (default) = tcgen05 tensor
  * cores with every operand split into bf16 hi+lo and three products per k-step

@@ -35,7 +35,7 @@ SYMBOLS = [
     "taco_embed", "taco_check_ids", "taco_encoder", "taco_decode", "taco_cbhg", "taco_postnet",
     "taco_bigru", "taco_conv1d", "taco_maxpool_affine", "taco_bn_batch_stats",
     "taco_set_gemm_mode", "taco_launch_count", "taco_decoder_geometry", "taco_set_decoder_clusters", "taco_set_profiling", "taco_last_stage_ms", "taco_set_cuda_graphs",
-    "taco_wav_length", "taco_griffin_lim",
+    "taco_wav_length", "taco_griffin_lim", "taco_spectrogram_frames", "taco_spectrogram",
     "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit",
 ]
 
@@ -140,6 +140,9 @@ def load() -> C.CDLL:
     lib.taco_wav_length.argtypes = [C.POINTER(TacoAudioParams), i]
     lib.taco_wav_length.restype = i64
     lib.taco_griffin_lim.argtypes = [H, C.POINTER(TacoAudioParams), fp, i, i, i64, fp, vp]
+    lib.taco_spectrogram_frames.argtypes = [C.POINTER(TacoAudioParams), i64]
+    lib.taco_spectrogram_frames.restype = i64
+    lib.taco_spectrogram.argtypes = [H, C.POINTER(TacoAudioParams), fp, C.c_void_p, i, i64, i, fp, fp, vp]
     lib.taco_umma_plan.argtypes = [C.POINTER(TacoGemmDesc), i, C.POINTER(TacoGemmPlan)]
     lib.taco_gemm_unit.argtypes = [H, C.POINTER(TacoGemmDesc), C.POINTER(TacoGemmPlan), vp]
     lib.taco_highway4_unit.argtypes = [H, fp, i64, i, vp, vp, vp, vp, fp, vp, vp, vp]

@@ -9,11 +9,17 @@
   it does NOT undo the pre-emphasis.
 * ``synthesize_wav(engine, linear)`` -- the same followed by
   ``inv_preemphasis`` (``:23-24``), fused into the same call on the device.
-* ``save_wav`` (``:14-16``), ``find_endpoint`` (``:55-63``),
+* ``spectrogram(engine, wav)`` / ``melspectrogram(engine, wav)`` -- the
+  analysis half (``preemphasis`` -> ``librosa.stft`` -> ``_amp_to_db`` ->
+  ``_normalize``, and ``_linear_to_mel`` with ``librosa.filters.mel``) as the
+  ``taco_spectrogram`` kernel.  They return ``[T, F]``, the layout the model
+  and the feeder consume (the reference returns ``[F, T]`` and its
+  preprocessing saves the transpose).
+* ``save_wav`` (``:14-16``), ``load_wav``, ``find_endpoint`` (``:55-63``),
   ``_stft_parameters`` (``:114-118``) are host code (numpy / ``wave``): they
   handle a finished waveform once per utterance.
 
-There is no CPU Griffin-Lim here: without the CUDA library these raise.
+There is no CPU Griffin-Lim or STFT here: without the CUDA library these raise.
 """
 from __future__ import annotations
 
@@ -38,6 +44,30 @@ def inv_spectrogram_tensorflow(engine, spectrogram, griffin_lim_iters=None):
 def synthesize_wav(engine, spectrogram, griffin_lim_iters=None):
     """``inv_preemphasis(inv_spectrogram_tensorflow(x))`` in one device call (synthesizer.py:47-50)."""
     return engine.griffin_lim(spectrogram, griffin_lim_iters, inv_preemphasis=True)
+
+
+def spectrogram(engine, wav):
+    """Normalised linear spectrogram ``[T, num_freq]`` of one waveform (``[N, T, num_freq]`` for a batch or a list of
+    waveforms), on the device."""
+    return engine.spectrogram(wav)[0]
+
+
+def melspectrogram(engine, wav):
+    """Normalised mel spectrogram ``[T, num_mels]`` of one waveform (``[N, T, num_mels]`` for a batch or a list of
+    waveforms), on the device."""
+    return engine.spectrogram(wav)[1]
+
+
+def load_wav(path, sample_rate):
+    """Mono 16-bit PCM WAV file -> float32 samples in [-1, 1) (divided by 32768).  The reference's
+    ``librosa.core.load(path, sr=sample_rate)`` also resamples and mixes down; that is not restated here, so any other
+    sample rate, channel count or sample width raises ``ValueError``."""
+    with wave.open(str(path), "rb") as f:
+        if f.getframerate() != int(sample_rate) or f.getnchannels() != 1 or f.getsampwidth() != 2:
+            raise ValueError("%s: need mono 16-bit PCM at %d Hz, got %d channel(s), %d-bit, %d Hz (no resampling here)"
+                             % (path, int(sample_rate), f.getnchannels(), 8 * f.getsampwidth(), f.getframerate()))
+        pcm = np.frombuffer(f.readframes(f.getnframes()), "<i2")
+    return pcm.astype(np.float32) / np.float32(32768.0)
 
 
 def wav_to_int16(wav) -> np.ndarray:

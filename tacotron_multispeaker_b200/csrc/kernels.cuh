@@ -154,4 +154,22 @@ struct GriffinLimArgs {
 size_t griffin_lim_ws_bytes(int N, int T, int win);
 cudaError_t launch_griffin_lim(const GriffinLimArgs& a, void* ws, cudaStream_t st, int* launches);
 
+// Spectrogram analysis (spectrogram.cu): util/audio.py spectrogram / melspectrogram (librosa 0.5.1 stft + filters.mel) on
+// the device.  tw / window: the twiddles (GL_N / 4 + 1 float2) and periodic Hann window that launch_fft_tables writes.
+// band: [num_mels][3] ints (first bin, bin count, offset into band_w) of the mel filter bank, band_w its fp32 weights.
+struct SpectrogramArgs {
+  const float* wav;      // [N][L]
+  long long L;
+  const int* lengths;    // [N] device, or null (all L)
+  int N, T_out, win, hop, num_mels;
+  float preemphasis;
+  double min_level_db, ref_level_db;
+  const float2* tw; const float* window;
+  const int* band; const float* band_w;
+  float* linear;         // [N][T_out][1025] or null
+  float* mel;            // [N][T_out][num_mels] or null
+};
+void launch_fft_tables(float2* tw, float* win, int win_len, cudaStream_t st);
+cudaError_t launch_spectrogram(const SpectrogramArgs& a, cudaStream_t st);
+
 }  // namespace taco

@@ -130,6 +130,13 @@ struct taco_handle {
   // the vocoder's ~105 launches per call likewise (key: arguments, workspace, stream)
   struct GlKey { GriffinLimArgs a; const void* ws; void* stream; };
   struct GlGraph { GlKey key; bool have_key = false; cudaGraphExec_t exec = nullptr; int launches = 0; } gl_graph;
+  // taco_spectrogram's tables (twiddles, analysis window, mel band table) in an allocation of their own, so that a workspace
+  // regrow does not drop them; rebuilt when (sample_rate, win) changes.  `host` is the source of the last upload.
+  struct SpecTables {
+    char* dev = nullptr; size_t bytes = 0;
+    int sample_rate = 0, win = 0;
+    std::vector<char> host;
+  } spec_tab;
   bool launch_failed = false;        // a kernel launcher returned an error (sticky until check_launch reports it)
   bool profiling = false;
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // [4],[5] bracket the decoder kernel
@@ -973,6 +980,7 @@ int taco_destroy(taco_handle* h) {
   if (h->ws) cudaFree(h->ws);
   if (h->stg) cudaFree(h->stg);
   if (h->d_ints) cudaFree(h->d_ints);
+  if (h->spec_tab.dev) cudaFree(h->spec_tab.dev);
   if (h->h_pinned) cudaFreeHost(h->h_pinned);
   for (int i = 0; i < 6; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->ev_compute) cudaEventDestroy(h->ev_compute);
@@ -1740,6 +1748,123 @@ int taco_griffin_lim(taco_handle* h, const taco_audio_params* ap, const float* l
   }
   h->launches += launches;
   return check_launch(h, "griffin_lim");
+}
+
+// librosa 0.5.1 filters.mel(sr, n_fft, n_mels) with fmin 0, fmax sr / 2, htk=False (the Slaney scale: linear below 1 kHz
+// at 200/3 Hz per mel, log step ln(6.4) / 27 above), in double: the triangle of band i over linspace(0, sr/2, n_fft/2 + 1)
+// is max(0, min((f - f_i) / (f_{i+1} - f_i), (f_{i+2} - f) / (f_{i+2} - f_{i+1}))) * 2 / (f_{i+2} - f_i).  Stored sparse:
+// band[3 i ..] = (first bin, bin count, offset into w) of the bins where the triangle is positive.
+static void mel_band_table(int sr, int n_fft, int num_mels, std::vector<int>& band, std::vector<float>& w) {
+  const double f_sp = 200.0 / 3.0, min_log_hz = 1000.0, min_log_mel = min_log_hz / f_sp, logstep = log(6.4) / 27.0;
+  auto hz_to_mel = [&](double f) { return f >= min_log_hz ? min_log_mel + log(f / min_log_hz) / logstep : f / f_sp; };
+  auto mel_to_hz = [&](double m) { return m >= min_log_mel ? min_log_hz * exp(logstep * (m - min_log_mel)) : f_sp * m; };
+  const int bins = n_fft / 2 + 1, npts = num_mels + 2;
+  const double f_max = sr / 2.0, mmax = hz_to_mel(f_max);
+  std::vector<double> mf(npts);
+  for (int i = 0; i < npts; ++i) mf[i] = mel_to_hz(i == npts - 1 ? mmax : i * (mmax / (npts - 1)));   // np.linspace
+  band.assign(3 * (size_t)num_mels, 0);
+  w.clear();
+  for (int i = 0; i < num_mels; ++i) {
+    const double enorm = 2.0 / (mf[i + 2] - mf[i]);
+    band[3 * i + 2] = (int)w.size();
+    for (int k = 0; k < bins; ++k) {
+      const double f = k == bins - 1 ? f_max : k * (f_max / (bins - 1));   // np.linspace(0, sr / 2, bins)
+      const double v = fmax(0.0, fmin((f - mf[i]) / (mf[i + 1] - mf[i]), (mf[i + 2] - f) / (mf[i + 2] - mf[i + 1])));
+      if (v > 0.0) {
+        if (band[3 * i + 1] == 0) band[3 * i] = k;
+        band[3 * i + 1] = k - band[3 * i] + 1;
+        w.resize(band[3 * i + 2] + band[3 * i + 1], 0.0f);
+        w.back() = (float)(v * enorm);
+      }
+    }
+  }
+}
+
+// byte offsets in h->spec_tab.dev: twiddles (513 float2) | window (up to 2048 floats) | band [num_mels][3] | band weights
+struct SpecLayout { size_t win, band, w; };
+static SpecLayout spec_layout(int num_mels) {
+  auto a256 = [](size_t x) { return (x + 255) & ~size_t(255); };
+  SpecLayout o;
+  o.win = a256(513 * sizeof(float2));
+  o.band = o.win + a256(2048 * sizeof(float));
+  o.w = o.band + a256(3 * (size_t)num_mels * sizeof(int));
+  return o;
+}
+
+// (re)builds h->spec_tab when the sample rate or the window length changes
+static int ensure_spec_tables(taco_handle* h, int sr, int win, cudaStream_t st) {
+  auto& S = h->spec_tab;
+  if (S.dev && S.sample_rate == sr && S.win == win) return TACO_OK;
+  std::vector<int> band;
+  std::vector<float> bw;
+  mel_band_table(sr, 2048, h->hp.num_mels, band, bw);
+  const SpecLayout o = spec_layout(h->hp.num_mels);
+  const size_t o_win = o.win, o_band = o.band, o_w = o.w, bytes = o_w + bw.size() * sizeof(float) + 256;
+  if (S.dev) cudaDeviceSynchronize();   // work on other streams may still read the old tables
+  if (bytes > S.bytes) {
+    if (S.dev) { cudaFree(S.dev); S.dev = nullptr; S.bytes = 0; }
+    CUDA_OK(h, cudaMalloc(&S.dev, bytes));
+    S.bytes = bytes;
+  }
+  S.sample_rate = 0;
+  S.host.assign(bytes - o_band, 0);
+  memcpy(S.host.data(), band.data(), band.size() * sizeof(int));
+  memcpy(S.host.data() + (o_w - o_band), bw.data(), bw.size() * sizeof(float));
+  CUDA_OK(h, cudaMemcpyAsync(S.dev + o_band, S.host.data(), S.host.size(), cudaMemcpyHostToDevice, st));
+  launch_fft_tables(reinterpret_cast<float2*>(S.dev), reinterpret_cast<float*>(S.dev + o_win), win, st);
+  h->launches += 1;
+  CUDA_OK(h, cudaPeekAtLastError());
+  S.sample_rate = sr;
+  S.win = win;
+  return TACO_OK;
+}
+
+int64_t taco_spectrogram_frames(const taco_audio_params* ap, int64_t L) {
+  int hop = 0, win = 0;
+  if (L < 1 || !audio_geometry(ap, &hop, &win)) return -1;
+  return 1 + L / hop;
+}
+
+int taco_spectrogram(taco_handle* h, const taco_audio_params* ap, const float* wav, const int32_t* lengths_host, int N,
+                     int64_t L, int T_out, float* linear_out, float* mel_out, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  int hop = 0, win = 0;
+  if (!wav || N <= 0 || L <= 0 || T_out <= 0 || !audio_geometry(ap, &hop, &win))
+    return fail(h, TACO_ERR_INVALID, "spectrogram: bad argument");
+  int64_t max_frames = 0;
+  for (int n = 0; n < N; ++n) {
+    const int64_t len = lengths_host ? lengths_host[n] : L;
+    if (len < 1 || len > L) return fail(h, TACO_ERR_INVALID, "spectrogram: a length outside [1, L]");
+    if (1 + len / hop > max_frames) max_frames = 1 + len / hop;
+  }
+  if (T_out < max_frames) return fail(h, TACO_ERR_INVALID, "spectrogram: T_out is shorter than the longest utterance's frames");
+  const int n_fft = (h->hp.num_freq - 1) * 2;
+  if (n_fft != 2048 || win > n_fft) return fail(h, TACO_ERR_UNSUPPORTED, "spectrogram: n_fft must be 2048 and win <= n_fft");
+  if ((int64_t)N * T_out * 1025 >= ((int64_t)1 << 31)) return fail(h, TACO_ERR_UNSUPPORTED, "spectrogram: too many frames for one call");
+  if (!linear_out && !mel_out) return TACO_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = ensure_spec_tables(h, ap->sample_rate, win, st);
+  if (rc) return rc;
+  int* d_len = nullptr;
+  if (lengths_host) {
+    rc = ensure_ws(h, sizeof(int32_t) * (size_t)N + 256);
+    if (rc) return rc;
+    d_len = reinterpret_cast<int*>(h->ws);
+    CUDA_OK(h, cudaMemcpyAsync(d_len, lengths_host, sizeof(int32_t) * (size_t)N, cudaMemcpyHostToDevice, st));
+  }
+  const char* base = h->spec_tab.dev;
+  const SpecLayout o = spec_layout(h->hp.num_mels);
+  SpectrogramArgs a;
+  a.wav = wav; a.L = L; a.lengths = d_len;
+  a.N = N; a.T_out = T_out; a.win = win; a.hop = hop; a.num_mels = h->hp.num_mels;
+  a.preemphasis = (float)ap->preemphasis; a.min_level_db = ap->min_level_db; a.ref_level_db = ap->ref_level_db;
+  a.tw = reinterpret_cast<const float2*>(base); a.window = reinterpret_cast<const float*>(base + o.win);
+  a.band = reinterpret_cast<const int*>(base + o.band); a.band_w = reinterpret_cast<const float*>(base + o.w);
+  a.linear = linear_out; a.mel = mel_out;
+  CUDA_OK(h, launch_spectrogram(a, st));
+  h->launches += 1;
+  return check_launch(h, "spectrogram");
 }
 
 int64_t taco_launch_count(const taco_handle* h) { return h ? h->launches : 0; }

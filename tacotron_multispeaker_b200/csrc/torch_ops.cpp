@@ -12,13 +12,17 @@
 //   taco_b200::decode(handle, memory, mel_targets?, teacher_force) -> (decoder_out [N,steps,M*r], alignments, steps)
 //   taco_b200::postnet(handle, mel, bn_mode) -> linear [N,T,F]
 //   taco_b200::griffin_lim(handle, linear, iters, sample_rate, frame_shift_ms, frame_length_ms, ...) -> wav [N,L]
+//   taco_b200::spectrogram(handle, wav, lengths?, T_out?, sample_rate, frame_shift_ms, frame_length_ms, ...)
+//       -> (linear [N,T_out,num_freq], mel [N,T_out,num_mels])
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
 #include <torch/types.h>
 
+#include <algorithm>
 #include <string>
 #include <tuple>
+#include <vector>
 
 #include "../../include/taco_b200.h"
 
@@ -157,6 +161,46 @@ at::Tensor griffin_lim(int64_t handle, const at::Tensor& linear, int64_t iters, 
   return wav;
 }
 
+// wav [N, L] on the device; lengths (host integers, each in [1, L]) or None = all L; T_out None = the longest utterance's frames
+std::tuple<at::Tensor, at::Tensor> spectrogram(int64_t handle, const at::Tensor& wav, at::OptionalIntArrayRef lengths,
+                                               c10::optional<int64_t> T_out, int64_t sample_rate, double frame_shift_ms,
+                                               double frame_length_ms, double min_level_db, double ref_level_db,
+                                               double preemphasis, int64_t num_mels, int64_t num_freq) {
+  taco_handle* h = H(handle);
+  dev_f32(wav, "wav");
+  TORCH_CHECK(wav.dim() == 2, "taco_b200::spectrogram: wav [N,L]");
+  c10::cuda::CUDAGuard guard(wav.device());
+  taco_audio_params ap{};
+  ap.sample_rate = (int32_t)sample_rate;
+  ap.frame_length_ms = frame_length_ms;
+  ap.frame_shift_ms = frame_shift_ms;
+  ap.preemphasis = preemphasis;
+  ap.min_level_db = min_level_db;
+  ap.ref_level_db = ref_level_db;
+  const int N = (int)wav.size(0);
+  const int64_t L = wav.size(1);
+  std::vector<int32_t> len;
+  int64_t T = 0;
+  if (lengths.has_value()) {
+    TORCH_CHECK((int64_t)lengths->size() == N, "taco_b200::spectrogram: lengths [N]");
+    for (int64_t v : *lengths) {
+      TORCH_CHECK(v >= 1 && v <= L, "taco_b200::spectrogram: lengths must be in [1, L]");
+      len.push_back((int32_t)v);
+      T = std::max<int64_t>(T, taco_spectrogram_frames(&ap, v));
+    }
+  } else {
+    T = taco_spectrogram_frames(&ap, L);
+  }
+  TORCH_CHECK(T > 0, "taco_b200::spectrogram: bad audio parameters");
+  if (T_out.has_value()) T = *T_out;
+  at::Tensor lin = at::empty({N, T, num_freq}, wav.options());
+  at::Tensor mel = at::empty({N, T, num_mels}, wav.options());
+  ck(h, taco_spectrogram(h, &ap, wav.data_ptr<float>(), lengths.has_value() ? len.data() : nullptr, N, L, (int)T,
+                         lin.data_ptr<float>(), mel.data_ptr<float>(), stream_of(wav)),
+     "spectrogram");
+  return std::make_tuple(lin, mel);
+}
+
 }  // namespace
 
 TORCH_LIBRARY(taco_b200, m) {
@@ -167,6 +211,8 @@ TORCH_LIBRARY(taco_b200, m) {
   m.def("postnet(int handle, Tensor mel, int bn_mode, int num_freq) -> Tensor");
   m.def("griffin_lim(int handle, Tensor linear, int iters, int sample_rate, float frame_shift_ms, float frame_length_ms, float min_level_db, "
         "float ref_level_db, float power, float preemphasis) -> Tensor");
+  m.def("spectrogram(int handle, Tensor wav, int[]? lengths, int? T_out, int sample_rate, float frame_shift_ms, float frame_length_ms, "
+        "float min_level_db, float ref_level_db, float preemphasis, int num_mels, int num_freq) -> (Tensor, Tensor)");
 }
 TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("forward", &forward);
@@ -174,4 +220,5 @@ TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("decode", &decode);
   m.impl("postnet", &postnet);
   m.impl("griffin_lim", &griffin_lim);
+  m.impl("spectrogram", &spectrogram);
 }

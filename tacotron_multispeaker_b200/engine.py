@@ -309,6 +309,54 @@ class Engine:
         self._ck(self.lib.taco_griffin_lim(self._h, C.byref(ap), _ptr(linear), N, T, 0, _ptr(wav), self.stream))
         return wav[0] if single else wav
 
+    def spectrogram_frames(self, num_samples: int) -> int:
+        """Frames the analysis gives ``num_samples`` samples: ``1 + num_samples // hop`` (``taco_spectrogram_frames``)."""
+        T = int(self.lib.taco_spectrogram_frames(C.byref(self.audio_params()), int(num_samples)))
+        if T < 0:
+            raise ValueError("bad audio hparams or length")
+        return T
+
+    def spectrogram(self, wav, lengths=None, T_out: Optional[int] = None):
+        """``audio.spectrogram`` and ``audio.melspectrogram`` of the reference (``taco_spectrogram``) for one waveform
+        ``[L]``, a batch ``[N, L]`` (with optional per-utterance ``lengths``) or a list of 1-D waveforms of different
+        lengths.  Returns ``(linear, mel)`` CUDA tensors ``[N, T_out, num_freq]`` / ``[N, T_out, num_mels]`` (``[T, F]``
+        for one 1-D waveform); ``T_out`` defaults to the longest utterance's frames, and rows past an utterance's own
+        frames are 0.0, the padding of the teacher-forcing targets."""
+        single = False
+        if isinstance(wav, (list, tuple)):
+            if lengths is not None:
+                raise ValueError("lengths are implied by a list of waveforms")
+            seqs = [np.asarray(w.detach().cpu() if isinstance(w, torch.Tensor) else w, dtype=np.float32) for w in wav]
+            if not seqs or any(s.ndim != 1 or s.size == 0 for s in seqs):
+                raise ValueError("expected a non-empty list of non-empty 1-D waveforms")
+            lengths = [s.size for s in seqs]
+            batch = np.zeros((len(seqs), max(lengths)), np.float32)
+            for i, s in enumerate(seqs):
+                batch[i, :s.size] = s
+            wav = batch
+        wav = self._f32(wav)
+        if wav.dim() == 1:
+            if lengths is not None:
+                raise ValueError("lengths need a batch [N, L]")
+            single, wav = True, wav[None]
+        if wav.dim() != 2 or wav.shape[1] == 0:
+            raise ValueError("wav must be [L] or [N, L] with L >= 1")
+        N, L = wav.shape
+        len_host = None
+        if lengths is not None:
+            len_host = np.ascontiguousarray(np.asarray(lengths).reshape(-1), dtype=np.int32)
+            if len_host.shape != (N,):
+                raise ValueError("lengths must be [N]")
+        longest = int(len_host.max()) if len_host is not None else L
+        T = self.spectrogram_frames(longest) if T_out is None else int(T_out)
+        hp = self.hp
+        lin = torch.empty(N, T, hp.num_freq, device=self.device, dtype=torch.float32)
+        mel = torch.empty(N, T, hp.num_mels, device=self.device, dtype=torch.float32)
+        self._ck(self.lib.taco_spectrogram(self._h, C.byref(self.audio_params()), _ptr(wav),
+                                           None if len_host is None else len_host.ctypes.data, N, L, T, _ptr(lin),
+                                           _ptr(mel), self.stream))
+        return (lin[0], mel[0]) if single else (lin, mel)
+
     # ---- whole path ----
     def forward(self, ids, lengths, spk=None, mel_targets=None, teacher_force=False,
                 bn_mode=_abi.BN_MOVING, want_linear=True, want_alignments=True, out=None):

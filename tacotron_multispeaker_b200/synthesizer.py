@@ -27,6 +27,7 @@ from typing import Optional
 import numpy as np
 
 from . import audio, plot
+from .engine import pad_targets
 from .hparams import HParams, hparams as default_hparams
 from .tacotron import create_model
 from .text import sequence_to_text2, text_to_sequence2
@@ -78,6 +79,28 @@ class Synthesizer:
         self.model.initialize(seq, lengths, identities=ident, id_num=self.id_num)
         wav = audio.synthesize_wav(self.model.engine, self.model.linear_outputs[0])
         return wav.cpu().numpy(), self.model.alignments[0].cpu().numpy()
+
+    def teacher_forced(self, text, identity, wav, path_align=None):
+        """Teacher-forced run on a text and its recording: the attention alignment of the two and the ground-truth-aligned
+        mel outputs.  ``wav`` is a path (``audio.load_wav``: mono 16-bit PCM at ``hparams.sample_rate``) or an array of
+        samples.  Its mel spectrogram (``audio.melspectrogram`` on the GPU), padded as the feeder pads targets
+        (``pad_targets``), feeds the decoder through ``initialize(..., teacher_force=True)``; batch norm keeps its
+        moving statistics.  As in the reference, the decoder stops after min(max_iters, T_targets / r) steps, and
+        ``load`` sets max_iters to 400, so a recording longer than 400 * r frames is cut there.  Returns
+        ``(mel_outputs [steps*r, num_mels], alignment [T_in, steps])`` as numpy arrays and writes the alignment image
+        to ``path_align`` when given."""
+        if isinstance(wav, (str, bytes)) or hasattr(wav, "__fspath__"):
+            wav = audio.load_wav(wav, self.hparams.sample_rate)
+        seq = np.asarray(text_to_sequence2(text, [x.strip() for x in self.hparams.cleaners.split(",")])[:-1], np.int32)
+        engine = self.model._get_engine(self.id_num if self.id_num > 1 else 0)
+        mel = audio.melspectrogram(engine, np.asarray(wav, dtype=np.float32).reshape(-1))
+        targets = pad_targets([mel.cpu().numpy()], self.hparams.outputs_per_step)
+        self.model.initialize(seq[None, :], np.asarray([seq.size], np.int32), mel_targets=targets,
+                              identities=np.asarray([identity], np.int32), id_num=self.id_num, teacher_force=True)
+        alignment = self.model.alignments[0].cpu().numpy()
+        if path_align is not None:
+            plot.plot_alignment(alignment, path_align)
+        return self.model.mel_outputs[0].cpu().numpy(), alignment
 
     def synthesize(self, text, identity, path=None, path_align=None):
         seq = text_to_sequence2(text, [x.strip() for x in self.hparams.cleaners.split(",")])[:-1]
