@@ -293,10 +293,21 @@ int64_t taco_launch_count(const taco_handle* h);
  * cluster used for batch N. */
 int taco_decoder_geometry(const taco_handle* h, int N, int* cluster_size, int* samples_per_cluster,
                           int* num_clusters);
-/* Decoder geometry: 0 (default) picks the number of 16-CTA clusters for the shortest decode (batch 32: 7 clusters of
- * 5/4 utterances, 112 SMs for 2.2 ms); n > 0 uses n clusters of up to 8 utterances each -- a throughput setting for
- * callers that keep several batches in flight (batch 32, n = 4: 64 SMs for 2.9 ms; +10 % mel frames/s with four batches
- * in flight, +16 % latency of a single one). */
+/* How the default decoder (16-CTA clusters, mma.sync) runs a batch of N utterances with T_in input positions on a device
+ * where max_clusters of its clusters are co-resident (7 on a B200).  No device needed. */
+typedef struct taco_decoder_plan_t {
+  int32_t valid;         /* 0: the decoder refuses the shape (T_in outside 1..512, N < 1) */
+  int32_t clusters;      /* as taco_set_decoder_clusters(h, 0) picks them */
+  int32_t s_max;         /* utterances in the largest cluster */
+  int32_t att_res;       /* where the attention operands (exp(2 key) rows, memory columns) live: 3 shared memory,
+                            4 tensor memory, 1 keys only / 2 memory only / 0 neither (re-read from global memory) */
+  int32_t ring_kb;       /* weight-ring depth per background warp (1 KB chunk-tiles; batches of <= 2 per cluster may
+                            deepen it at launch to hold a whole step) */
+  int32_t smem_bytes;    /* dynamic shared memory per CTA */
+} taco_decoder_plan_t;
+int taco_decoder_plan(int N, int T_in, int max_clusters, taco_decoder_plan_t* plan);
+/* Decoder geometry: 0 (default) picks the number of 16-CTA clusters (taco_decoder_plan; batch 32: 4 clusters of 8
+ * utterances on 64 SMs); n > 0 uses n clusters of up to 8 utterances each. */
 int taco_set_decoder_clusters(taco_handle* h, int n);
 /* Device time (ms, CUDA events on `stream`) of the stages of the last
  * taco_forward when profiling is on: [0]=encoder [1]=decoder stage (memory

@@ -36,7 +36,7 @@ SYMBOLS = [
     "taco_bigru", "taco_conv1d", "taco_maxpool_affine", "taco_bn_batch_stats",
     "taco_set_gemm_mode", "taco_launch_count", "taco_decoder_geometry", "taco_set_decoder_clusters", "taco_set_profiling", "taco_last_stage_ms", "taco_set_cuda_graphs",
     "taco_wav_length", "taco_griffin_lim", "taco_spectrogram_frames", "taco_spectrogram",
-    "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit",
+    "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit", "taco_decoder_plan",
 ]
 
 
@@ -76,6 +76,14 @@ class TacoGemmPlan(C.Structure):
     """``taco_gemm_plan``: the launch shape of a tensor-core GEMM."""
     _fields_ = [(n, C.c_int32) for n in ("valid", "tiles", "ctas", "persistent", "long_k", "stages", "epi_warps",
                                          "acc_cols", "vec_epi", "variant", "smem_bytes")]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
+class TacoDecoderPlan(C.Structure):
+    """``taco_decoder_plan_t``: how the default decoder runs a batch (clusters, residency of the attention operands)."""
+    _fields_ = [(n, C.c_int32) for n in ("valid", "clusters", "s_max", "att_res", "ring_kb", "smem_bytes")]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
@@ -146,6 +154,7 @@ def load() -> C.CDLL:
     lib.taco_umma_plan.argtypes = [C.POINTER(TacoGemmDesc), i, C.POINTER(TacoGemmPlan)]
     lib.taco_gemm_unit.argtypes = [H, C.POINTER(TacoGemmDesc), C.POINTER(TacoGemmPlan), vp]
     lib.taco_highway4_unit.argtypes = [H, fp, i64, i, vp, vp, vp, vp, fp, vp, vp, vp]
+    lib.taco_decoder_plan.argtypes = [i, i, i, C.POINTER(TacoDecoderPlan)]
     for name in SYMBOLS:
         getattr(lib, name)  # AttributeError here = header and library out of sync
     _lib = lib
@@ -156,6 +165,14 @@ def umma_plan(desc: TacoGemmDesc, sms: int = 148) -> dict:
     """``taco_umma_plan``: how the tensor-core kernel would run ``desc`` on ``sms`` SMs (host only, no device)."""
     plan = TacoGemmPlan()
     load().taco_umma_plan(C.byref(desc), int(sms), C.byref(plan))
+    return plan.as_dict()
+
+
+def decoder_plan(N: int, T_in: int, max_clusters: int = 7) -> dict:
+    """``taco_decoder_plan``: clusters, utterances per cluster and attention residency of the default decoder for a batch of
+    ``N`` utterances of ``T_in`` positions, ``max_clusters`` co-resident (7 on a B200).  Host only, no device."""
+    plan = TacoDecoderPlan()
+    load().taco_decoder_plan(int(N), int(T_in), int(max_clusters), C.byref(plan))
     return plan.as_dict()
 
 

@@ -153,7 +153,21 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint4& hi, const 
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                :: "r"(taddr), "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w), "r"(lo.x), "r"(lo.y), "r"(lo.z), "r"(lo.w) : "memory");
 }
+// attention operands in tensor memory (layout TL_ATT): four 32-bit words per lane
+__device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint4& v) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint4& v) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" :: "r"(taddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ float4 u2f(const uint4& v) {
+  return make_float4(__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w));
+}
+__device__ __forceinline__ uint4 f2u(const float4& v) {
+  return make_uint4(__float_as_uint(v.x), __float_as_uint(v.y), __float_as_uint(v.z), __float_as_uint(v.w));
+}
+__device__ __forceinline__ void reg_fence1(uint4& a) { asm volatile("" : "+r"(a.x), "+r"(a.y), "+r"(a.z), "+r"(a.w)); }
 __device__ __forceinline__ void reg_fence(uint4& a, uint4& b) {
   asm volatile("" : "+r"(a.x), "+r"(a.y), "+r"(a.z), "+r"(a.w), "+r"(b.x), "+r"(b.y), "+r"(b.z), "+r"(b.w));
 }
@@ -232,7 +246,7 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
   const int S = base + (cid < rem ? 1 : 0);
   const int n0 = cid * base + min(cid, rem);
   const int M = w.M, Dout = w.Dout, T_in = a.T_in;
-  const bool res_k = (a.att_res & 1) != 0, res_m = (a.att_res & 2) != 0;
+  const bool res_k = (a.att_res & 1) != 0, res_m = (a.att_res & 2) != 0, att_tm = (a.att_res & ATT_TMEM) != 0;
   const bool exact = w.exact_softmax != 0;
   const Dyn L = make_dyn(S, T_in, a.att_res, w.ring_kb);
   const uint32_t sbase = smem_u32(smem_raw);
@@ -290,14 +304,37 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
   const uint32_t tq = tmem_base + ((uint32_t)(gw * 32) << 16);                 // this warp's lane quarter, column 0
   {   // fill the quarter: the four warps of a quarter take every fourth chunk-tile
     const uint4* img = reinterpret_cast<const uint4*>(w.tmem_img) + ((size_t)(q * 4 + gw) * TMEM_TILES) * 64 + lane;
-    for (int i0 = (warp >> 2); i0 < TMEM_TILES; i0 += 16) {
+    const int tiles = att_tm ? TMEM_ATT_TILES : TMEM_TILES;
+    for (int i0 = (warp >> 2); i0 < tiles; i0 += 16) {
       uint4 hi[4], lo[4];
 #pragma unroll
       for (int k = 0; k < 4; ++k)
-        if (i0 + 4 * k < TMEM_TILES) { hi[k] = ldg_stream(img + (size_t)(i0 + 4 * k) * 64); lo[k] = ldg_stream(img + (size_t)(i0 + 4 * k) * 64 + 32); }
+        if (i0 + 4 * k < tiles) { hi[k] = ldg_stream(img + (size_t)(i0 + 4 * k) * 64); lo[k] = ldg_stream(img + (size_t)(i0 + 4 * k) * 64 + 32); }
 #pragma unroll
       for (int k = 0; k < 4; ++k)
-        if (i0 + 4 * k < TMEM_TILES) tmem_st8(tq + (uint32_t)(i0 + 4 * k) * 8u, hi[k], lo[k]);
+        if (i0 + 4 * k < tiles) tmem_st8(tq + (uint32_t)(i0 + 4 * k) * 8u, hi[k], lo[k]);
+    }
+    if (att_tm) {   // attention operands of this quarter (decoder_cw.h, TL_ATT), split over its four warps
+      const uint32_t tk = tq + (uint32_t)TMEM_ATT_COL0, tm = tk + (uint32_t)att_key_cols(S, T_in);
+      for (int m = warp >> 2; 8 * m + 2 * gw < npq; m += 4)   // pairs 8 m + 2 gw + e
+        for (int e = 0; e < 2; ++e) {
+          const int pp = 8 * m + 2 * gw + e;
+          if (pp >= npq) break;
+          const int p = p0 + pp, j = p / S, n = p - j * S;
+          const float* krow = a.keys + ((size_t)(n0 + n) * T_in + j) * DHID + 4 * lane;
+          float4 k0 = ldg_f4(krow), k1 = ldg_f4(krow + 128);
+          k0.x = __expf(2.0f * fminf(fmaxf(k0.x, -30.f), 30.f)); k0.y = __expf(2.0f * fminf(fmaxf(k0.y, -30.f), 30.f));
+          k0.z = __expf(2.0f * fminf(fmaxf(k0.z, -30.f), 30.f)); k0.w = __expf(2.0f * fminf(fmaxf(k0.w, -30.f), 30.f));
+          k1.x = __expf(2.0f * fminf(fmaxf(k1.x, -30.f), 30.f)); k1.y = __expf(2.0f * fminf(fmaxf(k1.y, -30.f), 30.f));
+          k1.z = __expf(2.0f * fminf(fmaxf(k1.z, -30.f), 30.f)); k1.w = __expf(2.0f * fminf(fmaxf(k1.w, -30.f), 30.f));
+          tmem_st8(tk + (uint32_t)(2 * m + e) * 8u, f2u(k0), f2u(k1));
+        }
+      for (int jq = warp >> 2; 4 * jq + gw < T_in; jq += 4) {   // positions j = 4 jq + gw
+        const int j = 4 * jq + gw;
+        float4 m4 = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (g < S) m4 = ldg_f4(a.memory + ((size_t)(n0 + g) * T_in + j) * DHID + q * 16 + 4 * t);
+        tmem_st4(tm + (uint32_t)jq * 4u, f2u(m4));
+      }
     }
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
   }
@@ -358,6 +395,10 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
       const float nab = fmaf(v.x, db, v.y * da), ncd = fmaf(v.z, dd, v.w * dc);
       return fmaf(nab, cd, ncd * ab) * rcp_approx(ab * cd);
     };
+    auto pair_q = [&](const float4& k0, const float4& k1, int n) -> float {
+      const float4 e0 = lds_f4(pq_l + (uint32_t)n * 64u), e1 = lds_f4(pq_l + (uint32_t)n * 64u + 8 * csb);
+      return quad(k0, e0, v0) + quad(k1, e1, v1);
+    };
     // keys first (their address does not depend on the sample index), then the query of the pair's sample
     auto pair_sum = [&](int pl, int n) -> float {
       float4 k0, k1;
@@ -373,15 +414,26 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
         k1.x = __expf(2.0f * fminf(fmaxf(k1.x, -30.f), 30.f)); k1.y = __expf(2.0f * fminf(fmaxf(k1.y, -30.f), 30.f));
         k1.z = __expf(2.0f * fminf(fmaxf(k1.z, -30.f), 30.f)); k1.w = __expf(2.0f * fminf(fmaxf(k1.w, -30.f), 30.f));
       }
-      const float4 e0 = lds_f4(pq_l + (uint32_t)n * 64u), e1 = lds_f4(pq_l + (uint32_t)n * 64u + 8 * csb);
-      return quad(k0, e0, v0) + quad(k1, e1, v1);
+      return pair_q(k0, k1, n);
     };
     const float vb = lds_f(sbase + OFF_VB);
     // the critical warps (12..15) own the first pairs: with few utterances per cluster nobody waits for a background warp here
     for (int pp = 2 * p6_wr; pp < npq; pp += pair_stride) {
       const bool two = pp + 1 < npq, first = pp == 2 * p6_wr;
       const int na = first ? p6_na : (int)smem_raw[L.pn + pp], nb = first ? p6_nb : (int)smem_raw[L.pn + (two ? pp + 1 : pp)];
-      const float sa = pair_sum(pp, na), sb = pair_sum(two ? pp + 1 : pp, nb);
+      float sa, sb;
+      if (att_tm) {   // pp is even and (pp >> 1) & 3 == gw: both rows sit in this warp's lane quarter, side by side
+        uint4 ka0, ka1, kb0, kb1;
+        const uint32_t kc = tq + (uint32_t)TMEM_ATT_COL0 + (uint32_t)(pp >> 3) * 16u;
+        tmem_ld8(kc, ka0, ka1);
+        tmem_ld8(kc + (two ? 8u : 0u), kb0, kb1);
+        tmem_wait_ld();
+        reg_fence(ka0, ka1); reg_fence(kb0, kb1);
+        sa = pair_q(u2f(ka0), u2f(ka1), na);
+        sb = pair_q(u2f(kb0), u2f(kb1), nb);
+      } else {
+        sa = pair_sum(pp, na); sb = pair_sum(two ? pp + 1 : pp, nb);
+      }
       const bool up = lane >= 16;
       float sv = (up ? sb : sa) + __shfl_xor_sync(0xffffffffu, up ? sa : sb, 16);
 #pragma unroll
@@ -409,7 +461,41 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
       mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
       if (warp == 12 && t == 0 && g < S) sts_f(sbase + OFF_MX + g * 4, mx);
     }
-    if (g < S) {
+    if (att_tm) {
+      // the resident loop below with the memory columns read from this warp's lane quarter: position j sits in quarter j & 3 =
+      // warp & 3.  tcgen05.ld takes the whole warp, so lanes of absent samples (g >= S) run along with zero weights.
+      const bool live = g < S;
+      uint32_t pa = sbase + L.sc + (uint32_t)(warp * S + min(g, S - 1)) * 4u;
+      const uint32_t dp = (uint32_t)NW * S * 4u;
+      const uint32_t tm = tq + (uint32_t)(TMEM_ATT_COL0 + att_key_cols(S, T_in)) + (uint32_t)(warp >> 2) * 4u;
+      for (int j = warp; j < T_in; j += 4 * NW) {
+        float pv[4];
+        uint4 mr[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const uint32_t o = j + i * NW < T_in ? (uint32_t)i : 0u;
+          pv[i] = lds_f(pa + o * dp);
+          tmem_ld4(tm + (uint32_t)(j >> 4) * 16u + o * 16u, mr[i]);
+        }
+        tmem_wait_ld();
+        float4 mv[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          reg_fence1(mr[i]);
+          mv[i] = u2f(mr[i]);
+          if (exact) pv[i] = __expf(pv[i] - mx);
+          if (j + i * NW >= T_in || !live) pv[i] = 0.f;
+        }
+        acc.x = fmaf(pv[0], mv[0].x, acc.x); acc.y = fmaf(pv[0], mv[0].y, acc.y); acc.z = fmaf(pv[0], mv[0].z, acc.z); acc.w = fmaf(pv[0], mv[0].w, acc.w);
+        acc2.x = fmaf(pv[1], mv[1].x, acc2.x); acc2.y = fmaf(pv[1], mv[1].y, acc2.y); acc2.z = fmaf(pv[1], mv[1].z, acc2.z); acc2.w = fmaf(pv[1], mv[1].w, acc2.w);
+        acc.x = fmaf(pv[2], mv[2].x, acc.x); acc.y = fmaf(pv[2], mv[2].y, acc.y); acc.z = fmaf(pv[2], mv[2].z, acc.z); acc.w = fmaf(pv[2], mv[2].w, acc.w);
+        acc2.x = fmaf(pv[3], mv[3].x, acc2.x); acc2.y = fmaf(pv[3], mv[3].y, acc2.y); acc2.z = fmaf(pv[3], mv[3].z, acc2.z); acc2.w = fmaf(pv[3], mv[3].w, acc2.w);
+        ssum += pv[0] + pv[2]; ssum2 += pv[1] + pv[3];
+        pa += 4 * dp;
+      }
+      acc.x += acc2.x; acc.y += acc2.y; acc.z += acc2.z; acc.w += acc2.w;
+      ssum += ssum2;
+    } else if (g < S) {
       uint32_t pa = sbase + L.sc + (uint32_t)(warp * S + g) * 4u;
       const uint32_t dp = (uint32_t)NW * S * 4u;
       if (res_m) {
@@ -921,6 +1007,26 @@ decoder_cw_kernel(const __grid_constant__ Args w, const __grid_constant__ Progra
 
 size_t decoder_cw_smem_bytes(int s_max, int T_in, int att_res, int ring_kb) { return make_dyn(s_max, T_in, att_res, ring_kb).total; }
 
+// Residency of the attention operands, in order of preference, each with the deepest weight ring (>= 4 KB per background warp:
+// an item takes up to four chunk-tiles at once) that fits 227 KB of shared memory:
+//   3 keys and memory in shared memory (weights fill tensor memory: TL_WIDE), the plan of every S <= 5 at T_in <= 100;
+//   ATT_TMEM keys and memory in tensor memory (TL_ATT: 26 background chunk-tiles per quarter move to the ring), if they fit its
+//     224 free columns: S = 8 up to T_in = 105;
+//   1 keys only, 2 memory only, 0 neither (P6 reloads keys from global memory and recomputes their exponentials, P7 walks the
+//     memory rows serially): long inputs.
+bool decoder_cw_plan(int s_max, int T_in, int* att_res, int* ring_kb, size_t* smem) {
+  static const int masks[5] = {3, ATT_TMEM, 1, 2, 0};
+  static const int rings[3] = {6, 5, 4};
+  for (int m = 0; m < 5; ++m) {
+    if (masks[m] == ATT_TMEM && att_tmem_cols(s_max, T_in) > TMEM_ATT_COLS) continue;
+    for (int k = 0; k < 3; ++k) {
+      const size_t b = decoder_cw_smem_bytes(s_max, T_in, masks[m], rings[k]);
+      if (b <= 227 * 1024) { *att_res = masks[m]; *ring_kb = rings[k]; *smem = b; return true; }
+    }
+  }
+  return false;
+}
+
 int decoder_cw_max_clusters() {
   auto kern = decoder_cw_kernel<false, false, false>;
   const int smem = 200 * 1024;
@@ -953,31 +1059,22 @@ cudaError_t launch_decoder_cw(const cw::Weights& wt, const DecoderArgs& a_in, in
   a.s_max = (a.N + nclusters - 1) / nclusters;
   if (a.s_max > 8 || (wt.M & 15) || (wt.Dout & 15) || wt.M > 128 || wt.Dout > 512) return cudaErrorInvalidValue;
   const int mode = a.targets != nullptr ? 1 : 0;
-  // shared memory: the attention operands resident if they fit, with the deepest weight ring that fits (>= 4 KB per background warp:
-  // an item takes up to four chunk-tiles at once)
-  static const int masks[4] = {3, 1, 2, 0};
-  static const int rings[3] = {6, 5, 4};
   int ring_kb = 0;
   size_t smem = 0;
-  bool ok = false;
-  for (int m = 0; m < 4 && !ok; ++m)
-    for (int k = 0; k < 3 && !ok; ++k) {
-      smem = decoder_cw_smem_bytes(a.s_max, a.T_in, masks[m], rings[k]);
-      if (smem <= 227 * 1024) { a.att_res = masks[m]; ring_kb = rings[k]; ok = true; }
-    }
-  if (!ok) return cudaErrorInvalidValue;
+  if (!decoder_cw_plan(a.s_max, a.T_in, &a.att_res, &ring_kb, &smem)) return cudaErrorInvalidValue;
+  const int lay = (a.att_res & ATT_TMEM) ? TL_ATT : TL_WIDE;
   if (a.s_max <= 2) {   // small batches: let the ring hold a whole lap if it fits (no refills at all)
     int longest = 0;
-    for (int i = 0; i < 12; ++i) longest = wt.ring_len[mode][i] > longest ? wt.ring_len[mode][i] : longest;
+    for (int i = 0; i < 12; ++i) longest = wt.ring_len[lay][mode][i] > longest ? wt.ring_len[lay][mode][i] : longest;
     if (longest <= 7 && decoder_cw_smem_bytes(a.s_max, a.T_in, a.att_res, longest) <= 227 * 1024) {
       ring_kb = longest;
       smem = decoder_cw_smem_bytes(a.s_max, a.T_in, a.att_res, ring_kb);
     }
   }
   Args k{};
-  k.tmem_img = wt.tmem_img;
-  k.ring = reinterpret_cast<const char*>(wt.ring) + (size_t)mode * 16 * 12 * wt.ring_stride * 1024;
-  for (int i = 0; i < 12; ++i) k.ring_len[i] = wt.ring_len[mode][i];
+  k.tmem_img = wt.tmem_img[lay];
+  k.ring = reinterpret_cast<const char*>(wt.ring[lay]) + (size_t)mode * 16 * 12 * wt.ring_stride * 1024;
+  for (int i = 0; i < 12; ++i) k.ring_len[i] = wt.ring_len[lay][mode][i];
   k.ring_stride = wt.ring_stride;
   k.bias = wt.bias;
   k.att_v = wt.att_v;
@@ -1002,7 +1099,7 @@ cudaError_t launch_decoder_cw(const cw::Weights& wt, const DecoderArgs& a_in, in
   attr[0].val.clusterDim.x = CS; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kern, k, wt.prog[mode], a, nclusters);
+  return cudaLaunchKernelEx(&cfg, kern, k, wt.prog[lay][mode], a, nclusters);
 }
 
 }  // namespace taco

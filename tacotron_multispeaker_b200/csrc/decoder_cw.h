@@ -69,6 +69,22 @@ constexpr int CP_TOTAL = 34;      // sum of CP_N: chunk-tiles 0..33 of the quart
 constexpr int TMEM_BG0 = CP_TOTAL;   // background chunk-tiles start here (30 per lane quarter)
 constexpr int TMEM_TILES = 64;    // chunk-tiles per lane quarter (512 columns / 8)
 
+// ---- tensor-memory layouts -------------------------------------------------------------------------------------------
+// TL_WIDE: all 64 chunk-tiles of a lane quarter are weights.  TL_ATT: only the first TMEM_ATT_TILES are (the critical tiles and
+// two background tiles; every other background tile streams through the ring), and columns TMEM_ATT_COL0..511 hold this CTA's
+// attention operands, so that eight utterances per cluster keep them on chip (shared memory has room for neither).  In lane
+// quarter gq (the quarter the P6 / P7 warps w with w & 3 == gq can read):
+//   * exp(2 key) row of pair pp, (pp >> 1) & 3 == gq, at column TMEM_ATT_COL0 + 8 (2 (pp >> 3) + (pp & 1)); lane l holds
+//     elements 4l..4l+3 and 128+4l..128+4l+3 (the registers pair_sum works on);
+//   * memory columns of position j, j & 3 == gq, at column TMEM_ATT_COL0 + att_key_cols + 4 (j >> 2); lane 4 n + t holds
+//     memory[n][j][16 q + 4 t .. + 3] (zero for n >= S).
+enum { TL_WIDE = 0, TL_ATT = 1 };
+constexpr int TMEM_ATT_TILES = 36;
+constexpr int TMEM_ATT_COL0 = TMEM_ATT_TILES * 8, TMEM_ATT_COLS = 512 - TMEM_ATT_COL0;
+constexpr int ATT_TMEM = 4;       // att_res bit: attention operands in tensor memory (layout TL_ATT)
+__host__ __device__ constexpr int att_key_cols(int S, int T_in) { return 16 * (((T_in * S) / CS + 4 + 7) / 8); }
+__host__ __device__ constexpr int att_tmem_cols(int S, int T_in) { return att_key_cols(S, T_in) + 4 * ((T_in + 3) / 4); }
+
 // ---- bias table per CTA (floats) ----------------------------------------------------------------------------------
 enum { BI_P1 = 0, BI_P1S0 = 16 /* step 0 of a free run: the go frame is zero, not W_o y + b_o */, BI_P2 = 32, BI_RA = 48, BI_UA = 64,
        BI_CA = 80, BI_Y0 = 96, BI_R1 = 112, BI_U1 = 128, BI_C1 = 144, BI_R2 = 160, BI_U2 = 176, BI_C2 = 192, BI_OA = 208,
@@ -76,14 +92,14 @@ enum { BI_P1 = 0, BI_P1S0 = 16 /* step 0 of a free run: the go frame is zero, no
 
 struct Weights {
   int M, Dout;
-  const void* tmem_img;    // [16 CTAs][4 quarters][64 chunk-tiles][2][32 lanes] uint4 (free run), then the same for teacher forcing
-  const void* ring;        // [2 modes][16 CTAs][12 background warps][ring_len] chunk-tiles of 1 KB, consumption order
-  int ring_len[2][12];     // chunk-tiles per step of each background warp (by mode)
+  const void* tmem_img[2]; // by layout: [16 CTAs][4 quarters][64 chunk-tiles][2][32 lanes] uint4 (TL_ATT: tiles >= 36 unused)
+  const void* ring[2];     // by layout: [2 modes][16 CTAs][12 background warps][ring_stride] chunk-tiles of 1 KB, consumption order
+  int ring_len[2][2][12];  // chunk-tiles per step of each background warp (by layout, mode)
   int ring_stride;         // chunk-tiles reserved per warp in `ring`
   const float* bias;       // [2 modes][16 CTAs][N_BIAS]
   const float* att_v;      // [256]
   float v_l1;              // ||attention_v||_1
-  Program prog[2];         // [0] free running, [1] teacher forcing
+  Program prog[2][2];     // by layout, then [0] free running, [1] teacher forcing
 };
 
 }  // namespace cw

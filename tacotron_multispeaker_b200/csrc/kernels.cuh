@@ -122,7 +122,7 @@ struct DecoderArgs {
   const float* keys;     // [N,T_in,256] = memory * W_mem
   const float* targets;  // [N,T_tgt,M] or null (free running)
   int N, T_in, T_tgt, r, steps, max_steps;
-  int att_res;           // keys/memory slices resident in shared memory (set by launch_decoder)
+  int att_res;           // keys/memory slices resident in shared memory, or (decoder_cw, cw::ATT_TMEM) in tensor memory (set by the launcher)
   int s_max;             // decoder_cw: largest number of samples per cluster in this launch (set by the launcher)
   float* dec_out;        // [N,max_steps,Dout]
   float* align_out;      // [N,T_in,max_steps] or null
@@ -134,6 +134,9 @@ struct DecoderArgs {
 // bf16_only: one product per chunk-tile (W_hi x_hi) instead of the fp32-class three (taco_set_gemm_mode(2)).
 cudaError_t launch_decoder_cw(const cw::Weights& w, const DecoderArgs& a, int nclusters, cudaStream_t st, bool bf16_only = false);
 size_t decoder_cw_smem_bytes(int s_max, int T_in, int att_res, int ring_kb);
+// Host only: where the attention operands of a launch with <= s_max utterances per cluster live (att_res: 3 shared memory,
+// cw::ATT_TMEM tensor memory, 1 / 2 / 0 partly or not resident) and the weight-ring depth; false if nothing fits.
+bool decoder_cw_plan(int s_max, int T_in, int* att_res, int* ring_kb, size_t* smem);
 int decoder_cw_max_clusters();
 
 // S = samples per cluster (1,2,4,8).  Returns cudaError of the launch.

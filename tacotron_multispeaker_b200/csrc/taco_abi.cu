@@ -710,25 +710,38 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
 // decoder weight set once per step, so fewer/larger clusters save L2 bandwidth while more
 // clusters shorten the per-sample work; clusters beyond the co-resident maximum run as extra
 // waves.  Per-wave step times (us) measured on B200 (tools/dec_sweep.py, round 1).
-// Clusters for the mma.sync decoder: whole waves of co-resident clusters, <= 8 samples each; the
-// per-wave time grows with the samples per cluster (exchange bytes), roughly 1 + 0.1 S.
+// Clusters for the mma.sync decoder (decoder_cw.cu), <= 8 utterances each, maxc of them co-resident.  Every cluster count from
+// ceil(N / 8) up is costed as waves x t(S), with t the step time of a cluster of S utterances; among the counts within
+// CW_PICK_MARGIN of the cheapest, the fewest clusters win: a cluster holds 16 SMs for the whole decode, so fewer clusters leave
+// more of the GPU to the other work in flight.  The margin is 20 %: batch 32 as 4 clusters of 8 decodes 18 % slower than as
+// 7 clusters of 5 (11.03 vs 9.38 us/step) but takes 33 % fewer SM-microseconds per step, which is what several batches in
+// flight share (+15 % mel frames/s with four in flight).  Small batches pay the same way: batch 4 runs as one cluster of 4.
+constexpr float CW_PICK_MARGIN = 0.20f;
+// t(S), us per free-running step, S = 1..8: decoder_cw_kernel with four clusters of S utterances at T_in 100 (attention
+// operands on chip at every S), tools/dec_sweep.py on a B200 at a 1000 W power limit.
+constexpr float CW_STEP_US[8] = {7.60f, 8.21f, 8.86f, 9.11f, 9.38f, 10.45f, 10.78f, 11.03f};
+int pick_cw_clusters(int N, int maxc) {
+  maxc = std::max(1, maxc);
+  const int lo = (N + 7) / 8;
+  float best = 1e30f;
+  std::vector<float> cost;
+  for (int ncl = lo; ncl <= N; ++ncl) {
+    const int S = (N + ncl - 1) / ncl;
+    cost.push_back((float)((ncl + maxc - 1) / maxc) * CW_STEP_US[S - 1]);
+    best = std::min(best, cost.back());
+    if (S == 1) break;
+  }
+  for (size_t i = 0; i < cost.size(); ++i)
+    if (cost[i] <= best * (1.0f + CW_PICK_MARGIN)) return lo + (int)i;
+  return lo;
+}
 int pick_mma_clusters(const taco_handle* h, int N) {
   if (h->dec_clusters > 0) return std::min(N, std::max(h->dec_clusters, (N + 7) / 8));
   const char* en = h->dev_env ? getenv("TACO_DEC_NCL") : nullptr;
   if (en && atoi(en) > 0) return std::min(N, std::max(atoi(en), (N + 7) / 8));
   const char* es = h->dev_env ? getenv("TACO_DEC_S") : nullptr;   // samples per cluster (tests sweep it; TACO_DEV=1)
   if (es && atoi(es) > 0) return (N + std::min(atoi(es), 8) - 1) / std::min(atoi(es), 8);
-  const int maxc = std::max(1, h->max_clusters_mma);
-  float best = 1e30f;
-  int bn = (N + 7) / 8;
-  for (int waves = 1; waves <= 64; ++waves) {
-    const int ncl = std::min(N, waves * maxc), S = (N + ncl - 1) / ncl;
-    if (S > 8) continue;
-    const float cost = ((ncl + maxc - 1) / maxc) * (1.0f + 0.1f * S);
-    if (cost < best - 1e-4f) { best = cost; bn = ncl; }
-    if (ncl == N) break;
-  }
-  return bn;
+  return pick_cw_clusters(N, h->max_clusters_mma);
 }
 
 void pick_geometry(const taco_handle* h, int N, int* cs_out, int* s_out) {
@@ -1101,7 +1114,8 @@ int taco_finalize_weights(taco_handle* h) {
   {
     const char* ei = getenv("TACO_DEC_IMPL");   // "cw" (default) | "v2": developer switch to the fp32 FFMA decoder
     // "cw" (default): decoder_cw.cu
-    h->decw.tmem_img = B + O6.tmem; h->decw.ring = B + O6.ring; h->decw.bias = B + O6.bias; h->decw.att_v = B + O6.att_v;
+    for (int lay = 0; lay < 2; ++lay) { h->decw.tmem_img[lay] = B + O6.tmem[lay]; h->decw.ring[lay] = B + O6.ring[lay]; }
+    h->decw.bias = B + O6.bias; h->decw.att_v = B + O6.att_v;
     h->use_cw = mma_ok && decoder_cw_max_clusters() >= 1 && !(ei && strcmp(ei, "cw") != 0);
     h->max_clusters_mma = h->use_cw ? decoder_cw_max_clusters() : 0;
   }
@@ -1888,6 +1902,19 @@ int taco_decoder_geometry(const taco_handle* h, int N, int* cluster_size, int* s
 int taco_set_gemm_mode(taco_handle* h, int mode) {
   if (!h || mode < 0 || mode > 2) return TACO_ERR_INVALID;
   h->gemm_mode = mode;
+  return TACO_OK;
+}
+
+int taco_decoder_plan(int N, int T_in, int max_clusters, taco_decoder_plan_t* plan) {
+  if (!plan) return TACO_ERR_INVALID;
+  memset(plan, 0, sizeof(*plan));
+  if (N < 1 || T_in < 1 || T_in > 512 || max_clusters < 1) return TACO_ERR_INVALID;
+  const int ncl = pick_cw_clusters(N, max_clusters), S = (N + ncl - 1) / ncl;
+  int att_res = 0, ring_kb = 0;
+  size_t smem = 0;
+  if (!decoder_cw_plan(S, T_in, &att_res, &ring_kb, &smem)) return TACO_ERR_INVALID;
+  plan->valid = 1; plan->clusters = ncl; plan->s_max = S; plan->att_res = att_res; plan->ring_kb = ring_kb;
+  plan->smem_bytes = (int32_t)smem;
   return TACO_OK;
 }
 

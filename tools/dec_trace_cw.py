@@ -64,8 +64,9 @@ def run(N, T_in, S, tag, iters=40, teacher=False, cta=0):
 
 if __name__ == "__main__":
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    for wtr in os.environ.get("TRACE_WARPS", "8,0,4").split(","):
-        os.environ["TACO_DEC_TRACE_WARP"] = wtr
-        run(32, 100, 5, "cw_n32_s5_w" + wtr)
+    for S in (int(x) for x in os.environ.get("TRACE_S", "5").split(",")):   # config 3 cut into clusters of S
+        for wtr in os.environ.get("TRACE_WARPS", "8,0,4").split(","):
+            os.environ["TACO_DEC_TRACE_WARP"] = wtr
+            run(32, 100, S, "cw_n32_s%d_w%s" % (S, wtr))
     if os.environ.get("TRACE_N1"):
         run(1, 100, 1, "cw_n1_s1")
