@@ -276,6 +276,26 @@ int64_t taco_spectrogram_frames(const taco_audio_params* ap, int64_t L);
 int taco_spectrogram(taco_handle* h, const taco_audio_params* ap, const float* wav, const int32_t* lengths_host, int N,
                      int64_t L, int T_out, float* linear_out, float* mel_out, void* stream);
 
+/* ---- resampling: librosa 0.5.1 core.resample / core.load -------------------- */
+/* Samples librosa.core.resample(y, sr_orig, sr_new, fix=True) returns for L input samples: ceil(L * (double)sr_new /
+ * sr_orig), as numpy computes it.  < 0 on bad arguments.  No device needed. */
+int64_t taco_resample_length(int64_t L, int32_t sr_orig, int32_t sr_new);
+/* Where resampy 0.1.5's resample_f reads the filter for outputs t0 .. t0+count-1: n = int(reg) of the double time register
+ * advanced by 1/ratio per output, and the table offset and interpolation factor of the left (frac = scale (reg - n)) and
+ * right (scale - frac) wings, eta rounded to float.  The replay taco_resample uses.  TACO_ERR_INVALID on rates <= 0 or
+ * t0 + count > 2^24.  Host only. */
+int taco_resample_positions(int32_t sr_orig, int32_t sr_new, int64_t t0, int64_t count, int32_t* n, int32_t* offset_l,
+                            float* eta_l, int32_t* offset_r, float* eta_r);
+/* librosa.core.resample(x, sr_orig, sr_new, res_type='kaiser_best', fix=True) for a batch: resampy's band-limited
+ * interpolation (kaiser_best: 64 zero crossings, 512 table entries per crossing, index step truncated to
+ * int(min(1, ratio) 512), the accumulated time register) then fix_length.  x [N, L] dense float32 on the device;
+ * lengths_host [N] (HOST, each in [1, L]) or NULL (all L).  y [N, L_out]: row n gets ceil(len * ratio) samples, of which
+ * [int(len * ratio), ceil) are 0.0, and 0.0 up to L_out.  Equal rates copy the input.  Needs no weights.
+ * TACO_ERR_INVALID: a rate <= 0, a length outside [1, L], or L_out < the longest output.  TACO_ERR_UNSUPPORTED:
+ * N * L_out >= 2^31, sr_orig > 8 sr_new, or more than 2^24 filter outputs in a row. */
+int taco_resample(taco_handle* h, int32_t sr_orig, int32_t sr_new, const float* x, const int32_t* lengths_host, int N,
+                  int64_t L, float* y, int64_t L_out, void* stream);
+
 /* ---- arithmetic mode of the dense layers ----------------------------------- */
 /* The reference computes in fp32.  0 = fp32 FFMA kernels; 1 (default) = tcgen05 tensor
  * cores with every operand split into bf16 hi+lo and three products per k-step

@@ -15,11 +15,17 @@
   ``taco_spectrogram`` kernel.  They return ``[T, F]``, the layout the model
   and the feeder consume (the reference returns ``[F, T]`` and its
   preprocessing saves the transpose).
+* ``resample(engine, y, orig_sr, target_sr)`` / ``load(engine, path,
+  sample_rate)`` -- ``librosa.core.resample`` (resampy ``kaiser_best``,
+  ``fix=True``) as the ``taco_resample`` kernel, and ``librosa.core.load``
+  (16-bit PCM of any rate and channel count, mixed down on the host, resampled
+  on the device): the reference reads its corpora with
+  ``librosa.core.load(path, sr=hparams.sample_rate)``.
 * ``save_wav`` (``:14-16``), ``load_wav``, ``find_endpoint`` (``:55-63``),
   ``_stft_parameters`` (``:114-118``) are host code (numpy / ``wave``): they
   handle a finished waveform once per utterance.
 
-There is no CPU Griffin-Lim or STFT here: without the CUDA library these raise.
+There is no CPU Griffin-Lim, STFT or resampler here: without the CUDA library these raise.
 """
 from __future__ import annotations
 
@@ -68,6 +74,36 @@ def load_wav(path, sample_rate):
                              % (path, int(sample_rate), f.getnchannels(), 8 * f.getsampwidth(), f.getframerate()))
         pcm = np.frombuffer(f.readframes(f.getnframes()), "<i2")
     return pcm.astype(np.float32) / np.float32(32768.0)
+
+
+def resample(engine, y, orig_sr, target_sr):
+    """``librosa.core.resample(y, orig_sr, target_sr)`` (``res_type='kaiser_best'``, ``fix=True``) of one waveform on the
+    device: ``ceil(len(y) * target_sr / orig_sr)`` samples, the input unchanged when the rates are equal."""
+    return engine.resample(y, orig_sr, target_sr)
+
+
+def read_pcm(path):
+    """librosa.core.load's samples before resampling, on the host: a 16-bit PCM WAV file as float32 ``pcm * (1 /
+    32768)`` (audioread's conversion), channels mixed down with ``np.mean`` (``librosa.to_mono``).  Returns ``(samples,
+    native rate)``.  Other sample widths raise ``ValueError``."""
+    with wave.open(str(path), "rb") as f:
+        channels, width, rate = f.getnchannels(), f.getsampwidth(), f.getframerate()
+        if width != 2:
+            raise ValueError("%s: need 16-bit PCM, got %d-bit" % (path, 8 * width))
+        pcm = np.frombuffer(f.readframes(f.getnframes()), "<i2")
+    y = np.float32(1.0 / 32768) * pcm.astype(np.float32)
+    if channels > 1:
+        y = np.mean(y.reshape((-1, channels)).T, axis=0)
+    return y, rate
+
+
+def load(engine, path, sample_rate):
+    """``librosa.core.load(path, sr=sample_rate)`` for 16-bit PCM WAV files of any sample rate and channel count: read and
+    mixed down on the host (``read_pcm``), resampled on the device (``resample``).  Returns a float32 CUDA tensor."""
+    y, rate = read_pcm(path)
+    if y.size == 0:
+        raise ValueError("%s: no samples" % path)
+    return engine.resample(y, rate, int(sample_rate))
 
 
 def wav_to_int16(wav) -> np.ndarray:

@@ -175,4 +175,23 @@ struct SpectrogramArgs {
 void launch_fft_tables(float2* tw, float* win, int win_len, cudaStream_t st);
 cudaError_t launch_spectrogram(const SpectrogramArgs& a, cudaStream_t st);
 
+// Resampling (resample.cu): librosa 0.5.1 core.resample with resampy's kaiser_best filter.  pos[t] for t < n_pos: where
+// output t reads the filter (the host's replay of resampy's time register); rows [RS_ROWS][taps]: (win, delta) of the
+// filter at offset o + i index_step.  span: the longest input window a CTA of RS_T outputs stages (samples).
+constexpr int RS_T = 128, RS_U = 16, RS_BLK = 32, RS_ROWS = 513;
+struct ResamplePos { int n, off_l, off_r; float eta_l, eta_r; };
+struct ResampleArgs {
+  const float* x;        // [N][L]
+  long long L;
+  int N;
+  const int* lengths;    // device [2N]: input samples per row, then the outputs the filter computes (int(len ratio))
+  const ResamplePos* pos; long long n_pos;
+  const float2* rows; int taps, span;
+  float* y;              // [N][L_out]
+  long long L_out;
+  bool copy;             // equal rates: y = x, zero past each length
+};
+size_t resample_smem_bytes(int span);
+cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t st);
+
 }  // namespace taco

@@ -8,6 +8,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
+#include <cmath>
 #include <map>
 #include <string>
 #include <vector>
@@ -137,6 +139,14 @@ struct taco_handle {
     int sample_rate = 0, win = 0;
     std::vector<char> host;
   } spec_tab;
+  // taco_resample's filter rows and replayed positions in an allocation of their own: [RS_ROWS][taps] float2 rows, then
+  // n_pos ResamplePos; rebuilt when the rate pair changes or a call needs more positions.  span: the longest window a CTA
+  // stages over those positions.
+  struct ResTables {
+    char* dev = nullptr; size_t bytes = 0;
+    int sr_orig = 0, sr_new = 0, taps = 0, span = 0;
+    int64_t n_pos = -1;
+  } res_tab;
   bool launch_failed = false;        // a kernel launcher returned an error (sticky until check_launch reports it)
   bool profiling = false;
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // [4],[5] bracket the decoder kernel
@@ -994,6 +1004,7 @@ int taco_destroy(taco_handle* h) {
   if (h->stg) cudaFree(h->stg);
   if (h->d_ints) cudaFree(h->d_ints);
   if (h->spec_tab.dev) cudaFree(h->spec_tab.dev);
+  if (h->res_tab.dev) cudaFree(h->res_tab.dev);
   if (h->h_pinned) cudaFreeHost(h->h_pinned);
   for (int i = 0; i < 6; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->ev_compute) cudaEventDestroy(h->ev_compute);
@@ -1879,6 +1890,157 @@ int taco_spectrogram(taco_handle* h, const taco_audio_params* ap, const float* w
   CUDA_OK(h, launch_spectrogram(a, st));
   h->launches += 1;
   return check_launch(h, "spectrogram");
+}
+
+// ---- resampling: librosa 0.5.1 core.resample / resampy 0.1.5 kaiser_best ----------------------------------------------
+static constexpr int kResZeros = 64, kResTable = 512;                   // num_zeros, 2^precision
+static constexpr int kResNwin = kResZeros * kResTable + 1;              // 32 769 entries
+static constexpr double kResBeta = 14.769656459379492, kResRolloff = 0.9475937167399596;
+static constexpr int64_t kResMaxOutputs = (int64_t)1 << 24;            // cap on the replayed positions (20 B each)
+
+static double res_ratio(int32_t sr_orig, int32_t sr_new) { return (double)sr_new / (double)sr_orig; }
+static int res_index_step(double ratio) { return (int)(std::min(1.0, ratio) * kResTable); }
+
+// resampy's resample_f register, replayed exactly: a double advanced by 1 / ratio per output (never t / ratio).  Output t
+// takes n = int(reg), frac = scale (reg - n); offset / eta of the left wing from frac * 512, of the right wing from
+// (scale - frac) * 512.  Kept free of contractions so that it matches the float64 replay of the tests bit for bit.
+__attribute__((optimize("fp-contract=off")))
+static void res_replay(int32_t sr_orig, int32_t sr_new, int64_t t0, int64_t count, int32_t* n, int32_t* off_l, float* eta_l,
+                       int32_t* off_r, float* eta_r) {
+  const double ratio = res_ratio(sr_orig, sr_new), scale = std::min(1.0, ratio), inc = 1.0 / ratio;
+  double reg = 0.0;
+  for (int64_t t = 0; t < t0 + count; reg += inc, ++t) {
+    if (t < t0) continue;
+    const int64_t k = t - t0;
+    const int32_t nn = (int32_t)reg;
+    double frac = scale * (reg - nn);
+    double index_frac = frac * kResTable;
+    const int32_t ol = (int32_t)index_frac;
+    const double el = index_frac - ol;
+    frac = scale - frac;
+    index_frac = frac * kResTable;
+    const int32_t orr = (int32_t)index_frac;
+    n[k] = nn; off_l[k] = ol; eta_l[k] = (float)el; off_r[k] = orr; eta_r[k] = (float)(index_frac - orr);
+  }
+}
+
+// kaiser_best's half window (resampy sinc_window: kaiser(2n+1, beta)[n:] * rolloff * sinc(rolloff * linspace(0, 64, n+1)))
+// times ratio when downsampling, and its forward difference (last entry 0), laid out as rows[o][i] = (win, delta) at
+// o + i index_step for i < (nwin - o) / index_step, zero after.
+static void res_rows(double ratio, int taps, std::vector<float2>& rows) {
+  std::vector<double> win(kResNwin), delta(kResNwin, 0.0);
+  const double n = kResNwin - 1, i0b = std::cyl_bessel_i(0.0, kResBeta);
+  for (int m = 0; m < kResNwin; ++m) {
+    const double r = m / n, taper = std::cyl_bessel_i(0.0, kResBeta * sqrt(std::max(0.0, 1.0 - r * r))) / i0b;
+    const double x = kResRolloff * (m * ((double)kResZeros / n)), s = m == 0 ? 1.0 : sin(M_PI * x) / (M_PI * x);
+    win[m] = taper * (kResRolloff * s);
+    if (ratio < 1) win[m] *= ratio;
+  }
+  for (int m = 0; m + 1 < kResNwin; ++m) delta[m] = win[m + 1] - win[m];
+  const int step = res_index_step(ratio);
+  rows.assign((size_t)RS_ROWS * taps, make_float2(0.0f, 0.0f));
+  for (int o = 0; o < RS_ROWS; ++o)
+    for (int i = 0; i < (kResNwin - o) / step && i < taps; ++i)
+      rows[(size_t)o * taps + i] = make_float2((float)win[o + i * step], (float)delta[o + i * step]);
+}
+
+// (re)builds h->res_tab when the rate pair changes or more than the cached positions are needed
+static int ensure_res_tables(taco_handle* h, int32_t sr_orig, int32_t sr_new, int64_t n_pos, cudaStream_t st) {
+  auto& R = h->res_tab;
+  if (R.dev && R.sr_orig == sr_orig && R.sr_new == sr_new && R.n_pos >= n_pos) return TACO_OK;
+  const double ratio = res_ratio(sr_orig, sr_new);
+  const int taps = kResNwin / res_index_step(ratio);
+  std::vector<float2> rows;
+  res_rows(ratio, taps, rows);
+  std::vector<int32_t> n(n_pos), ol(n_pos), orr(n_pos);
+  std::vector<float> el(n_pos), er(n_pos);
+  res_replay(sr_orig, sr_new, 0, n_pos, n.data(), ol.data(), el.data(), orr.data(), er.data());
+  std::vector<ResamplePos> pos(n_pos);
+  int span = 1;
+  for (int64_t t = 0; t < n_pos; ++t) {
+    pos[t] = ResamplePos{n[t], ol[t], orr[t], el[t], er[t]};
+    if (t % RS_T == 0) {
+      const int64_t tl = std::min(t + RS_T, n_pos) - 1;
+      span = std::max<int64_t>(span, n[tl] - n[t] + 2 * (int64_t)taps);
+    }
+  }
+  const size_t rows_bytes = ((rows.size() * sizeof(float2)) + 255) & ~size_t(255);
+  const size_t bytes = rows_bytes + pos.size() * sizeof(ResamplePos);
+  if (R.dev) cudaDeviceSynchronize();   // work on other streams may still read the old tables
+  R.n_pos = -1;
+  if (bytes > R.bytes) {
+    if (R.dev) { cudaFree(R.dev); R.dev = nullptr; R.bytes = 0; }
+    CUDA_OK(h, cudaMalloc(&R.dev, bytes));
+    R.bytes = bytes;
+  }
+  CUDA_OK(h, cudaMemcpyAsync(R.dev, rows.data(), rows.size() * sizeof(float2), cudaMemcpyHostToDevice, st));
+  if (n_pos)
+    CUDA_OK(h, cudaMemcpyAsync(R.dev + rows_bytes, pos.data(), pos.size() * sizeof(ResamplePos), cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaStreamSynchronize(st));   // the host vectors are the copies' sources
+  R.sr_orig = sr_orig; R.sr_new = sr_new; R.taps = taps; R.span = span; R.n_pos = n_pos;
+  return TACO_OK;
+}
+
+int64_t taco_resample_length(int64_t L, int32_t sr_orig, int32_t sr_new) {
+  if (L < 1 || sr_orig <= 0 || sr_new <= 0) return -1;
+  return (int64_t)ceil((double)L * res_ratio(sr_orig, sr_new));
+}
+
+int taco_resample_positions(int32_t sr_orig, int32_t sr_new, int64_t t0, int64_t count, int32_t* n, int32_t* offset_l,
+                            float* eta_l, int32_t* offset_r, float* eta_r) {
+  if (sr_orig <= 0 || sr_new <= 0 || t0 < 0 || count < 0 || t0 + count > kResMaxOutputs) return TACO_ERR_INVALID;
+  if (count && (!n || !offset_l || !eta_l || !offset_r || !eta_r)) return TACO_ERR_INVALID;
+  res_replay(sr_orig, sr_new, t0, count, n, offset_l, eta_l, offset_r, eta_r);
+  return TACO_OK;
+}
+
+int taco_resample(taco_handle* h, int32_t sr_orig, int32_t sr_new, const float* x, const int32_t* lengths_host, int N,
+                  int64_t L, float* y, int64_t L_out, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (!x || !y || N <= 0 || L <= 0 || L_out <= 0 || sr_orig <= 0 || sr_new <= 0)
+    return fail(h, TACO_ERR_INVALID, "resample: bad argument");
+  const double ratio = res_ratio(sr_orig, sr_new);
+  const bool copy = sr_orig == sr_new;
+  std::vector<int32_t> len(2 * (size_t)N);
+  int64_t longest = 0, n_pos = 0;
+  for (int i = 0; i < N; ++i) {
+    const int64_t li = lengths_host ? lengths_host[i] : L;
+    if (li < 1 || li > L) return fail(h, TACO_ERR_INVALID, "resample: a length outside [1, L]");
+    const int64_t computed = copy ? li : (int64_t)((double)li * ratio);   // resampy: int(L ratio) filter outputs
+    len[i] = (int32_t)li;
+    len[N + i] = (int32_t)std::min<int64_t>(computed, INT32_MAX);
+    longest = std::max(longest, taco_resample_length(li, sr_orig, sr_new));
+    n_pos = std::max(n_pos, computed);
+  }
+  if (L_out < longest) return fail(h, TACO_ERR_INVALID, "resample: L_out is shorter than the longest output");
+  if ((int64_t)N * L_out >= ((int64_t)1 << 31)) return fail(h, TACO_ERR_UNSUPPORTED, "resample: N * L_out >= 2^31");
+  if (!copy && (int64_t)sr_orig > 8 * (int64_t)sr_new)   // the staged window of a CTA grows with the factor (130 KB at 8x)
+    return fail(h, TACO_ERR_UNSUPPORTED, "resample: downsampling by more than 8x");
+  if (!copy && n_pos > kResMaxOutputs) return fail(h, TACO_ERR_UNSUPPORTED, "resample: more than 2^24 outputs per row");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!copy) {
+    const int rc = ensure_res_tables(h, sr_orig, sr_new, n_pos, st);
+    if (rc) return rc;
+  }
+  int rc = ensure_ws(h, len.size() * sizeof(int32_t) + 256);
+  if (rc) return rc;
+  int* d_len = reinterpret_cast<int*>(h->ws);
+  CUDA_OK(h, cudaMemcpyAsync(d_len, len.data(), len.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  ResampleArgs a;
+  a.x = x; a.L = L; a.N = N; a.lengths = d_len;
+  a.pos = nullptr; a.n_pos = 0; a.rows = nullptr; a.taps = 0; a.span = 0;
+  a.y = y; a.L_out = L_out; a.copy = copy;
+  if (!copy) {
+    const auto& R = h->res_tab;
+    const size_t rows_bytes = (((size_t)RS_ROWS * R.taps * sizeof(float2)) + 255) & ~size_t(255);
+    a.rows = reinterpret_cast<const float2*>(R.dev);
+    a.pos = reinterpret_cast<const ResamplePos*>(R.dev + rows_bytes);
+    a.n_pos = n_pos; a.taps = R.taps; a.span = R.span;
+  }
+  CUDA_OK(h, launch_resample(a, st));
+  h->launches += 1;
+  return check_launch(h, "resample");
 }
 
 int64_t taco_launch_count(const taco_handle* h) { return h ? h->launches : 0; }

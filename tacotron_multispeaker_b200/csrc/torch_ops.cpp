@@ -14,6 +14,7 @@
 //   taco_b200::griffin_lim(handle, linear, iters, sample_rate, frame_shift_ms, frame_length_ms, ...) -> wav [N,L]
 //   taco_b200::spectrogram(handle, wav, lengths?, T_out?, sample_rate, frame_shift_ms, frame_length_ms, ...)
 //       -> (linear [N,T_out,num_freq], mel [N,T_out,num_mels])
+//   taco_b200::resample(handle, wav, lengths?, orig_sr, target_sr) -> y [N, L_out] (L_out: the longest ceil(len ratio))
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
@@ -201,6 +202,34 @@ std::tuple<at::Tensor, at::Tensor> spectrogram(int64_t handle, const at::Tensor&
   return std::make_tuple(lin, mel);
 }
 
+// wav [N, L] on the device; lengths (host integers, each in [1, L]) or None = all L
+at::Tensor resample(int64_t handle, const at::Tensor& wav, at::OptionalIntArrayRef lengths, int64_t orig_sr, int64_t target_sr) {
+  taco_handle* h = H(handle);
+  dev_f32(wav, "wav");
+  TORCH_CHECK(wav.dim() == 2, "taco_b200::resample: wav [N,L]");
+  c10::cuda::CUDAGuard guard(wav.device());
+  const int N = (int)wav.size(0);
+  const int64_t L = wav.size(1);
+  std::vector<int32_t> len;
+  int64_t L_out = 0;
+  if (lengths.has_value()) {
+    TORCH_CHECK((int64_t)lengths->size() == N, "taco_b200::resample: lengths [N]");
+    for (int64_t v : *lengths) {
+      TORCH_CHECK(v >= 1 && v <= L, "taco_b200::resample: lengths must be in [1, L]");
+      len.push_back((int32_t)v);
+      L_out = std::max<int64_t>(L_out, taco_resample_length(v, (int32_t)orig_sr, (int32_t)target_sr));
+    }
+  } else {
+    L_out = taco_resample_length(L, (int32_t)orig_sr, (int32_t)target_sr);
+  }
+  TORCH_CHECK(L_out > 0, "taco_b200::resample: bad sample rates");
+  at::Tensor y = at::empty({N, L_out}, wav.options());
+  ck(h, taco_resample(h, (int32_t)orig_sr, (int32_t)target_sr, wav.data_ptr<float>(), lengths.has_value() ? len.data() : nullptr,
+                      N, L, y.data_ptr<float>(), L_out, stream_of(wav)),
+     "resample");
+  return y;
+}
+
 }  // namespace
 
 TORCH_LIBRARY(taco_b200, m) {
@@ -213,6 +242,7 @@ TORCH_LIBRARY(taco_b200, m) {
         "float ref_level_db, float power, float preemphasis) -> Tensor");
   m.def("spectrogram(int handle, Tensor wav, int[]? lengths, int? T_out, int sample_rate, float frame_shift_ms, float frame_length_ms, "
         "float min_level_db, float ref_level_db, float preemphasis, int num_mels, int num_freq) -> (Tensor, Tensor)");
+  m.def("resample(int handle, Tensor wav, int[]? lengths, int orig_sr, int target_sr) -> Tensor");
 }
 TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("forward", &forward);
@@ -221,4 +251,5 @@ TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("postnet", &postnet);
   m.impl("griffin_lim", &griffin_lim);
   m.impl("spectrogram", &spectrogram);
+  m.impl("resample", &resample);
 }

@@ -323,7 +323,46 @@ class Engine:
         lengths.  Returns ``(linear, mel)`` CUDA tensors ``[N, T_out, num_freq]`` / ``[N, T_out, num_mels]`` (``[T, F]``
         for one 1-D waveform); ``T_out`` defaults to the longest utterance's frames, and rows past an utterance's own
         frames are 0.0, the padding of the teacher-forcing targets."""
-        single = False
+        wav, len_host, single = self._batch(wav, lengths)
+        N, L = wav.shape
+        longest = int(len_host.max()) if len_host is not None else L
+        T = self.spectrogram_frames(longest) if T_out is None else int(T_out)
+        hp = self.hp
+        lin = torch.empty(N, T, hp.num_freq, device=self.device, dtype=torch.float32)
+        mel = torch.empty(N, T, hp.num_mels, device=self.device, dtype=torch.float32)
+        self._ck(self.lib.taco_spectrogram(self._h, C.byref(self.audio_params()), _ptr(wav),
+                                           None if len_host is None else len_host.ctypes.data, N, L, T, _ptr(lin),
+                                           _ptr(mel), self.stream))
+        return (lin[0], mel[0]) if single else (lin, mel)
+
+    def resample_length(self, num_samples: int, orig_sr: int, target_sr: int) -> int:
+        """Samples ``librosa.core.resample`` returns for ``num_samples`` inputs: ``ceil(num_samples * target_sr /
+        orig_sr)`` (``taco_resample_length``)."""
+        n = int(self.lib.taco_resample_length(int(num_samples), int(orig_sr), int(target_sr)))
+        if n < 0:
+            raise ValueError("bad sample rate or length")
+        return n
+
+    def resample(self, wav, orig_sr: int, target_sr: int, lengths=None):
+        """``librosa.core.resample(wav, orig_sr, target_sr)`` with resampy's ``kaiser_best`` filter and ``fix=True``
+        (``taco_resample``) for one waveform ``[L]``, a batch ``[N, L]`` (with optional per-utterance ``lengths``) or a
+        list of 1-D waveforms of different lengths.  Returns a CUDA tensor ``[L_out]`` for one waveform; for a batch
+        ``(y [N, L_out], out_lengths)``, where row n holds ``out_lengths[n] = ceil(len_n * target_sr / orig_sr)`` samples
+        and 0.0 after them."""
+        wav, len_host, single = self._batch(wav, lengths)
+        N, L = wav.shape
+        lens = len_host if len_host is not None else np.full(N, L, np.int32)
+        out_len = np.asarray([self.resample_length(v, orig_sr, target_sr) for v in lens], np.int64)
+        L_out = int(out_len.max())
+        y = torch.empty(N, L_out, device=self.device, dtype=torch.float32)
+        self._ck(self.lib.taco_resample(self._h, int(orig_sr), int(target_sr), _ptr(wav),
+                                        None if len_host is None else len_host.ctypes.data, N, L, _ptr(y), L_out,
+                                        self.stream))
+        return y[0] if single else (y, out_len)
+
+    def _batch(self, wav, lengths):
+        """(wav [N, L] float32 on the device, host int32 lengths [N] or None, whether the input was one 1-D waveform) for
+        a waveform, a batch with optional lengths or a list of 1-D waveforms."""
         if isinstance(wav, (list, tuple)):
             if lengths is not None:
                 raise ValueError("lengths are implied by a list of waveforms")
@@ -336,27 +375,19 @@ class Engine:
                 batch[i, :s.size] = s
             wav = batch
         wav = self._f32(wav)
+        single = False
         if wav.dim() == 1:
             if lengths is not None:
                 raise ValueError("lengths need a batch [N, L]")
             single, wav = True, wav[None]
         if wav.dim() != 2 or wav.shape[1] == 0:
             raise ValueError("wav must be [L] or [N, L] with L >= 1")
-        N, L = wav.shape
         len_host = None
         if lengths is not None:
             len_host = np.ascontiguousarray(np.asarray(lengths).reshape(-1), dtype=np.int32)
-            if len_host.shape != (N,):
+            if len_host.shape != (wav.shape[0],):
                 raise ValueError("lengths must be [N]")
-        longest = int(len_host.max()) if len_host is not None else L
-        T = self.spectrogram_frames(longest) if T_out is None else int(T_out)
-        hp = self.hp
-        lin = torch.empty(N, T, hp.num_freq, device=self.device, dtype=torch.float32)
-        mel = torch.empty(N, T, hp.num_mels, device=self.device, dtype=torch.float32)
-        self._ck(self.lib.taco_spectrogram(self._h, C.byref(self.audio_params()), _ptr(wav),
-                                           None if len_host is None else len_host.ctypes.data, N, L, T, _ptr(lin),
-                                           _ptr(mel), self.stream))
-        return (lin[0], mel[0]) if single else (lin, mel)
+        return wav, len_host, single
 
     # ---- whole path ----
     def forward(self, ids, lengths, spk=None, mel_targets=None, teacher_force=False,

@@ -25,6 +25,7 @@ import io
 from typing import Optional
 
 import numpy as np
+import torch
 
 from . import audio, plot
 from .engine import pad_targets
@@ -80,20 +81,25 @@ class Synthesizer:
         wav = audio.synthesize_wav(self.model.engine, self.model.linear_outputs[0])
         return wav.cpu().numpy(), self.model.alignments[0].cpu().numpy()
 
-    def teacher_forced(self, text, identity, wav, path_align=None):
+    def teacher_forced(self, text, identity, wav, path_align=None, orig_sr=None):
         """Teacher-forced run on a text and its recording: the attention alignment of the two and the ground-truth-aligned
-        mel outputs.  ``wav`` is a path (``audio.load_wav``: mono 16-bit PCM at ``hparams.sample_rate``) or an array of
-        samples.  Its mel spectrogram (``audio.melspectrogram`` on the GPU), padded as the feeder pads targets
-        (``pad_targets``), feeds the decoder through ``initialize(..., teacher_force=True)``; batch norm keeps its
-        moving statistics.  As in the reference, the decoder stops after min(max_iters, T_targets / r) steps, and
-        ``load`` sets max_iters to 400, so a recording longer than 400 * r frames is cut there.  Returns
-        ``(mel_outputs [steps*r, num_mels], alignment [T_in, steps])`` as numpy arrays and writes the alignment image
-        to ``path_align`` when given."""
-        if isinstance(wav, (str, bytes)) or hasattr(wav, "__fspath__"):
-            wav = audio.load_wav(wav, self.hparams.sample_rate)
+        mel outputs.  ``wav`` is a path (``audio.load``: 16-bit PCM WAV of any sample rate and channel count, mixed down
+        and resampled to ``hparams.sample_rate`` as ``librosa.core.load`` does), an array of samples or a CUDA tensor;
+        an array or tensor recorded at another rate is resampled from ``orig_sr``.  Its mel spectrogram
+        (``audio.melspectrogram`` on the GPU), padded as the feeder pads targets (``pad_targets``), feeds the decoder
+        through ``initialize(..., teacher_force=True)``; batch norm keeps its moving statistics.  As in the reference, the
+        decoder stops after min(max_iters, T_targets / r) steps, and ``load`` sets max_iters to 400, so a recording longer
+        than 400 * r frames is cut there.  Returns ``(mel_outputs [steps*r, num_mels], alignment [T_in, steps])`` as
+        numpy arrays and writes the alignment image to ``path_align`` when given."""
         seq = np.asarray(text_to_sequence2(text, [x.strip() for x in self.hparams.cleaners.split(",")])[:-1], np.int32)
         engine = self.model._get_engine(self.id_num if self.id_num > 1 else 0)
-        mel = audio.melspectrogram(engine, np.asarray(wav, dtype=np.float32).reshape(-1))
+        if isinstance(wav, (str, bytes)) or hasattr(wav, "__fspath__"):
+            wav = audio.load(engine, wav, self.hparams.sample_rate)
+        elif orig_sr is not None:
+            wav = audio.resample(engine, torch.as_tensor(wav).reshape(-1), orig_sr, self.hparams.sample_rate)
+        if not isinstance(wav, torch.Tensor):
+            wav = np.asarray(wav, dtype=np.float32)
+        mel = audio.melspectrogram(engine, wav.reshape(-1))
         targets = pad_targets([mel.cpu().numpy()], self.hparams.outputs_per_step)
         self.model.initialize(seq[None, :], np.asarray([seq.size], np.int32), mel_targets=targets,
                               identities=np.asarray([identity], np.int32), id_num=self.id_num, teacher_force=True)

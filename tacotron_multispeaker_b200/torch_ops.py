@@ -18,7 +18,7 @@ from . import _abi
 _LIB = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libtaco_b200_torch.so")
 _loaded = False
 
-OPS = ("forward", "encoder", "decode", "postnet", "griffin_lim", "spectrogram")
+OPS = ("forward", "encoder", "decode", "postnet", "griffin_lim", "spectrogram", "resample")
 
 
 def load() -> str:
