@@ -236,6 +236,14 @@ int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan
 int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers, const float* w_h_host,
                        const float* b_h_host, const float* w_t_host, const float* b_t_host, float* out, void* out_hi,
                        void* out_lo, void* stream);
+/* The BiGRU recurrence of modules.py:68-74 alone, on caller-supplied hoisted projections and recurrent kernels.
+ * impl 0: the fp32 FFMA kernel (bigru.cu), 1: the tensor-core kernel (bigru_mma.cu); independent of TACO_BIGRU and
+ * of the gemm mode.  xproj [N,T,768] device, 16-byte aligned: [fw gates 256 | fw cand 128 | bw gates 256 | bw cand 128]
+ * with the input biases included; lengths device int32 [N] or NULL; ug_host [2][128][256], uc_host [2][128][128]:
+ * the recurrent halves (rows 128..255) of each direction's gates / candidate kernel; out [N,T,256] device, 16-byte
+ * aligned.  TACO_ERR_INVALID for a bad impl, N <= 0, T <= 0, a NULL pointer or a misaligned xproj / out. */
+int taco_bigru_unit(taco_handle* h, int impl, const float* xproj, const int32_t* lengths, int N, int T,
+                    const float* ug_host, const float* uc_host, float* out, void* stream);
 
 /* ---- vocoder: the step right after the path (SURVEY.md 8f rank 2) ----------- */
 /* Fields of reference hparams.py:13-18,35-36 that util/audio.py reads. */

@@ -37,7 +37,7 @@ SYMBOLS = [
     "taco_set_gemm_mode", "taco_launch_count", "taco_decoder_geometry", "taco_set_decoder_clusters", "taco_set_profiling", "taco_last_stage_ms", "taco_set_cuda_graphs",
     "taco_wav_length", "taco_griffin_lim", "taco_spectrogram_frames", "taco_spectrogram",
     "taco_resample_length", "taco_resample_positions", "taco_resample",
-    "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit", "taco_decoder_plan",
+    "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit", "taco_bigru_unit", "taco_decoder_plan",
 ]
 
 
@@ -159,6 +159,7 @@ def load() -> C.CDLL:
     lib.taco_umma_plan.argtypes = [C.POINTER(TacoGemmDesc), i, C.POINTER(TacoGemmPlan)]
     lib.taco_gemm_unit.argtypes = [H, C.POINTER(TacoGemmDesc), C.POINTER(TacoGemmPlan), vp]
     lib.taco_highway4_unit.argtypes = [H, fp, i64, i, vp, vp, vp, vp, fp, vp, vp, vp]
+    lib.taco_bigru_unit.argtypes = [H, i, fp, ip, i, i, vp, vp, fp, vp]
     lib.taco_decoder_plan.argtypes = [i, i, i, C.POINTER(TacoDecoderPlan)]
     for name in SYMBOLS:
         getattr(lib, name)  # AttributeError here = header and library out of sync

@@ -1447,6 +1447,41 @@ int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers,
   return check_launch(h, "highway4 unit");
 }
 
+int taco_bigru_unit(taco_handle* h, int impl, const float* xproj, const int32_t* lengths, int N, int T, const float* ug_host,
+                    const float* uc_host, float* out, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if ((impl != 0 && impl != 1) || !xproj || !ug_host || !uc_host || !out || N <= 0 || T <= 0)
+    return fail(h, TACO_ERR_INVALID, "bad argument");
+  if (!al16(xproj) || !al16(out)) return fail(h, TACO_ERR_INVALID, "xproj and out must be 16-byte aligned");
+  // the recurrent kernels (and for impl 1 their fragment stream), staged on the host as pack_cbhg stages them
+  Arena A;
+  const size_t ug = A.alloc(2 * 128 * 256), uc = A.alloc(2 * 128 * 128);
+  memcpy(&A.buf[ug], ug_host, sizeof(float) * 2 * 128 * 256);
+  memcpy(&A.buf[uc], uc_host, sizeof(float) * 2 * 128 * 128);
+  size_t frag = 0;
+  if (impl == 1) {
+    frag = A.alloc(bigru_mma_frag_words());
+    bigru_mma_pack(&A.buf[ug], &A.buf[uc], reinterpret_cast<uint32_t*>(&A.buf[frag]));
+  }
+  int rc = ensure_ws(h, sizeof(float) * A.buf.size() + 65536);
+  if (rc) return rc;
+  Bump ws(h->ws, h->ws_bytes);
+  float* dP = ws.take<float>(A.buf.size());
+  if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (bigru unit)");
+  cudaStream_t st = (cudaStream_t)stream;
+  CUDA_OK(h, cudaMemcpyAsync(dP, A.buf.data(), sizeof(float) * A.buf.size(), cudaMemcpyHostToDevice, st));
+  const int64_t out_bs = (int64_t)T * 256;
+  if (impl == 1) {
+    cudaError_t e = launch_bigru_mma(xproj, dP + frag, lengths, N, T, out, out_bs, st);
+    if (e != cudaSuccess) return fail(h, TACO_ERR_CUDA, std::string("bigru_mma launch: ") + cudaGetErrorString(e));
+  } else {
+    launch_bigru(xproj, dP + ug, dP + uc, lengths, N, T, out, out_bs, st);
+  }
+  h->launches += 1;
+  return check_launch(h, "bigru unit");
+}
+
 // Post-net again on the true length after an early stop (the all-zero frame case): rare, synchronous.
 static int redo_postnet(taco_handle* h, int N, int T_in, int max_steps, int steps, int bn_mode, const float* mel,
                         float* linear_out, cudaStream_t st) {

@@ -277,6 +277,19 @@ class Engine:
         self._ck(self.lib.taco_highway4_unit(self._h, _ptr(x), x.shape[0], w_h.shape[0], w_h.ctypes.data, b_h.ctypes.data,
                                              w_t.ctypes.data, b_t.ctypes.data, _ptr(out), _ptr(hi), _ptr(lo), self.stream))
 
+    def bigru_unit(self, xproj, ug, uc, lengths=None, impl=0, out=None):
+        """``taco_bigru_unit``: the BiGRU recurrence alone on hoisted projections xproj [N, T, 768] (device, fp32) with host
+        recurrent kernels ug [2, 128, 256], uc [2, 128, 128]; impl 0 = fp32 FFMA kernel, 1 = tensor-core kernel.  Writes
+        ``out`` [N, T, 256] (device; allocated when None, else any 16-byte aligned dense view) and returns it."""
+        ug, uc = (np.ascontiguousarray(a, dtype=np.float32) for a in (ug, uc))
+        N, T, _ = xproj.shape
+        lengths = self._i32(lengths)
+        if out is None:
+            out = torch.empty(N, T, 256, device=self.device, dtype=torch.float32)
+        self._ck(self.lib.taco_bigru_unit(self._h, int(impl), _ptr(xproj), _ptr(lengths), N, T, ug.ctypes.data,
+                                          uc.ctypes.data, _ptr(out), self.stream))
+        return out
+
     # ---- vocoder (the step after the path) ----
     def audio_params(self, griffin_lim_iters: Optional[int] = None) -> "_abi.TacoAudioParams":
         hp = self.hp

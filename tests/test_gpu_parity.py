@@ -148,7 +148,8 @@ def test_bn_batch_stats_kat(eng, N, T, C):
 
 
 @pytest.mark.parametrize("which,N,T,masked", [(0, 5, 23, True), (0, 3, 11, False), (1, 2, 60, False),
-                                              (0, 80, 9, True), (1, 1, 150, False), (0, 8, 31, True), (0, 9, 31, True), (1, 33, 40, False)])
+                                              (0, 80, 9, True), (1, 1, 150, False), (0, 8, 31, True), (0, 9, 31, True), (1, 33, 40, False),
+                                              (0, 149, 40, True)])
 def test_bigru(eng, ow, which, N, T, masked):
     rng = np.random.default_rng(N * 100 + T)
     x = rng.standard_normal((N, T, 128)).astype(np.float32)
@@ -165,7 +166,8 @@ def test_bigru(eng, ow, which, N, T, masked):
             assert np.all(g[i, lengths[i]:] == 0.0)
 
 
-@pytest.mark.parametrize("which,N,T,masked", [(0, 5, 23, True), (1, 2, 60, False), (0, 19, 9, True)])
+@pytest.mark.parametrize("which,N,T,masked", [(0, 5, 23, True), (1, 2, 60, False), (0, 19, 9, True), (1, 8, 40, True),
+                                              (0, 16, 31, True)])
 def test_bigru_tensor_core_variant(eng, ow, which, N, T, masked, monkeypatch):
     """TACO_BIGRU=mma: the same recurrence on mma.sync with the recurrent weights in tensor memory, 8 utterances per
     CTA (bf16 hi/lo operands: fp32-class; ragged lengths, a last CTA with fewer than 8 utterances)."""
