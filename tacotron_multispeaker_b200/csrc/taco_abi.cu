@@ -37,15 +37,21 @@ struct HostVar {
 };
 
 // One GEMM-shaped weight: fp32 [taps*Cin][ldw] for the FFMA path and W^T split into bf16 hi/lo
-// ([b_rows][Kld], K contiguous) for the tcgen05 path.
+// ([b_rows][Kld], K contiguous) for the tcgen05 path.  A bank holds its convolutions back to back: conv ci has ci+1 taps,
+// its fp32 rows [(ci+1)*Cin][ldw] start at row Cin*ci*(ci+1)/2 and its W^T rows are [ci*Cout, (ci+1)*Cout).
 struct GemmW {
-  size_t w = 0; int ldw = 0;
-  size_t bt = 0;                       // bf16 element offset of the hi matrix (lo follows at + b_rows*Kld)
+  size_t off = 0;                      // float offset of the fp32 weights in the staging arena, until w points at the upload
+  const float* w = nullptr; int ldw = 0;
+  uint16_t* b_hi = nullptr; uint16_t* b_lo = nullptr;
   int taps = 1, Cin = 0, Cout = 0, Cp = 0, Kld = 0, b_rows = 0, bank = 1;
+  int member_taps(int ci) const { return bank > 1 ? ci + 1 : taps; }
+  const float* member_w(int ci) const { return w + (size_t)ci * (ci + 1) / 2 * Cin * ldw; }
+  // the fp32 weights in `arena` as uploaded; W^T hi at bt, lo right after it
+  void place(const float* arena, uint16_t* bt) { w = arena + off; b_hi = bt; b_lo = bt + (size_t)b_rows * Kld; }
 };
-GemmW make_gemmw(size_t w, int ldw, int taps, int Cin, int Cout, int bank = 1) {
+GemmW make_gemmw(size_t off, int ldw, int taps, int Cin, int Cout, int bank = 1) {
   GemmW g;
-  g.w = w; g.ldw = ldw; g.taps = taps; g.Cin = Cin; g.Cout = Cout; g.bank = bank;
+  g.off = off; g.ldw = ldw; g.taps = taps; g.Cin = Cin; g.Cout = Cout; g.bank = bank;
   g.Cp = (Cin + 63) & ~63;
   g.Kld = taps * g.Cp;
   g.b_rows = bank > 1 ? bank * Cout : Cout;
@@ -54,13 +60,12 @@ GemmW make_gemmw(size_t w, int ldw, int taps, int Cin, int Cout, int bank = 1) {
 
 struct CbhgDev {   // offsets (floats) into the device weight arena
   int K = 0, Cin = 0, P1 = 0, P2 = 0;
-  std::vector<size_t> bank_w, bank_b;
   size_t bank_scale = 0, bank_shift = 0, bank_gamma = 0, bank_beta = 0;
-  size_t p1_w = 0, p1_b = 0, p1_scale = 0, p1_shift = 0, p1_gamma = 0, p1_beta = 0;
-  size_t p2_w = 0, p2_b = 0, p2_scale = 0, p2_shift = 0, p2_gamma = 0, p2_beta = 0;
-  size_t dense_w = 0, dense_b = 0;
-  size_t hw_w[4] = {0, 0, 0, 0}, hw_b[4] = {0, 0, 0, 0};
-  size_t gru_wx = 0, gru_bx = 0, gru_ug = 0, gru_uc = 0, gru_frag = 0;   // gru_frag: MMA fragment stream (bigru_mma.cu)
+  size_t p1_b = 0, p1_scale = 0, p1_shift = 0, p1_gamma = 0, p1_beta = 0;
+  size_t p2_b = 0, p2_scale = 0, p2_shift = 0, p2_gamma = 0, p2_beta = 0;
+  size_t dense_b = 0;
+  size_t hw_b[4] = {0, 0, 0, 0};
+  size_t gru_bx = 0, gru_ug = 0, gru_uc = 0, gru_frag = 0;   // gru_frag: MMA fragment stream (bigru_mma.cu)
   size_t bank_bias = 0;                // biases of the K bank convolutions back to back
   GemmW g_bank, g_p1, g_p2, g_dense, g_hw[4], g_xproj;
 };
@@ -85,8 +90,8 @@ struct taco_handle {
   bool finalized = false;
   // packed weights
   float* dW = nullptr;
-  size_t emb = 0, emb_id = 0, pre1_w = 0, pre1_b = 0, pre2_w = 0, pre2_b = 0, mem_w = 0, lin_w = 0, lin_b = 0;
-  int lin_ld = 0, emb_dim = 0;
+  size_t emb = 0, emb_id = 0, pre1_b = 0, pre2_b = 0, lin_b = 0;
+  int emb_dim = 0;
   GemmW g_pre1, g_pre2, g_mem, g_lin;
   uint16_t* dB = nullptr;              // bf16 arena: W^T hi/lo for the tensor-core path
   int gemm_mode = 1;                   // 0 = fp32 FFMA, 1 = bf16x3 tcgen05 (fp32-class), 2 = bf16 tcgen05
@@ -274,8 +279,9 @@ size_t put_vec(Arena& A, const float* src, int n) {
 
 // One highway layer (modules.py:79-89) as ONE GEMM: W_H, W_T [128][128] -> [128][256] with columns interleaved (H_c, T_c),
 // biases likewise [256] (the epilogues and highway4_kernel read the gate pair of channel c from columns 2c, 2c + 1).
-void put_highway(Arena& A, const float* wh, const float* bh, const float* wt, const float* bt, size_t& w_off, size_t& b_off) {
-  w_off = A.alloc(128 * 256);
+// Returns the offset of the weights.
+size_t put_highway(Arena& A, const float* wh, const float* bh, const float* wt, const float* bt, size_t& b_off) {
+  const size_t w_off = A.alloc(128 * 256);
   b_off = A.alloc(256);
   for (int r = 0; r < 128; ++r)
     for (int c = 0; c < 128; ++c) {
@@ -286,18 +292,13 @@ void put_highway(Arena& A, const float* wh, const float* bh, const float* wt, co
     A.buf[b_off + 2 * c] = bh[c];
     A.buf[b_off + 2 * c + 1] = bt[c];
   }
+  return w_off;
 }
 
-// W^T of a GEMM as bf16 hi / lo [b_rows][Kld] at hi (lo follows), from the fp32 weights at base + w_off[0] ([taps*Cin][ldw]);
-// a bank reads conv ci ([(ci+1)*Cin][ldw]) at base + w_off[ci] into rows ci*Cout ...
-void pack_gemmw(const GemmW& g, const float* base, const size_t* w_off, uint16_t* hi, cudaStream_t st) {
-  uint16_t* lo = hi + (size_t)g.b_rows * g.Kld;
-  if (g.bank > 1) {
-    for (int ci = 0; ci < g.bank; ++ci)
-      launch_pack_wt(base + w_off[ci], g.ldw, ci + 1, g.Cin, g.Cout, g.Cp, g.Kld, ci * g.Cout, hi, lo, st);
-  } else {
-    launch_pack_wt(base + w_off[0], g.ldw, g.taps, g.Cin, g.Cout, g.Cp, g.Kld, 0, hi, lo, st);
-  }
+// W^T of a GEMM as bf16 hi / lo at g.b_hi / g.b_lo, from its fp32 weights at g.w: one pack launch per bank member
+void pack_gemmw(const GemmW& g, cudaStream_t st) {
+  for (int ci = 0; ci < g.bank; ++ci)
+    launch_pack_wt(g.member_w(ci), g.ldw, g.member_taps(ci), g.Cin, g.Cout, g.Cp, g.Kld, ci * g.Cout, g.b_hi, g.b_lo, st);
 }
 
 // conv1d() of the reference: kernel/bias + BN.  Emits weights, bias and the four
@@ -324,14 +325,13 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
   D.K = K; D.Cin = Cin; D.P1 = P1; D.P2 = P2;
   const int BC = K * 128;
   D.bank_scale = A.alloc(BC); D.bank_shift = A.alloc(BC); D.bank_gamma = A.alloc(BC); D.bank_beta = A.alloc(BC);
-  D.bank_w.resize(K); D.bank_b.resize(K);
   D.bank_bias = A.alloc(BC);
+  D.g_bank = make_gemmw(A.alloc((size_t)K * (K + 1) / 2 * Cin * 128), 128, K, Cin, 128, K);
   for (int k = 1; k <= K; ++k) {
     const std::string sc = s + "/conv_bank/conv1d_" + std::to_string(k);
     GETV(w, sc + "/conv1d/kernel", k, Cin, 128);
     GETV(b, sc + "/conv1d/bias", 128);
-    D.bank_w[k - 1] = put_matrix(A, w->data.data(), k * Cin, 128, 128);
-    D.bank_b[k - 1] = put_vec(A, b->data.data(), 128);
+    memcpy(&A.buf[D.g_bank.off + (size_t)(k - 1) * k / 2 * Cin * 128], w->data.data(), sizeof(float) * k * Cin * 128);
     const int o = (k - 1) * 128;
     memcpy(&A.buf[D.bank_bias + o], b->data.data(), sizeof(float) * 128);
     if (!pack_bn(h, sc, 128, &A.buf[D.bank_scale + o], &A.buf[D.bank_shift + o], &A.buf[D.bank_gamma + o],
@@ -341,7 +341,7 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
   {
     GETV(w, s + "/proj_1/conv1d/kernel", 3, BC, P1);
     GETV(b, s + "/proj_1/conv1d/bias", P1);
-    D.p1_w = put_matrix(A, w->data.data(), 3 * BC, P1, P1);
+    D.g_p1 = make_gemmw(put_matrix(A, w->data.data(), 3 * BC, P1, P1), P1, 3, BC, P1);
     D.p1_b = put_vec(A, b->data.data(), P1);
     D.p1_scale = A.alloc(P1); D.p1_shift = A.alloc(P1); D.p1_gamma = A.alloc(P1); D.p1_beta = A.alloc(P1);
     if (!pack_bn(h, s + "/proj_1", P1, &A.buf[D.p1_scale], &A.buf[D.p1_shift], &A.buf[D.p1_gamma],
@@ -351,7 +351,7 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
   {
     GETV(w, s + "/proj_2/conv1d/kernel", 3, P1, P2);
     GETV(b, s + "/proj_2/conv1d/bias", P2);
-    D.p2_w = put_matrix(A, w->data.data(), 3 * P1, P2, P2);
+    D.g_p2 = make_gemmw(put_matrix(A, w->data.data(), 3 * P1, P2, P2), P2, 3, P1, P2);
     D.p2_b = put_vec(A, b->data.data(), P2);
     D.p2_scale = A.alloc(P2); D.p2_shift = A.alloc(P2); D.p2_gamma = A.alloc(P2); D.p2_beta = A.alloc(P2);
     if (!pack_bn(h, s + "/proj_2", P2, &A.buf[D.p2_scale], &A.buf[D.p2_shift], &A.buf[D.p2_gamma],
@@ -361,7 +361,7 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
   if (P2 != 128) {   // reference modules.py:59-60
     GETV(w, s + "/dense/kernel", P2, 128);
     GETV(b, s + "/dense/bias", 128);
-    D.dense_w = put_matrix(A, w->data.data(), P2, 128, 128);
+    D.g_dense = make_gemmw(put_matrix(A, w->data.data(), P2, 128, 128), 128, 1, P2, 128);
     D.dense_b = put_vec(A, b->data.data(), 128);
   }
   for (int i = 0; i < 4; ++i) {
@@ -370,10 +370,12 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
     GETV(bh, hs + "/H/bias", 128);
     GETV(wt, hs + "/T/kernel", 128, 128);
     GETV(bt, hs + "/T/bias", 128);
-    put_highway(A, wh->data.data(), bh->data.data(), wt->data.data(), bt->data.data(), D.hw_w[i], D.hw_b[i]);
+    D.g_hw[i] = make_gemmw(put_highway(A, wh->data.data(), bh->data.data(), wt->data.data(), bt->data.data(), D.hw_b[i]),
+                           256, 1, 128, 256);
   }
   // BiGRU: gates/kernel [256,256] rows = [x(128); h(128)], candidate/kernel [256,128] likewise.
-  D.gru_wx = A.alloc(128 * 768); D.gru_bx = A.alloc(768);
+  const size_t gru_wx = A.alloc(128 * 768);
+  D.gru_bx = A.alloc(768);
   D.gru_ug = A.alloc(2 * 128 * 256); D.gru_uc = A.alloc(2 * 128 * 128);
   int d = 0;
   for (const char* dn : {"fw", "bw"}) {
@@ -383,8 +385,8 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
     GETV(wc, gs + "/candidate/kernel", 256, 128);
     GETV(bc, gs + "/candidate/bias", 128);
     for (int r = 0; r < 128; ++r) {
-      memcpy(&A.buf[D.gru_wx + (size_t)r * 768 + d * 384], &wg->data[(size_t)r * 256], sizeof(float) * 256);
-      memcpy(&A.buf[D.gru_wx + (size_t)r * 768 + d * 384 + 256], &wc->data[(size_t)r * 128], sizeof(float) * 128);
+      memcpy(&A.buf[gru_wx + (size_t)r * 768 + d * 384], &wg->data[(size_t)r * 256], sizeof(float) * 256);
+      memcpy(&A.buf[gru_wx + (size_t)r * 768 + d * 384 + 256], &wc->data[(size_t)r * 128], sizeof(float) * 128);
       memcpy(&A.buf[D.gru_ug + ((size_t)d * 128 + r) * 256], &wg->data[(size_t)(128 + r) * 256], sizeof(float) * 256);
       memcpy(&A.buf[D.gru_uc + ((size_t)d * 128 + r) * 128], &wc->data[(size_t)(128 + r) * 128], sizeof(float) * 128);
     }
@@ -394,12 +396,7 @@ bool pack_cbhg(taco_handle* h, Arena& A, const std::string& s, int K, int Cin, i
   }
   D.gru_frag = A.alloc(bigru_mma_frag_words());
   bigru_mma_pack(&A.buf[D.gru_ug], &A.buf[D.gru_uc], reinterpret_cast<uint32_t*>(&A.buf[D.gru_frag]));
-  D.g_bank = make_gemmw(0, 128, K, Cin, 128, K);
-  D.g_p1 = make_gemmw(D.p1_w, P1, 3, BC, P1);
-  D.g_p2 = make_gemmw(D.p2_w, P2, 3, P1, P2);
-  if (P2 != 128) D.g_dense = make_gemmw(D.dense_w, 128, 1, P2, 128);
-  for (int i = 0; i < 4; ++i) D.g_hw[i] = make_gemmw(D.hw_w[i], 256, 1, 128, 256);
-  D.g_xproj = make_gemmw(D.gru_wx, 768, 1, 128, 768);
+  D.g_xproj = make_gemmw(gru_wx, 768, 1, 128, 768);
   return true;
 }
 
@@ -540,19 +537,15 @@ struct Ctx {
   const float* W(size_t off) const { return h->dW + off; }
 };
 
-void conv(Ctx& c, const float* x, int64_t x_bs, int ldx, int N, int T, int Cin, int k, const float* w, int ldw,
-          const float* bias, const float* scale, const float* shift, const float* res, int64_t res_bs, int ldres,
-          float* out, int64_t out_bs, int ldo, int col_off, int Cout, int act, int epi = EPI_PLAIN) {
-  ConvGemm p;
-  p.x = x; p.x_bs = x_bs; p.ldx = ldx; p.N = N; p.T = T; p.Cin = Cin; p.k = k; p.w = w; p.ldw = ldw;
-  p.bias = bias; p.scale = scale; p.shift = shift; p.res = res; p.res_bs = res_bs; p.ldres = ldres;
-  p.out = out; p.out_bs = out_bs; p.ldo = ldo; p.col_off = col_off; p.Cout = Cout; p.act = act; p.epi = epi;
-  launch_conv_gemm(p, c.st);
-  c.h->launches += 1;
+// A launcher returned e: the first such error of a call stays in h->err, and check_launch returns it at the end of the call.
+void launch_error(taco_handle* h, cudaError_t e, const char* what) {
+  if (e == cudaSuccess) return;
+  if (!h->launch_failed) h->err = std::string(what) + ": " + cudaGetErrorString(e);
+  h->launch_failed = true;
 }
 
 // bf16 hi/lo staging of a GEMM's activation operand (tcgen05 path)
-struct BfScratch { uint16_t* hi = nullptr; uint16_t* lo = nullptr; };
+struct BfScratch { void* hi = nullptr; void* lo = nullptr; };
 BfScratch take_bf(Bump& ws, int64_t rows, int maxCp) {
   BfScratch s;
   s.hi = ws.take<uint16_t>((size_t)rows * maxCp);
@@ -560,37 +553,61 @@ BfScratch take_bf(Bump& ws, int64_t rows, int maxCp) {
   return s;
 }
 
-// One conv1d/dense site: tensor cores (default) or the fp32 FFMA kernel (gemm_mode 0).
-void gemm(Ctx& c, const GemmW& g, const BfScratch& sc, const float* x, int64_t x_bs, int ldx, int N, int T,
-          const float* bias, const float* scale, const float* shift, const float* res, int64_t res_bs, int ldres,
-          float* out, int64_t out_bs, int ldo, int col_off, int act, int epi = EPI_PLAIN, bool presplit = false,
-          const BfScratch* next = nullptr, int next_cp = 0, bool skip_fp32 = false) {
-  // presplit: sc already holds the bf16 hi/lo operand (written by the producer), x is not read
-  // next (tensor-core path only): the epilogue also writes the result as the hi/lo operand [N][T][next_cp] of the GEMM that
-  // consumes it (no split pass in between); skip_fp32: and does not write the fp32 copy at all (nothing else reads it)
+// A operand [N][T][Cin] of a GEMM: fp32 x[n*x_bs + t*ldx + c], split into bf ahead of a tensor-core launch; or, presplit,
+// already in bf as the hi / lo operand (written by the producer's epilogue), and x is not read.
+struct GemmIn { const float* x; int64_t x_bs; int ldx; BfScratch bf; bool presplit = false; };
+// Epilogue: act(acc + bias), then the per-channel affine, then the residual; EPI_HIGHWAY reads res as the carry input.
+// A bank's convolution ci reads bias / scale / shift at ci*Cout.
+struct GemmEpi {
+  int act = TACO_ACT_NONE;
+  const float* bias = nullptr; const float* scale = nullptr; const float* shift = nullptr;
+  const float* res = nullptr; int64_t res_bs = 0; int ldres = 0;
+  int epi = EPI_PLAIN;
+};
+// Results: fp32 out[n*out_bs + t*ldo + col_off + c], not written when out is null; on the tensor cores, optionally also the
+// hi / lo operand [N][T][copy_cp] of the GEMM that consumes the result, so that no split pass runs in between.
+struct GemmOut {
+  float* out; int64_t out_bs; int ldo; int col_off = 0;
+  const BfScratch* copy = nullptr; int copy_cp = 0;
+};
+
+// The tensor-core launch of one GEMM site; a is the split A operand.
+ConvUmma make_umma(const GemmW& g, int N, int T, const BfScratch& a, const GemmEpi& ep, const GemmOut& o, int nsplit) {
+  ConvUmma u;
+  u.a_hi = a.hi; u.a_lo = a.lo; u.N = N; u.T = T; u.Cp = g.Cp; u.Cin = g.Cin;
+  u.b_hi = g.b_hi; u.b_lo = g.b_lo; u.b_rows = g.b_rows; u.Kld = g.Kld;
+  u.taps = g.taps; u.bank = g.bank; u.Cout = g.Cout; u.nsplit = nsplit;
+  u.bias = ep.bias; u.scale = ep.scale; u.shift = ep.shift; u.res = ep.res; u.res_bs = ep.res_bs; u.ldres = ep.ldres;
+  u.out = o.out; u.out_bs = o.out_bs; u.ldo = o.ldo; u.col_off = o.col_off; u.act = ep.act; u.epi = ep.epi;
+  if (o.copy) { u.out_hi = o.copy->hi; u.out_lo = o.copy->lo; u.out_cp = o.copy_cp; }
+  return u;
+}
+
+// One conv1d / dense site in the handle's gemm mode: the fp32 FFMA kernel (mode 0, one launch per bank member), or the split
+// pass unless the operand is presplit, then the tensor-core kernel (mode 1: three bf16 products, mode 2: one).  *plan (if
+// given) receives the tensor-core launch's plan.  A failed launch is also recorded as the call's sticky launch error.
+cudaError_t run_gemm(Ctx& c, const GemmW& g, int N, int T, const GemmIn& in, const GemmEpi& ep, const GemmOut& o,
+                     taco_gemm_plan* plan = nullptr) {
   taco_handle* h = c.h;
   if (h->gemm_mode == 0) {
-    conv(c, x, x_bs, ldx, N, T, g.Cin, g.taps, c.W(g.w), g.ldw, bias, scale, shift, res, res_bs, ldres, out, out_bs, ldo,
-         col_off, g.Cout, act, epi);
-    return;
+    for (int ci = 0; ci < g.bank; ++ci) {
+      const int m = ci * g.Cout;
+      ConvGemm p;
+      p.x = in.x; p.x_bs = in.x_bs; p.ldx = in.ldx; p.N = N; p.T = T; p.Cin = g.Cin; p.k = g.member_taps(ci);
+      p.w = g.member_w(ci); p.ldw = g.ldw;
+      p.bias = ep.bias ? ep.bias + m : nullptr; p.scale = ep.scale ? ep.scale + m : nullptr; p.shift = ep.shift ? ep.shift + m : nullptr;
+      p.res = ep.res; p.res_bs = ep.res_bs; p.ldres = ep.ldres;
+      p.out = o.out; p.out_bs = o.out_bs; p.ldo = o.ldo; p.col_off = o.col_off + m; p.Cout = g.Cout; p.act = ep.act; p.epi = ep.epi;
+      launch_conv_gemm(p, c.st);
+    }
+    h->launches += g.bank;
+    return cudaSuccess;
   }
-  if (!presplit) launch_split_bf16(x, x_bs, ldx, N, T, g.Cin, g.Cp, sc.hi, sc.lo, c.st);
-  ConvUmma u;
-  u.a_hi = sc.hi; u.a_lo = sc.lo; u.N = N; u.T = T; u.Cp = g.Cp; u.Cin = g.Cin;
-  u.b_hi = h->dB + g.bt; u.b_lo = h->dB + g.bt + (size_t)g.b_rows * g.Kld; u.b_rows = g.b_rows; u.Kld = g.Kld;
-  u.taps = g.taps; u.bank = g.bank; u.Cout = g.Cout; u.nsplit = h->gemm_mode == 2 ? 1 : 3;
-  u.bias = bias; u.scale = scale; u.shift = shift; u.res = res; u.res_bs = res_bs; u.ldres = ldres;
-  u.out = out; u.out_bs = out_bs; u.ldo = ldo; u.col_off = col_off; u.act = act; u.epi = epi;
-  if (next != nullptr) {
-    u.out_hi = next->hi; u.out_lo = next->lo; u.out_cp = next_cp;
-    if (skip_fp32) u.out = nullptr;
-  }
-  cudaError_t e = launch_conv_umma(u, c.st);
-  if (e != cudaSuccess) {
-    if (!h->launch_failed) h->err = std::string("conv_umma launch: ") + cudaGetErrorString(e);
-    h->launch_failed = true;
-  }
-  h->launches += presplit ? 1 : 2;
+  if (!in.presplit) launch_split_bf16(in.x, in.x_bs, in.ldx, N, T, g.Cin, g.Cp, in.bf.hi, in.bf.lo, c.st);
+  const cudaError_t e = launch_conv_umma(make_umma(g, N, T, in.bf, ep, o, h->gemm_mode == 2 ? 1 : 3), c.st, plan);
+  launch_error(h, e, "conv_umma launch");
+  h->launches += in.presplit ? 1 : 2;
+  return e;
 }
 
 // BiGRU recurrence: the fp32 FFMA kernel (1 utterance per CTA, weights in registers; default) or, TACO_BIGRU=mma, the
@@ -600,11 +617,7 @@ void run_bigru(Ctx& c, const CbhgDev& D, const float* xproj, const int32_t* leng
   const char* impl = c.h->dev_env ? getenv("TACO_BIGRU") : nullptr;   // developer switch (TACO_DEV=1): the parity tests run both
   const bool use_mma = impl && std::string(impl) == "mma";
   if (use_mma) {
-    cudaError_t e = launch_bigru_mma(xproj, c.W(D.gru_frag), lengths, N, T, out, out_bs, c.st);
-    if (e != cudaSuccess) {
-      if (!c.h->launch_failed) c.h->err = std::string("bigru_mma launch: ") + cudaGetErrorString(e);
-      c.h->launch_failed = true;
-    }
+    launch_error(c.h, launch_bigru_mma(xproj, c.W(D.gru_frag), lengths, N, T, out, out_bs, c.st), "bigru_mma launch");
   } else {
     launch_bigru(xproj, c.W(D.gru_ug), c.W(D.gru_uc), lengths, N, T, out, out_bs, c.st);
   }
@@ -635,18 +648,9 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
   // trip through split_bf16_kernel.  Batch statistics need the fp32 tensors (moments, in-place affine): the split passes stay.
   const bool chain = c.h->gemm_mode != 0 && !batch;
   // conv bank: K convolutions written side by side (tf.concat, modules.py:39-42)
-  if (c.h->gemm_mode != 0) {   // one launch for the whole bank
-    gemm(c, D.g_bank, x_split != nullptr ? *x_split : sc, x, x_bs, Cin, N, T, c.W(D.bank_bias), batch ? nullptr : c.W(D.bank_scale),
-         batch ? nullptr : c.W(D.bank_shift), nullptr, 0, 0, bank, (int64_t)T * BC, BC, 0, TACO_ACT_RELU, EPI_PLAIN,
-         /*presplit=*/x_split != nullptr);
-  } else {
-    for (int k = 1; k <= K; ++k) {
-      const int o = (k - 1) * 128;
-      conv(c, x, x_bs, Cin, N, T, Cin, k, c.W(D.bank_w[k - 1]), 128, c.W(D.bank_b[k - 1]),
-           batch ? nullptr : c.W(D.bank_scale + o), batch ? nullptr : c.W(D.bank_shift + o), nullptr, 0, 0, bank,
-           (int64_t)T * BC, BC, o, 128, TACO_ACT_RELU);
-    }
-  }
+  run_gemm(c, D.g_bank, N, T, {x, x_bs, Cin, x_split != nullptr ? *x_split : sc, x_split != nullptr},
+           {TACO_ACT_RELU, c.W(D.bank_bias), batch ? nullptr : c.W(D.bank_scale), batch ? nullptr : c.W(D.bank_shift)},
+           {bank, (int64_t)T * BC, BC});
   // max-pool (+ batch-mode BN affine); on the tcgen05 path its output goes straight into the GEMM operand format
   const bool fuse_split = c.h->gemm_mode != 0 && D.g_p1.Cp == BC;
   if (batch) {
@@ -658,9 +662,9 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
   else launch_affine_maxpool(bank, pooled, N, T, BC, batch ? bnv : nullptr, batch ? bnv + 2048 : nullptr, c.st);
   c.h->launches += 1;
   // proj_1: conv k=3 + ReLU + BN
-  gemm(c, D.g_p1, sc, pooled, (int64_t)T * BC, BC, N, T, c.W(D.p1_b), batch ? nullptr : c.W(D.p1_scale),
-       batch ? nullptr : c.W(D.p1_shift), nullptr, 0, 0, p1, (int64_t)T * D.P1, D.P1, 0, TACO_ACT_RELU, EPI_PLAIN,
-       fuse_split, chain ? &sc2 : nullptr, D.g_p2.Cp, /*skip_fp32=*/chain);   // proj_1's output feeds proj_2 only
+  run_gemm(c, D.g_p1, N, T, {pooled, (int64_t)T * BC, BC, sc, fuse_split},
+           {TACO_ACT_RELU, c.W(D.p1_b), batch ? nullptr : c.W(D.p1_scale), batch ? nullptr : c.W(D.p1_shift)},
+           {chain ? nullptr : p1, (int64_t)T * D.P1, D.P1, 0, chain ? &sc2 : nullptr, D.g_p2.Cp});   // proj_1's output feeds proj_2 only
   if (batch) {
     launch_bn_batch_stats(p1, (int64_t)T * D.P1, D.P1, 0, N, T, D.P1, c.W(D.p1_gamma), c.W(D.p1_beta), kBnEps,
                           bnacc, bnv, bnv + 2048, c.st);
@@ -669,9 +673,10 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
   }
   // proj_2: conv k=3 + BN (no activation) + residual (modules.py:53,56)
   const bool p2_to_dense = chain && D.P2 != 128;   // post-net: proj_2's output feeds the 80 -> 128 dense only
-  gemm(c, D.g_p2, chain ? sc2 : sc, p1, (int64_t)T * D.P1, D.P1, N, T, c.W(D.p2_b), batch ? nullptr : c.W(D.p2_scale),
-       batch ? nullptr : c.W(D.p2_shift), batch ? nullptr : x, x_bs, Cin, p2, (int64_t)T * D.P2, D.P2, 0,
-       TACO_ACT_NONE, EPI_PLAIN, /*presplit=*/chain, p2_to_dense ? &sc : nullptr, D.g_dense.Cp, /*skip_fp32=*/p2_to_dense);
+  run_gemm(c, D.g_p2, N, T, {p1, (int64_t)T * D.P1, D.P1, chain ? sc2 : sc, chain},
+           {TACO_ACT_NONE, c.W(D.p2_b), batch ? nullptr : c.W(D.p2_scale), batch ? nullptr : c.W(D.p2_shift), batch ? nullptr : x,
+            x_bs, Cin},
+           {p2_to_dense ? nullptr : p2, (int64_t)T * D.P2, D.P2, 0, p2_to_dense ? &sc : nullptr, D.g_dense.Cp});
   if (batch) {
     launch_bn_batch_stats(p2, (int64_t)T * D.P2, D.P2, 0, N, T, D.P2, c.W(D.p2_gamma), c.W(D.p2_beta), kBnEps,
                           bnacc, bnv, bnv + 2048, c.st);
@@ -680,39 +685,32 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
   }
   const float* hin = p2;
   if (D.P2 != 128) {   // modules.py:59-60
-    gemm(c, D.g_dense, sc, p2, (int64_t)T * D.P2, D.P2, N, T, c.W(D.dense_b), nullptr, nullptr, nullptr, 0, 0, hwb,
-         (int64_t)T * 128, 128, 0, TACO_ACT_NONE, EPI_PLAIN, /*presplit=*/p2_to_dense);
+    run_gemm(c, D.g_dense, N, T, {p2, (int64_t)T * D.P2, D.P2, sc, p2_to_dense}, {TACO_ACT_NONE, c.W(D.dense_b)},
+             {hwb, (int64_t)T * 128, 128});
     hin = hwb;
   }
   // 4 highway layers (modules.py:63-64): one fused launch on the tensor-core path (the activation stays in registers, the result
-  // comes out as the hi / lo operand of the GRU input projection), four GEMM launches otherwise
-  static const bool hw_fuse_env = [] { const char* e = getenv("TACO_HW_FUSE"); return !(e && atoi(e) == 0); }();
-  bool hw_contig = c.h->gemm_mode != 0 && hw_fuse_env && D.g_xproj.Cp == 128;
-  for (int i = 0; i < 3 && hw_contig; ++i) hw_contig = D.g_hw[i + 1].bt == D.g_hw[i].bt + (size_t)2 * 256 * 128;
-  bool xproj_presplit = false;
-  if (hw_contig) {
+  // comes out as the hi / lo operand of the GRU input projection), four GEMM launches in gemm mode 0
+  const bool hw_fused = c.h->gemm_mode != 0;
+  if (hw_fused) {
     const float* hb[4] = {c.W(D.hw_b[0]), c.W(D.hw_b[1]), c.W(D.hw_b[2]), c.W(D.hw_b[3])};
-    cudaError_t e = launch_highway4(hin, nullptr, sc.hi, sc.lo, c.h->dB + D.g_hw[0].bt, hb, 4, rows, c.h->gemm_mode == 2 ? 1 : 3, c.st);
-    if (e != cudaSuccess) {
-      if (!c.h->launch_failed) c.h->err = std::string("highway4 launch: ") + cudaGetErrorString(e);
-      c.h->launch_failed = true;
-    }
+    launch_error(c.h, launch_highway4(hin, nullptr, sc.hi, sc.lo, D.g_hw[0].b_hi, hb, 4, rows, c.h->gemm_mode == 2 ? 1 : 3, c.st),
+                 "highway4 launch");
     c.h->launches += 1;
-    xproj_presplit = true;
   } else {
     float* bufs[2] = {hwa, hwb};
     int cur = 0;   // first output goes to hwa (hin is p2 or hwb)
     for (int i = 0; i < 4; ++i) {
       float* o = bufs[cur];
-      gemm(c, D.g_hw[i], sc, hin, (int64_t)T * 128, 128, N, T, c.W(D.hw_b[i]), nullptr, nullptr, hin, (int64_t)T * 128,
-           128, o, (int64_t)T * 128, 128, 0, TACO_ACT_NONE, EPI_HIGHWAY);
+      run_gemm(c, D.g_hw[i], N, T, {hin, (int64_t)T * 128, 128, sc},
+               {TACO_ACT_NONE, c.W(D.hw_b[i]), nullptr, nullptr, hin, (int64_t)T * 128, 128, EPI_HIGHWAY}, {o, (int64_t)T * 128, 128});
       hin = o;
       cur ^= 1;
     }
   }
   // hoisted GRU input projection for both directions, then the recurrence
-  gemm(c, D.g_xproj, sc, hin, (int64_t)T * 128, 128, N, T, c.W(D.gru_bx), nullptr, nullptr, nullptr, 0, 0, xproj,
-       (int64_t)T * 768, 768, 0, TACO_ACT_NONE, EPI_PLAIN, xproj_presplit);
+  run_gemm(c, D.g_xproj, N, T, {hin, (int64_t)T * 128, 128, sc, hw_fused}, {TACO_ACT_NONE, c.W(D.gru_bx)},
+           {xproj, (int64_t)T * 768, 768});
   run_bigru(c, D, xproj, lengths, N, T, out, (int64_t)T * 256);
 }
 
@@ -811,10 +809,10 @@ int do_encoder(taco_handle* h, Bump& ws, const int32_t* ids, const int32_t* leng
   // encoder prenet (modules.py:5-12; dropout is the identity, SURVEY §0)
   // prenet: dense_1's output feeds dense_2 only, dense_2's feeds the conv bank (as its operand) and proj_2 (as the fp32 residual)
   const bool chain = h->gemm_mode != 0;
-  gemm(c, h->g_pre1, sc, emb, (int64_t)T_in * (E + Es), E + Es, N, T_in, c.W(h->pre1_b), nullptr, nullptr, nullptr, 0, 0,
-       a1, (int64_t)T_in * 256, 256, 0, TACO_ACT_RELU, EPI_PLAIN, false, chain ? &sc2 : nullptr, h->g_pre2.Cp, /*skip_fp32=*/chain);
-  gemm(c, h->g_pre2, chain ? sc2 : sc, a1, (int64_t)T_in * 256, 256, N, T_in, c.W(h->pre2_b), nullptr, nullptr, nullptr, 0, 0, a2,
-       (int64_t)T_in * 128, 128, 0, TACO_ACT_RELU, EPI_PLAIN, /*presplit=*/chain, chain ? &sc : nullptr, h->enc.g_bank.Cp, false);
+  run_gemm(c, h->g_pre1, N, T_in, {emb, (int64_t)T_in * (E + Es), E + Es, sc}, {TACO_ACT_RELU, c.W(h->pre1_b)},
+           {chain ? nullptr : a1, (int64_t)T_in * 256, 256, 0, chain ? &sc2 : nullptr, h->g_pre2.Cp});
+  run_gemm(c, h->g_pre2, N, T_in, {a1, (int64_t)T_in * 256, 256, chain ? sc2 : sc, chain}, {TACO_ACT_RELU, c.W(h->pre2_b)},
+           {a2, (int64_t)T_in * 128, 128, 0, chain ? &sc : nullptr, h->enc.g_bank.Cp});
   run_cbhg(c, h->enc, ws, a2, (int64_t)T_in * 128, lengths, N, T_in, bn_mode, memory_out, chain ? &sc : nullptr);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (encoder cbhg)");
   return check_launch(h, "encoder");
@@ -856,8 +854,7 @@ int do_decode(taco_handle* h, Bump& ws, const float* memory, int N, int T_in, co
   if (h->gemm_mode != 0) sc = take_bf(ws, (int64_t)N * T_in, 256);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (decoder)");
   // BahdanauAttention memory_layer (no bias), once per utterance (tacotron.py:68)
-  gemm(c, h->g_mem, sc, memory, (int64_t)T_in * 256, 256, N, T_in, nullptr, nullptr, nullptr, nullptr, 0, 0, keys,
-       (int64_t)T_in * 256, 256, 0, TACO_ACT_NONE);
+  run_gemm(c, h->g_mem, N, T_in, {memory, (int64_t)T_in * 256, 256, sc}, {TACO_ACT_NONE}, {keys, (int64_t)T_in * 256, 256});
   DecoderArgs a;
   a.memory = memory; a.keys = keys; a.targets = teacher_force ? mel_targets : nullptr;
   a.N = N; a.T_in = T_in; a.T_tgt = T_tgt; a.r = hp.outputs_per_step; a.steps = max_steps; a.max_steps = max_steps;
@@ -921,24 +918,21 @@ int do_postnet(taco_handle* h, Bump& ws, const float* mel, int N, int T, int bn_
   run_cbhg(c, h->post, ws, mel, mel_bs, nullptr, N, T, bn_mode, post);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (postnet cbhg)");
   // linear_outputs = tf.layers.dense(post_outputs, num_freq)  (tacotron.py:101)
-  gemm(c, h->g_lin, sc, post, (int64_t)T * 256, 256, N, T, c.W(h->lin_b), nullptr, nullptr, nullptr, 0, 0, linear_out,
-       lin_bs, hp.num_freq, 0, TACO_ACT_NONE);
+  run_gemm(c, h->g_lin, N, T, {post, (int64_t)T * 256, 256, sc}, {TACO_ACT_NONE, c.W(h->lin_b)}, {linear_out, lin_bs, hp.num_freq});
   return check_launch(h, "postnet");
 }
 
-// The ConvUmma of a unit GEMM with its parameters at the given device pointers (the caller fills in the weight operand and,
-// unless d is presplit, the A operand).  For a bank, taps = bank: the heaviest conv and the width of the weight rows.
-ConvUmma unit_umma(const taco_gemm_desc& d, const float* bias, const float* scale, const float* shift) {
-  ConvUmma u;
-  const bool bank = d.bank > 1;
-  u.a_hi = d.x_hi; u.a_lo = d.x_lo; u.N = d.N; u.T = d.T; u.Cp = (d.Cin + 63) & ~63; u.Cin = d.Cin;
-  u.taps = bank ? d.bank : d.taps; u.bank = bank ? d.bank : 1; u.Cout = d.Cout; u.nsplit = 3;
-  u.b_hi = nullptr; u.b_lo = nullptr; u.b_rows = bank ? d.bank * d.Cout : d.Cout; u.Kld = u.taps * u.Cp;
-  u.bias = bias; u.scale = scale; u.shift = shift; u.res = d.res; u.res_bs = d.res_bs; u.ldres = d.ldres;
-  u.out = d.out; u.out_bs = d.out_bs; u.ldo = d.ldo; u.col_off = d.col_off; u.act = d.act; u.epi = d.epi;
-  u.out_hi = d.out_hi; u.out_lo = d.out_lo; u.out_cp = d.out_cp;
-  return u;
+// The weight of a unit GEMM (its fp32 weights staged at offset 0, ldw = Cout rounded up to 4).  For a bank, taps = bank: the
+// heaviest conv and the width of the weight rows.
+GemmW unit_gemmw(const taco_gemm_desc& d) {
+  const int bank = d.bank > 1 ? d.bank : 1;
+  return make_gemmw(0, (d.Cout + 3) & ~3, bank > 1 ? bank : d.taps, d.Cin, d.Cout, bank);
 }
+// Its epilogue and outputs, with the parameters at the given device pointers
+GemmEpi unit_epi(const taco_gemm_desc& d, const float* bias, const float* scale, const float* shift) {
+  return {d.act, bias, scale, shift, d.res, d.res_bs, d.ldres, d.epi};
+}
+GemmOut unit_out(const taco_gemm_desc& d, const BfScratch& copy) { return {d.out, d.out_bs, d.ldo, d.col_off, &copy, d.out_cp}; }
 
 }  // namespace
 
@@ -1060,23 +1054,19 @@ int taco_finalize_weights(taco_handle* h) {
     GETV(b1, "prenet/dense_1/bias", 256);
     GETV(w2, "prenet/dense_2/kernel", 256, 128);
     GETV(b2, "prenet/dense_2/bias", 128);
-    h->pre1_w = put_matrix(A, w1->data.data(), h->emb_dim, 256, 256);
+    h->g_pre1 = make_gemmw(put_matrix(A, w1->data.data(), h->emb_dim, 256, 256), 256, 1, h->emb_dim, 256);
     h->pre1_b = put_vec(A, b1->data.data(), 256);
-    h->pre2_w = put_matrix(A, w2->data.data(), 256, 128, 128);
+    h->g_pre2 = make_gemmw(put_matrix(A, w2->data.data(), 256, 128, 128), 128, 1, 256, 128);
     h->pre2_b = put_vec(A, b2->data.data(), 128);
     if (!pack_cbhg(h, A, "encoder_cbhg", 16, 128, 128, 128, h->enc, err)) return false;
     GETV(mw, "memory_layer/kernel", 256, 256);
-    h->mem_w = put_matrix(A, mw->data.data(), 256, 256, 256);
+    h->g_mem = make_gemmw(put_matrix(A, mw->data.data(), 256, 256, 256), 256, 1, 256, 256);
     if (!pack_cbhg(h, A, "post_cbhg", 8, hp.num_mels, 256, hp.num_mels, h->post, err)) return false;
     GETV(lw, "dense/kernel", 256, hp.num_freq);
     GETV(lb, "dense/bias", hp.num_freq);
-    h->lin_ld = (hp.num_freq + 3) & ~3;
-    h->lin_w = put_matrix(A, lw->data.data(), 256, hp.num_freq, h->lin_ld);
+    const int lin_ld = (hp.num_freq + 3) & ~3;
+    h->g_lin = make_gemmw(put_matrix(A, lw->data.data(), 256, hp.num_freq, lin_ld), lin_ld, 1, 256, hp.num_freq);
     h->lin_b = put_vec(A, lb->data.data(), hp.num_freq);
-    h->g_pre1 = make_gemmw(h->pre1_w, 256, 1, h->emb_dim, 256);
-    h->g_pre2 = make_gemmw(h->pre2_w, 128, 1, 256, 128);
-    h->g_mem = make_gemmw(h->mem_w, 256, 1, 256, 256);
-    h->g_lin = make_gemmw(h->lin_w, h->lin_ld, 1, 256, hp.num_freq);
     return true;
   };
   if (!build()) return bad(err.rfind("missing", 0) == 0 ? TACO_ERR_MISSING_WEIGHT : TACO_ERR_INVALID);
@@ -1105,17 +1095,22 @@ int taco_finalize_weights(taco_handle* h) {
     for (CbhgDev* D : {&h->enc, &h->post}) {
       gs.push_back(&D->g_bank); gs.push_back(&D->g_p1); gs.push_back(&D->g_p2);
       if (D->P2 != 128) gs.push_back(&D->g_dense);
+      // the four highway layers back to back, [layer][hi|lo][256][128] (2 * 256 * 128 elements each, a multiple of 128): the
+      // layout launch_highway4 reads from g_hw[0].b_hi
       for (int i = 0; i < 4; ++i) gs.push_back(&D->g_hw[i]);
       gs.push_back(&D->g_xproj);
     }
+    auto bt_elems = [](const GemmW* g) { return ((size_t)2 * g->b_rows * g->Kld + 127) & ~size_t(127); };
     size_t nb = 0;
-    for (GemmW* g : gs) { g->bt = nb; nb += ((size_t)2 * g->b_rows * g->Kld + 127) & ~size_t(127); }
+    for (GemmW* g : gs) nb += bt_elems(g);
     if (h->dB) { cudaDeviceSynchronize(); cudaFree(h->dB); h->dB = nullptr; }
     CUDA_OK(h, cudaMalloc(&h->dB, sizeof(uint16_t) * nb));
     CUDA_OK(h, cudaMemset(h->dB, 0, sizeof(uint16_t) * nb));
+    uint16_t* bt = h->dB;
     for (GemmW* g : gs) {
-      const CbhgDev& D = (g == &h->enc.g_bank) ? h->enc : h->post;
-      pack_gemmw(*g, h->dW, g->bank > 1 ? D.bank_w.data() : &g->w, h->dB + g->bt, 0);
+      g->place(h->dW, bt);
+      bt += bt_elems(g);
+      pack_gemmw(*g, 0);
     }
     CUDA_OK(h, cudaDeviceSynchronize());
     const char* gm = getenv("TACO_GEMM");
@@ -1249,8 +1244,7 @@ int taco_bigru(taco_handle* h, int which, const float* x, const int32_t* lengths
   float* xproj = ws.take<float>((size_t)N * T * 768);
   BfScratch sc;
   if (h->gemm_mode != 0) sc = take_bf(ws, (int64_t)N * T, 128);
-  gemm(c, D.g_xproj, sc, x, (int64_t)T * 128, 128, N, T, c.W(D.gru_bx), nullptr, nullptr, nullptr, 0, 0, xproj,
-       (int64_t)T * 768, 768, 0, TACO_ACT_NONE);
+  run_gemm(c, D.g_xproj, N, T, {x, (int64_t)T * 128, 128, sc}, {TACO_ACT_NONE, c.W(D.gru_bx)}, {xproj, (int64_t)T * 768, 768});
   run_bigru(c, D, xproj, lengths, N, T, out, (int64_t)T * 256);
   return check_launch(h, "bigru");
 }
@@ -1264,42 +1258,33 @@ int taco_conv1d(taco_handle* h, const float* x, int N, int T, int Cin, const flo
   if (!al16(x) || !al16(kernel)) return fail(h, TACO_ERR_INVALID, "x and kernel must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   Ctx c{h, st};
+  GemmIn in{x, (int64_t)T * Cin, Cin, {}};
+  GemmW g;
   if (h->gemm_mode != 0) {   // tensor-core path: pack W^T hi/lo and split x on the device, then one UMMA launch
-    GemmW g = make_gemmw(0, Cout, k, Cin, Cout);
+    g = make_gemmw(0, Cout, k, Cin, Cout);
     const size_t nb = (size_t)g.b_rows * g.Kld, na = (size_t)N * T * g.Cp;
     int rc = ensure_ws(h, sizeof(uint16_t) * 2 * (nb + na) + 65536);
     if (rc) return rc;
     Bump ws(h->ws, h->ws_bytes);
-    uint16_t* bhi = ws.take<uint16_t>(nb);
-    uint16_t* blo = ws.take<uint16_t>(nb);
-    BfScratch sc;
-    sc.hi = ws.take<uint16_t>(na);
-    sc.lo = ws.take<uint16_t>(na);
-    launch_pack_wt(kernel, Cout, k, Cin, Cout, g.Cp, g.Kld, 0, bhi, blo, st);
-    launch_split_bf16(x, (int64_t)T * Cin, Cin, N, T, Cin, g.Cp, sc.hi, sc.lo, st);
-    ConvUmma u;
-    u.a_hi = sc.hi; u.a_lo = sc.lo; u.N = N; u.T = T; u.Cp = g.Cp; u.Cin = g.Cin;
-    u.b_hi = bhi; u.b_lo = blo; u.b_rows = g.b_rows; u.Kld = g.Kld;
-    u.taps = k; u.bank = 1; u.Cout = Cout; u.nsplit = h->gemm_mode == 2 ? 1 : 3;
-    u.bias = bias; u.scale = nullptr; u.shift = nullptr; u.res = nullptr; u.res_bs = 0; u.ldres = 0;
-    u.out = out; u.out_bs = (int64_t)T * Cout; u.ldo = Cout; u.col_off = 0; u.act = act; u.epi = EPI_PLAIN;
-    cudaError_t e = launch_conv_umma(u, st);
-    if (e != cudaSuccess) return fail(h, TACO_ERR_CUDA, std::string("conv_umma launch: ") + cudaGetErrorString(e));
-    h->launches += 3;
-    return check_launch(h, "conv1d");
+    g.w = kernel;
+    g.b_hi = ws.take<uint16_t>(nb);
+    g.b_lo = ws.take<uint16_t>(nb);
+    in.bf = take_bf(ws, (int64_t)N * T, g.Cp);
+    pack_gemmw(g, st);
+    h->launches += 1;
+  } else {
+    g = make_gemmw(0, (Cout + 3) & ~3, k, Cin, Cout);
+    g.w = kernel;
+    if (g.ldw != Cout) {   // pad the leading dimension for 128-bit weight loads
+      int rc = ensure_ws(h, sizeof(float) * (size_t)k * Cin * g.ldw + 65536);
+      if (rc) return rc;
+      CUDA_OK(h, cudaMemsetAsync(h->ws, 0, sizeof(float) * (size_t)k * Cin * g.ldw, st));
+      CUDA_OK(h, cudaMemcpy2DAsync(h->ws, sizeof(float) * g.ldw, kernel, sizeof(float) * Cout, sizeof(float) * Cout,
+                                   (size_t)k * Cin, cudaMemcpyDeviceToDevice, st));
+      g.w = reinterpret_cast<const float*>(h->ws);
+    }
   }
-  const int ldw = (Cout + 3) & ~3;
-  const float* w = kernel;
-  if (ldw != Cout) {   // pad the leading dimension for 128-bit weight loads
-    int rc = ensure_ws(h, sizeof(float) * (size_t)k * Cin * ldw + 65536);
-    if (rc) return rc;
-    CUDA_OK(h, cudaMemsetAsync(h->ws, 0, sizeof(float) * (size_t)k * Cin * ldw, st));
-    CUDA_OK(h, cudaMemcpy2DAsync(h->ws, sizeof(float) * ldw, kernel, sizeof(float) * Cout, sizeof(float) * Cout,
-                                 (size_t)k * Cin, cudaMemcpyDeviceToDevice, st));
-    w = reinterpret_cast<const float*>(h->ws);
-  }
-  conv(c, x, (int64_t)T * Cin, Cin, N, T, Cin, k, w, ldw, bias, nullptr, nullptr, nullptr, 0, 0, out, (int64_t)T * Cout,
-       Cout, 0, Cout, act);
+  run_gemm(c, g, N, T, in, {act, bias}, {out, (int64_t)T * Cout, Cout});
   return check_launch(h, "conv1d");
 }
 
@@ -1333,7 +1318,11 @@ int taco_umma_plan(const taco_gemm_desc* d, int sms, taco_gemm_plan* plan) {
   memset(plan, 0, sizeof(*plan));
   if (!d) return TACO_ERR_INVALID;
   alignas(16) static const float param[4] = {0.f, 0.f, 0.f, 0.f};   // stands for the parameters the library stores aligned
-  *plan = umma_plan(unit_umma(*d, d->bias_host ? param : nullptr, d->scale_host ? param : nullptr, d->shift_host ? param : nullptr), sms);
+  const BfScratch copy{d->out_hi, d->out_lo};
+  *plan = umma_plan(make_umma(unit_gemmw(*d), d->N, d->T, {},
+                              unit_epi(*d, d->bias_host ? param : nullptr, d->scale_host ? param : nullptr, d->shift_host ? param : nullptr),
+                              unit_out(*d, copy), 3),
+                    sms);
   return plan->valid ? TACO_OK : TACO_ERR_INVALID;
 }
 
@@ -1353,23 +1342,13 @@ int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan
   const int gm = h->gemm_mode;
   if (gm == 0 && (presplit || d->out_hi != nullptr || d->out == nullptr))
     return fail(h, TACO_ERR_INVALID, "gemm mode 0 (FFMA) reads and writes fp32 only");
-  const int taps = bank ? d->bank : d->taps, nparam = bank ? d->bank * d->Cout : d->Cout;
-  GemmW g = make_gemmw(0, hw ? 256 : (d->Cout + 3) & ~3, taps, d->Cin, d->Cout, d->bank);
+  const int nparam = bank ? d->bank * d->Cout : d->Cout;
+  GemmW g = unit_gemmw(*d);
   // parameters: staged on the host as taco_finalize_weights stages them, then one copy to the device
   Arena A;
-  std::vector<size_t> w_off(bank ? d->bank : 1);
   size_t b_off = 0, sc_off = 0, sh_off = 0;
-  if (hw) {
-    put_highway(A, d->w_host, d->bias_host, d->w2_host, d->bias2_host, w_off[0], b_off);
-  } else if (bank) {
-    size_t src = 0;
-    for (int ci = 0; ci < d->bank; ++ci) {
-      w_off[ci] = put_matrix(A, d->w_host + src, (ci + 1) * d->Cin, d->Cout, g.ldw);
-      src += (size_t)(ci + 1) * d->Cin * d->Cout;
-    }
-  } else {
-    w_off[0] = put_matrix(A, d->w_host, taps * d->Cin, d->Cout, g.ldw);
-  }
+  if (hw) g.off = put_highway(A, d->w_host, d->bias_host, d->w2_host, d->bias2_host, b_off);
+  else g.off = put_matrix(A, d->w_host, (bank ? d->bank * (d->bank + 1) / 2 : d->taps) * d->Cin, d->Cout, g.ldw);
   if (!hw && d->bias_host) b_off = put_vec(A, d->bias_host, nparam);
   if (d->scale_host) { sc_off = put_vec(A, d->scale_host, nparam); sh_off = put_vec(A, d->shift_host, nparam); }
   const size_t nbt = gm ? (size_t)2 * g.b_rows * g.Kld : 0, na = gm && !presplit ? (size_t)2 * d->N * d->T * g.Cp : 0;
@@ -1386,30 +1365,20 @@ int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan
   const float* bias = d->bias_host ? dP + b_off : nullptr;
   const float* scale = d->scale_host ? dP + sc_off : nullptr;
   const float* shift = d->scale_host ? dP + sh_off : nullptr;
+  g.place(dP, bt);
+  if (gm) {
+    pack_gemmw(g, st);
+    h->launches += g.bank;
+  }
+  if (presplit) sc = {const_cast<void*>(d->x_hi), const_cast<void*>(d->x_lo)};
+  const BfScratch copy{d->out_hi, d->out_lo};
   Ctx c{h, st};
-  if (gm == 0) {   // the fp32 FFMA kernel, one launch per conv as run_cbhg does for a bank
-    for (int ci = 0; ci < (bank ? d->bank : 1); ++ci) {
-      const int o = ci * d->Cout;
-      conv(c, d->x, d->x_bs, d->ldx, d->N, d->T, d->Cin, bank ? ci + 1 : taps, dP + w_off[ci], g.ldw, bias ? bias + o : nullptr,
-           scale ? scale + o : nullptr, shift ? shift + o : nullptr, d->res, d->res_bs, d->ldres, d->out, d->out_bs, d->ldo,
-           d->col_off + o, d->Cout, d->act, d->epi);
-    }
-    return check_launch(h, "gemm unit");
-  }
-  pack_gemmw(g, dP, w_off.data(), bt, st);
-  ConvUmma u = unit_umma(*d, bias, scale, shift);
-  if (!presplit) {
-    launch_split_bf16(d->x, d->x_bs, d->ldx, d->N, d->T, d->Cin, g.Cp, sc.hi, sc.lo, st);
-    u.a_hi = sc.hi; u.a_lo = sc.lo;
-  }
-  u.b_hi = bt; u.b_lo = bt + (size_t)g.b_rows * g.Kld; u.nsplit = gm == 2 ? 1 : 3;
-  taco_gemm_plan q;
-  cudaError_t e = launch_conv_umma(u, st, &q);
+  taco_gemm_plan q = {};
+  const cudaError_t e = run_gemm(c, g, d->N, d->T, {d->x, d->x_bs, d->ldx, sc, presplit}, unit_epi(*d, bias, scale, shift),
+                                 unit_out(*d, copy), &q);
   if (plan) *plan = q;
-  if (e != cudaSuccess)
-    return fail(h, q.valid ? TACO_ERR_CUDA : TACO_ERR_INVALID, std::string("conv_umma launch: ") + cudaGetErrorString(e));
-  h->launches += (bank ? d->bank : 1) + (presplit ? 1 : 2);
-  return check_launch(h, "gemm unit");
+  rc = check_launch(h, "gemm unit");
+  return e != cudaSuccess && !q.valid ? TACO_ERR_INVALID : rc;   // a refused plan is an invalid argument
 }
 
 int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers, const float* w_h_host, const float* b_h_host,
@@ -1424,9 +1393,9 @@ int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers,
   Arena A;
   size_t w_off[4], b_off[4];
   for (int l = 0; l < layers; ++l)
-    put_highway(A, w_h_host + (size_t)l * 128 * 128, b_h_host + (size_t)l * 128, w_t_host + (size_t)l * 128 * 128,
-                b_t_host + (size_t)l * 128, w_off[l], b_off[l]);
-  const GemmW g = make_gemmw(0, 256, 1, 128, 256);
+    w_off[l] = put_highway(A, w_h_host + (size_t)l * 128 * 128, b_h_host + (size_t)l * 128, w_t_host + (size_t)l * 128 * 128,
+                           b_t_host + (size_t)l * 128, b_off[l]);
+  GemmW g = make_gemmw(0, 256, 1, 128, 256);
   const size_t per_layer = (size_t)2 * g.b_rows * g.Kld;   // [hi|lo][256][128]: the layout launch_highway4 reads, layer after layer
   int rc = ensure_ws(h, sizeof(float) * A.buf.size() + sizeof(uint16_t) * per_layer * layers + 65536);
   if (rc) return rc;
@@ -1438,7 +1407,9 @@ int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers,
   CUDA_OK(h, cudaMemcpyAsync(dP, A.buf.data(), sizeof(float) * A.buf.size(), cudaMemcpyHostToDevice, st));
   const float* hb[4] = {nullptr, nullptr, nullptr, nullptr};
   for (int l = 0; l < layers; ++l) {
-    pack_gemmw(g, dP, &w_off[l], bt + per_layer * l, st);
+    g.off = w_off[l];
+    g.place(dP, bt + per_layer * l);
+    pack_gemmw(g, st);
     hb[l] = dP + b_off[l];
   }
   cudaError_t e = launch_highway4(x, out, out_hi, out_lo, bt, hb, layers, rows, h->gemm_mode == 2 ? 1 : 3, st);
