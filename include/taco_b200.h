@@ -304,6 +304,20 @@ int taco_resample_positions(int32_t sr_orig, int32_t sr_new, int64_t t0, int64_t
 int taco_resample(taco_handle* h, int32_t sr_orig, int32_t sr_new, const float* x, const int32_t* lengths_host, int N,
                   int64_t L, float* y, int64_t L_out, void* stream);
 
+/* ---- durations: per-symbol frame counts from a teacher-forced alignment ---------- */
+/* Glow-TTS's monotonic alignment search (monotonic_align.maximum_path: recurrence, band, ties stay) in float64 over
+ * align [N, T_in, steps] (device, dense, as taco_forward / taco_decode write it).  Utterance n has len = text_lengths_host[n]
+ * symbols and F = frames_host[n] target frames (HOST int32), so Y = ceil(F / r) decoder steps (r = hparams
+ * outputs_per_step).  Score s[y][x] = log(max((double)a[n, x, y], 2^-149)); cells max(0, len + y - Y) <= x <= min(len - 1,
+ * y); Q[0][0] = s[0][0], Q[y][x] = s[y][x] + max(Q[y-1][x] (-inf if x == y), Q[y-1][x-1] (-inf if x == 0)); the
+ * backtrack starts at len - 1 on step Y - 1 and moves to x - 1 after step y when x != 0 and (x == y or Q[y-1][x] <
+ * Q[y-1][x-1]).  Step y covers min(r, F - y r) frames; durations_out [N, T_in] int32 (device) gets each symbol's frames
+ * (sum F, each >= 1) and 0 for x >= len.  Rows x >= len and columns y >= Y are not read.  Deterministic (no atomics).
+ * Needs no weights.  TACO_ERR_INVALID: a NULL pointer, N <= 0, steps <= 0, a length outside [1, T_in], frames outside
+ * [1, steps r], or ceil(frames / r) < len (no monotonic path).  TACO_ERR_UNSUPPORTED: T_in > 512 or steps > 65536. */
+int taco_durations(taco_handle* h, const float* align, int N, int T_in, int steps, const int32_t* text_lengths_host,
+                   const int32_t* frames_host, int32_t* durations_out, void* stream);
+
 /* ---- arithmetic mode of the dense layers ----------------------------------- */
 /* The reference computes in fp32.  0 = fp32 FFMA kernels; 1 (default) = tcgen05 tensor
  * cores with every operand split into bf16 hi+lo and three products per k-step

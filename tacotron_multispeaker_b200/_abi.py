@@ -36,7 +36,7 @@ SYMBOLS = [
     "taco_bigru", "taco_conv1d", "taco_maxpool_affine", "taco_bn_batch_stats",
     "taco_set_gemm_mode", "taco_launch_count", "taco_decoder_geometry", "taco_set_decoder_clusters", "taco_set_profiling", "taco_last_stage_ms", "taco_set_cuda_graphs",
     "taco_wav_length", "taco_griffin_lim", "taco_spectrogram_frames", "taco_spectrogram",
-    "taco_resample_length", "taco_resample_positions", "taco_resample",
+    "taco_resample_length", "taco_resample_positions", "taco_resample", "taco_durations",
     "taco_umma_plan", "taco_gemm_unit", "taco_highway4_unit", "taco_bigru_unit", "taco_decoder_plan",
 ]
 
@@ -156,6 +156,7 @@ def load() -> C.CDLL:
     lib.taco_resample_length.restype = i64
     lib.taco_resample_positions.argtypes = [C.c_int32, C.c_int32, i64, i64, vp, vp, vp, vp, vp]
     lib.taco_resample.argtypes = [H, C.c_int32, C.c_int32, fp, C.c_void_p, i, i64, fp, i64, vp]
+    lib.taco_durations.argtypes = [H, fp, i, i, i, C.c_void_p, C.c_void_p, ip, vp]
     lib.taco_umma_plan.argtypes = [C.POINTER(TacoGemmDesc), i, C.POINTER(TacoGemmPlan)]
     lib.taco_gemm_unit.argtypes = [H, C.POINTER(TacoGemmDesc), C.POINTER(TacoGemmPlan), vp]
     lib.taco_highway4_unit.argtypes = [H, fp, i64, i, vp, vp, vp, vp, fp, vp, vp, vp]

@@ -194,4 +194,19 @@ struct ResampleArgs {
 size_t resample_smem_bytes(int span);
 cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t st);
 
+// Per-symbol durations (durations.cu): Glow-TTS's monotonic alignment search over teacher-forced attention, float64
+// scores.  One CTA per utterance, one thread per symbol (blockDim = T_in rounded up to 32); alignment tiles of
+// DUR_TILE steps staged in shared memory.  bits: one backpointer bit per (utterance, step, symbol).
+constexpr int DUR_MAX_T_IN = 512, DUR_MAX_STEPS = 65536, DUR_TILE = 32;
+struct DurationsArgs {
+  const float* align;    // [N][T_in][steps]
+  int N, T_in, steps, r;
+  const int* lengths;    // device [2N]: text lengths, then target frame counts
+  uint32_t* bits;        // [N][y_max][T_in rounded up to 32 / 32] words
+  int y_max;             // the longest utterance's decoder steps, ceil(frames / r)
+  int32_t* out;          // [N][T_in] frames per symbol, 0 past the text length
+};
+size_t durations_bits_bytes(int N, int T_in, int y_max);
+cudaError_t launch_durations(const DurationsArgs& a, cudaStream_t st);
+
 }  // namespace taco

@@ -2049,6 +2049,44 @@ int taco_resample(taco_handle* h, int32_t sr_orig, int32_t sr_new, const float* 
   return check_launch(h, "resample");
 }
 
+// ---- durations: monotonic alignment search over teacher-forced attention ----------------------------------------------
+int taco_durations(taco_handle* h, const float* align, int N, int T_in, int steps, const int32_t* text_lengths_host,
+                   const int32_t* frames_host, int32_t* durations_out, void* stream) {
+  if (!h) return TACO_ERR_INVALID;
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (!align || !text_lengths_host || !frames_host || !durations_out || N <= 0 || T_in <= 0 || steps <= 0)
+    return fail(h, TACO_ERR_INVALID, "durations: bad argument");
+  if (T_in > DUR_MAX_T_IN) return fail(h, TACO_ERR_UNSUPPORTED, "durations: T_in > 512");
+  if (steps > DUR_MAX_STEPS) return fail(h, TACO_ERR_UNSUPPORTED, "durations: steps > 65536");
+  const int64_t r = h->hp.outputs_per_step;
+  std::vector<int32_t> len(2 * (size_t)N);
+  int y_max = 1;
+  for (int i = 0; i < N; ++i) {
+    const int32_t x = text_lengths_host[i], f = frames_host[i];
+    if (x < 1 || x > T_in) return fail(h, TACO_ERR_INVALID, "durations: a text length outside [1, T_in]");
+    if (f < 1 || f > steps * r) return fail(h, TACO_ERR_INVALID, "durations: frames outside [1, steps * r]");
+    const int y = (int)((f + r - 1) / r);
+    if (y < x) return fail(h, TACO_ERR_INVALID, "durations: fewer decoder steps than symbols (no monotonic path)");
+    len[i] = x;
+    len[N + i] = f;
+    y_max = std::max(y_max, y);
+  }
+  const size_t len_bytes = (len.size() * sizeof(int32_t) + 255) & ~size_t(255);
+  int rc = ensure_ws(h, len_bytes + durations_bits_bytes(N, T_in, y_max));
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  CUDA_OK(h, cudaMemcpyAsync(h->ws, len.data(), len.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  DurationsArgs a;
+  a.align = align; a.N = N; a.T_in = T_in; a.steps = steps; a.r = (int)r;
+  a.lengths = reinterpret_cast<const int*>(h->ws);
+  a.bits = reinterpret_cast<uint32_t*>(h->ws + len_bytes);
+  a.y_max = y_max;
+  a.out = durations_out;
+  CUDA_OK(h, launch_durations(a, st));
+  h->launches += 1;
+  return check_launch(h, "durations");
+}
+
 int64_t taco_launch_count(const taco_handle* h) { return h ? h->launches : 0; }
 
 int taco_decoder_geometry(const taco_handle* h, int N, int* cluster_size, int* samples_per_cluster, int* num_clusters) {

@@ -15,6 +15,7 @@
 //   taco_b200::spectrogram(handle, wav, lengths?, T_out?, sample_rate, frame_shift_ms, frame_length_ms, ...)
 //       -> (linear [N,T_out,num_freq], mel [N,T_out,num_mels])
 //   taco_b200::resample(handle, wav, lengths?, orig_sr, target_sr) -> y [N, L_out] (L_out: the longest ceil(len ratio))
+//   taco_b200::durations(handle, align, text_lengths, frames) -> int32 [N, T_in] frames per symbol
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
@@ -230,6 +231,30 @@ at::Tensor resample(int64_t handle, const at::Tensor& wav, at::OptionalIntArrayR
   return y;
 }
 
+// align [N, T_in, steps] on the device; text_lengths / frames host integers [N]
+at::Tensor durations(int64_t handle, const at::Tensor& align, at::IntArrayRef text_lengths, at::IntArrayRef frames) {
+  taco_handle* h = H(handle);
+  dev_f32(align, "align");
+  TORCH_CHECK(align.dim() == 3, "taco_b200::durations: align [N,T_in,steps]");
+  c10::cuda::CUDAGuard guard(align.device());
+  const int64_t N = align.size(0), T_in = align.size(1), steps = align.size(2);
+  TORCH_CHECK((int64_t)text_lengths.size() == N && (int64_t)frames.size() == N, "taco_b200::durations: text_lengths [N], frames [N]");
+  std::vector<int32_t> len, fr;
+  for (int64_t v : text_lengths) {
+    TORCH_CHECK(v >= 1 && v <= T_in, "taco_b200::durations: text_lengths must be in [1, T_in]");
+    len.push_back((int32_t)v);
+  }
+  for (int64_t v : frames) {
+    TORCH_CHECK(v >= 1 && v <= INT32_MAX, "taco_b200::durations: frames must be >= 1");
+    fr.push_back((int32_t)v);
+  }
+  at::Tensor out = at::empty({N, T_in}, align.options().dtype(at::kInt));
+  ck(h, taco_durations(h, align.data_ptr<float>(), (int)N, (int)T_in, (int)steps, len.data(), fr.data(), out.data_ptr<int32_t>(),
+                       stream_of(align)),
+     "durations");
+  return out;
+}
+
 }  // namespace
 
 TORCH_LIBRARY(taco_b200, m) {
@@ -243,6 +268,7 @@ TORCH_LIBRARY(taco_b200, m) {
   m.def("spectrogram(int handle, Tensor wav, int[]? lengths, int? T_out, int sample_rate, float frame_shift_ms, float frame_length_ms, "
         "float min_level_db, float ref_level_db, float preemphasis, int num_mels, int num_freq) -> (Tensor, Tensor)");
   m.def("resample(int handle, Tensor wav, int[]? lengths, int orig_sr, int target_sr) -> Tensor");
+  m.def("durations(int handle, Tensor align, int[] text_lengths, int[] frames) -> Tensor");
 }
 TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("forward", &forward);
@@ -252,4 +278,5 @@ TORCH_LIBRARY_IMPL(taco_b200, CUDA, m) {
   m.impl("griffin_lim", &griffin_lim);
   m.impl("spectrogram", &spectrogram);
   m.impl("resample", &resample);
+  m.impl("durations", &durations);
 }

@@ -373,6 +373,29 @@ class Engine:
                                         self.stream))
         return y[0] if single else (y, out_len)
 
+    def durations(self, align, text_lengths, frames):
+        """Frames per symbol of a teacher-forced alignment ``[N, T_in, steps]`` (``taco_durations``): Glow-TTS's
+        monotonic alignment search in float64 over ``log(max(a, 2^-149))``, ties staying on the same symbol, for
+        utterances of ``text_lengths[n]`` symbols and ``frames[n]`` target frames (``ceil(frames / r)`` decoder steps).
+        Returns a CUDA int32 tensor ``[N, T_in]``: each symbol's frames (they sum to ``frames[n]``, each >= 1), 0 past
+        the text length."""
+        align = self._f32(align)
+        if align.dim() != 3:
+            raise ValueError("align must be [N, T_in, steps]")
+        N, T_in, steps = align.shape
+
+        def host_i32(v):
+            v = v.cpu() if isinstance(v, torch.Tensor) else v
+            v = np.ascontiguousarray(np.asarray(v).reshape(-1), dtype=np.int32)
+            if v.shape != (N,):
+                raise ValueError("text_lengths and frames must be [N]")
+            return v
+        lens, fr = host_i32(text_lengths), host_i32(frames)
+        out = torch.empty(N, T_in, device=self.device, dtype=torch.int32)
+        self._ck(self.lib.taco_durations(self._h, _ptr(align), N, T_in, steps, lens.ctypes.data, fr.ctypes.data, _ptr(out),
+                                         self.stream))
+        return out
+
     def _batch(self, wav, lengths):
         """(wav [N, L] float32 on the device, host int32 lengths [N] or None, whether the input was one 1-D waveform) for
         a waveform, a batch with optional lengths or a list of 1-D waveforms."""

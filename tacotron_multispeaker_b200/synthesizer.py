@@ -28,7 +28,7 @@ import numpy as np
 import torch
 
 from . import audio, plot
-from .engine import pad_targets
+from .engine import pad_inputs, pad_targets
 from .hparams import HParams, hparams as default_hparams
 from .tacotron import create_model
 from .text import sequence_to_text2, text_to_sequence2
@@ -107,6 +107,58 @@ class Synthesizer:
         if path_align is not None:
             plot.plot_alignment(alignment, path_align)
         return self.model.mel_outputs[0].cpu().numpy(), alignment
+
+    def align(self, texts, identities, wavs, orig_sr=None):
+        """Batched teacher forcing of texts with their recordings, and per-symbol durations from the attention.
+        ``wavs`` are read as ``teacher_forced`` reads one (a path through ``audio.load``; an array or tensor, resampled
+        from ``orig_sr`` when given).  The batch's mel targets come from one spectrogram call padded as the feeder pads
+        targets (``max T_n + 1`` frames rounded up to r, zero rows) and feed one teacher-forced forward with the moving
+        statistics of batch norm.  Durations are the monotonic alignment search of ``Engine.durations`` over utterance n's
+        ``len_n`` symbols and ``1 + L_n // hop`` frames.  Returns, in input order, ``(durations int32 [len_n], alignment
+        float32 [len_n, Y_n])`` numpy pairs with ``Y_n = ceil(frames_n / r)`` decoder steps.
+
+        Attention is not length-masked (reference ``tacotron.py:68``), so a text padded to the batch's longest one
+        attends to the padding too and its alignment differs from a batch of its own -- as in the reference's training
+        graph.  ``align`` keeps the given order and does not re-bucket.  Raises ``ValueError`` naming the utterance for a
+        text longer than 512 symbols, a recording longer than max_iters * r frames (``load`` sets max_iters = 400), or
+        fewer decoder steps than symbols."""
+        hp = self.hparams
+        r = hp.outputs_per_step
+        if not len(texts) == len(identities) == len(wavs) or not texts:
+            raise ValueError("align needs as many identities and recordings as texts, and at least one")
+        cleaners = [x.strip() for x in hp.cleaners.split(",")]
+        seqs = [np.asarray(text_to_sequence2(t, cleaners)[:-1], np.int32) for t in texts]
+        for i, s in enumerate(seqs):
+            if not 1 <= s.size <= 512:
+                raise ValueError("utterance %d: a text of %d symbols (align takes 1 to 512)" % (i, s.size))
+        engine = self.model._get_engine(self.id_num if self.id_num > 1 else 0)
+        ys = []
+        for w in wavs:
+            if isinstance(w, (str, bytes)) or hasattr(w, "__fspath__"):
+                w = audio.load(engine, w, hp.sample_rate)
+            elif orig_sr is not None:
+                w = audio.resample(engine, torch.as_tensor(w).reshape(-1), orig_sr, hp.sample_rate)
+            ys.append(engine._f32(w).reshape(-1))
+        frames = [engine.spectrogram_frames(y.numel()) for y in ys]
+        for i, (s, f) in enumerate(zip(seqs, frames)):
+            if f > hp.max_iters * r:
+                raise ValueError("utterance %d: %d frames, more than max_iters * r = %d (load sets max_iters = 400)"
+                                 % (i, f, hp.max_iters * r))
+            if -(-f // r) < s.size:
+                raise ValueError("utterance %d: %d decoder steps for %d symbols" % (i, -(-f // r), s.size))
+        N = len(ys)
+        wav = torch.zeros(N, max(y.numel() for y in ys), device=engine.device, dtype=torch.float32)
+        for i, y in enumerate(ys):
+            wav[i, :y.numel()] = y
+        T_out = -(-(max(frames) + 1) // r) * r                     # pad_targets' length
+        _, mel = engine.spectrogram(wav, lengths=[y.numel() for y in ys], T_out=T_out)
+        lengths = np.asarray([s.size for s in seqs], np.int32)
+        _, _, al, _ = engine.forward(pad_inputs(seqs), lengths, np.asarray(identities, np.int32), mel, teacher_force=True,
+                                     want_linear=False)
+        engine.check_ids()
+        dur = engine.durations(al, lengths, frames).cpu().numpy()
+        al = al.cpu().numpy()
+        return [(dur[i, :s.size], al[i, :s.size, :-(-f // r)]) for i, (s, f) in enumerate(zip(seqs, frames))]
 
     def synthesize(self, text, identity, path=None, path_align=None):
         seq = text_to_sequence2(text, [x.strip() for x in self.hparams.cleaners.split(",")])[:-1]
