@@ -186,27 +186,22 @@ int taco_bn_batch_stats(taco_handle* h, const float* x, int N, int T, int C, con
 /* One conv1d('same') / dense layer with the whole epilogue of the forward's GEMMs:
  *   out[n, t, col_off + o] = act(sum_{j, c} x[n, t + j - (taps-1)/2, c] w[j, c, o] + bias[o]) * scale[o] + shift[o] + res[n, t, o]
  * (rows outside [0, T) read as zero).  bank > 1: `bank` convolutions of Cout channels side by side, conv ci with ci + 1 taps,
- * its outputs at columns col_off + ci Cout (the CBHG conv bank, modules.py:39-42).  epi = TACO_EPI_HIGHWAY: Cout = 2 x channels,
- * out[n, t, col_off + c] = relu(H_c) T_c + res[n, t, c] (1 - T_c), T_c = sigmoid(., modules.py:79-89).
+ * its outputs at columns col_off + ci Cout (the CBHG conv bank, modules.py:39-42).
  * Parameters are HOST float32 in the reference layouts, copied per call. */
-enum { TACO_EPI_PLAIN = 0, TACO_EPI_HIGHWAY = 1 };
 typedef struct taco_gemm_desc {
   /* A operand: device fp32 x[n x_bs + t ldx + c], or (x_hi, x_lo) already split into bf16 hi / lo [N][T][Cp] with
    * Cp = Cin rounded up to 64 (what out_hi / out_lo of a previous call wrote); x is then not read */
   const float* x; int64_t x_bs; int32_t ldx;
   const void* x_hi; const void* x_lo;
   int32_t N, T, Cin, taps, bank, Cout;
-  const float* w_host;      /* [taps, Cin, Cout]; bank: the kernels [ci + 1, Cin, Cout], ci = 0 .. bank-1, back to back;
-                               highway: W_H [Cin, Cout / 2] */
-  const float* w2_host;     /* highway: W_T [Cin, Cout / 2]; else NULL */
-  const float* bias_host;   /* [Cout] (bank: [bank Cout]) or NULL; highway: b_H [Cout / 2] */
-  const float* bias2_host;  /* highway: b_T [Cout / 2] */
+  const float* w_host;      /* [taps, Cin, Cout]; bank: the kernels [ci + 1, Cin, Cout], ci = 0 .. bank-1, back to back */
+  const float* bias_host;   /* [Cout] (bank: [bank Cout]) or NULL */
   const float* scale_host; const float* shift_host;   /* affine after the activation ([Cout], bank: [bank Cout]) or NULL */
-  const float* res; int64_t res_bs; int32_t ldres;    /* device residual (plain) / carry input (highway), or NULL */
-  int32_t act, epi;         /* TACO_ACT_*, TACO_EPI_* */
+  const float* res; int64_t res_bs; int32_t ldres;    /* device residual, or NULL */
+  int32_t act;              /* TACO_ACT_* */
   float* out; int64_t out_bs; int32_t ldo, col_off;   /* device; NULL when only the bf16 copy is wanted */
   void* out_hi; void* out_lo; int32_t out_cp;         /* optional bf16 hi / lo copy of the result [N][T][out_cp], channels
-                                                         Cout .. out_cp-1 zero (out_cp % 64 == 0; plain epilogue, no bank) */
+                                                         Cout .. out_cp-1 zero (out_cp % 64 == 0; no bank) */
 } taco_gemm_desc;
 /* How the tensor-core kernel runs a GEMM: */
 typedef struct taco_gemm_plan {
@@ -219,20 +214,20 @@ typedef struct taco_gemm_plan {
   int32_t epi_warps;     /* 4 or 8 */
   int32_t acc_cols;      /* tensor-memory columns: 256 = two accumulators alternating across tiles, 128 = one */
   int32_t vec_epi;       /* 1: 128-bit epilogue loads / stores; 0: scalar (rows not 16-byte aligned) */
-  int32_t variant;       /* compiled epilogue: 0 any (run time), 1 bias, 2 relu, 3 relu + affine, 4 affine + residual, 5 highway */
+  int32_t variant;       /* compiled epilogue: 0 any (run time), 1 bias, 2 relu, 3 relu + affine, 4 affine + residual */
   int32_t smem_bytes;
 } taco_gemm_plan;
 /* The plan the tensor-core GEMM `d` gets on a device with `sms` SMs.  Reads the shape, the flags and only whether each
  * pointer is NULL and 16-byte aligned (the parameters count as aligned: the library stores them so).  No device needed.
  * TACO_ERR_INVALID (plan->valid = 0) when the launch would be refused. */
 int taco_umma_plan(const taco_gemm_desc* d, int sms, taco_gemm_plan* plan);
-/* Runs `d` in the handle's gemm mode: the fp32 FFMA kernel (mode 0: no split operand in or out) or the tensor-core kernel
- * (1 / 2: three / one bf16 products per k-step); writes the plan it used to *plan (NULL allowed; valid = 0 in mode 0). */
+/* Runs `d` on the tensor-core kernel in the handle's gemm mode (1 / 2: three / one bf16 products per k-step); writes the
+ * plan it used to *plan (NULL allowed). */
 int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan, void* stream);
 /* The fused highway layers of a CBHG: `layers` (1..4) times y = relu(x W_H + b_H) T + x (1 - T), T = sigmoid(x W_T + b_T),
  * on x [rows][128] (device, dense).  W_H / W_T: HOST [layers][128][128], b_H / b_T: HOST [layers][128].  out [rows][128]
- * and / or the bf16 hi / lo copy out_hi / out_lo [rows][128] (device, NULL to skip).  Tensor-core gemm modes only (nsplit
- * 3 in mode 1, 1 in mode 2); TACO_ERR_UNSUPPORTED in mode 0. */
+ * and / or the bf16 hi / lo copy out_hi / out_lo [rows][128] (device, NULL to skip).  Three bf16 products per k-step in
+ * gemm mode 1, one in mode 2. */
 int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers, const float* w_h_host,
                        const float* b_h_host, const float* w_t_host, const float* b_t_host, float* out, void* out_hi,
                        void* out_lo, void* stream);
@@ -319,13 +314,13 @@ int taco_durations(taco_handle* h, const float* align, int N, int T_in, int step
                    const int32_t* frames_host, int32_t* durations_out, void* stream);
 
 /* ---- arithmetic mode of the dense layers ----------------------------------- */
-/* The reference computes in fp32.  0 = fp32 FFMA kernels; 1 (default) = tcgen05 tensor
- * cores with every operand split into bf16 hi+lo and three products per k-step
- * (fp32-class accuracy, meets the 1e-3 parity bound); 2 = plain bf16 operands with fp32
- * accumulation in the dense layers AND in the decoder loop's mat-vecs (one product per
- * k-step instead of three; separately stated tolerance 5e-2, tests/test_gpu_parity.py).
+/* The reference computes in fp32.  1 (default) = tcgen05 tensor cores with every operand
+ * split into bf16 hi+lo and three products per k-step (fp32-class accuracy, meets the 1e-3
+ * parity bound); 2 = plain bf16 operands with fp32 accumulation in the dense layers AND in
+ * the decoder loop's mat-vecs (one product per k-step instead of three; separately stated
+ * tolerance 5e-2, tests/test_gpu_parity.py).  Any other mode: TACO_ERR_INVALID.
  * The BiGRU recurrences always run in fp32. */
-enum { TACO_GEMM_FFMA = 0, TACO_GEMM_BF16X3 = 1, TACO_GEMM_BF16 = 2 };
+enum { TACO_GEMM_BF16X3 = 1, TACO_GEMM_BF16 = 2 };
 int taco_set_gemm_mode(taco_handle* h, int mode);
 
 /* ---- introspection for bench / tests ------------------------------------- */

@@ -23,8 +23,7 @@ TACO_ERR_UNSUPPORTED = -6
 BN_MOVING, BN_BATCH = 0, 1
 ACT_NONE, ACT_RELU, ACT_SIGMOID, ACT_TANH = 0, 1, 2, 3
 CBHG_ENCODER, CBHG_POST = 0, 1
-GEMM_FFMA, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
-EPI_PLAIN, EPI_HIGHWAY = 0, 1
+GEMM_BF16X3, GEMM_BF16 = 1, 2
 
 # Every symbol include/taco_b200.h declares (tests check the library exports all of them).
 SYMBOLS = [
@@ -64,10 +63,10 @@ class TacoGemmDesc(C.Structure):
         ("x_hi", C.c_void_p), ("x_lo", C.c_void_p),
         ("N", C.c_int32), ("T", C.c_int32), ("Cin", C.c_int32), ("taps", C.c_int32), ("bank", C.c_int32),
         ("Cout", C.c_int32),
-        ("w_host", C.c_void_p), ("w2_host", C.c_void_p), ("bias_host", C.c_void_p), ("bias2_host", C.c_void_p),
+        ("w_host", C.c_void_p), ("bias_host", C.c_void_p),
         ("scale_host", C.c_void_p), ("shift_host", C.c_void_p),
         ("res", C.c_void_p), ("res_bs", C.c_int64), ("ldres", C.c_int32),
-        ("act", C.c_int32), ("epi", C.c_int32),
+        ("act", C.c_int32),
         ("out", C.c_void_p), ("out_bs", C.c_int64), ("ldo", C.c_int32), ("col_off", C.c_int32),
         ("out_hi", C.c_void_p), ("out_lo", C.c_void_p), ("out_cp", C.c_int32),
     ]

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtaco_b200.so")
 OBJ_DIR = os.path.join(CSRC, "build")
 
-SOURCES = ["gather.cu", "conv_gemm.cu", "conv_umma.cu", "elementwise.cu", "bigru.cu", "bigru_mma.cu", "decoder.cu", "decoder_cw.cu", "griffin_lim.cu", "spectrogram.cu", "resample.cu", "durations.cu", "taco_abi.cu"]
+SOURCES = ["gather.cu", "conv_umma.cu", "elementwise.cu", "bigru.cu", "bigru_mma.cu", "decoder.cu", "decoder_cw.cu", "griffin_lim.cu", "spectrogram.cu", "resample.cu", "durations.cu", "taco_abi.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", "fft2048.cuh", "decoder_cw.h", "decoder_cw_pack.inc", os.path.join("..", "..", "include", "taco_b200.h")]
 
 NVCC_FLAGS = [

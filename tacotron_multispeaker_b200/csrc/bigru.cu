@@ -3,7 +3,7 @@
 // Replaces tf.nn.bidirectional_dynamic_rnn(GRUCell(128), GRUCell(128), x,
 // sequence_length) at reference models/modules.py:68-74 (a tf.while_loop of
 // T_in resp. T_out=1000 iterations per direction).  The input halves of the
-// GRU kernels are hoisted into one dense GEMM (xproj, conv_gemm.cu); what is
+// GRU kernels are hoisted into one dense GEMM (xproj, conv_umma.cu); what is
 // left per step and direction is
 //     [r|u] = sigmoid(xg_t + h U_g)      U_g [128,256]
 //     c     = tanh  (xc_t + (r*h) U_c)   U_c [128,128]   (reset BEFORE matmul: TF GRUCell)

@@ -1,7 +1,7 @@
 // conv1d('same') / dense as a TMA-fed tcgen05 implicit GEMM (sm_100a).
 //
-// Same operator as conv_gemm.cu (reference models/modules.py:93-101, :10,
-// :59-60, :79-89, models/tacotron.py:68,101) on the 5th-generation tensor
+// The dense and conv1d layers of the reference (models/modules.py:93-101, :10,
+// :59-60, models/tacotron.py:68,101) on the 5th-generation tensor
 // cores.  D[128 rows (n, t0..t0+127)] x [128 output channels] accumulates in
 // TMEM (fp32) over k-blocks of 64 input channels per filter tap:
 //
@@ -18,8 +18,8 @@
 //
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = MMA issuer (one
 // elected thread), warps 2..5 = epilogue (TMEM -> registers -> smem transpose
-// -> coalesced global stores, with bias / activation / folded BN / residual /
-// highway gate).  3-stage smem ring (64 KB per stage) with full/empty
+// -> coalesced global stores, with bias / activation / folded BN /
+// residual).  3-stage smem ring (64 KB per stage) with full/empty
 // mbarriers; tcgen05.commit releases stages and signals the epilogue.
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -55,7 +55,7 @@ struct UmmaArgs {
   const float* res; long long res_bs; int ldres;
   float* out; long long out_bs; int ldo; int col_off;
   void* out_hi; void* out_lo; int out_cp;   // bf16 hi / lo copy of the result [N][T][out_cp] (null: none)
-  int act, epi;
+  int act;
   int stages;              // smem ring depth (1..3)
   int vec_epi;             // 1: rows are 16 B aligned -> direct 128-bit stores from the TMEM registers
   int nx, ny, ntiles;      // tile list: nx = N * ceil(T / 128) row tiles, ny column tiles, ntiles = nx * ny * bank
@@ -284,89 +284,6 @@ __device__ __forceinline__ void epi_plain_scalar(const UmmaArgs& p, const EpiTil
   }
 }
 
-// Highway gate (modules.py:79-89): GEMM columns (2c, 2c+1) = (H_c, T_c); out_c = relu(H_c) T + x_c (1 - T), T = sigmoid(T_c).
-__device__ __forceinline__ void epi_highway_vec(const UmmaArgs& p, const EpiTile& e, float* stg, uint32_t acc, int ch_lo, int ch_hi, int lane) {
-#pragma unroll 1
-  for (int ch = ch_lo; ch < ch_hi; ++ch) {
-    const int cbase = e.o0 + ch * 32;
-    if (cbase >= p.Cout) break;
-    uint32_t v[32];
-    tmem_ld32(acc + (uint32_t)(ch * 32), v);
-    // staged per row: a_c = relu(H_c) * sigmoid(T_c) at floats 0..15, b_c = 1 - sigmoid(T_c) at floats 16..31
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      const int colb = cbase + 8 * g;
-      const bool bok = colb < p.Cout;                                     // Cout % 8 == 0 on this path
-      const float4 b0 = bok ? ldg_f4(e.bias + colb) : make_float4(0.f, 0.f, 0.f, 0.f);
-      const float4 b1 = bok ? ldg_f4(e.bias + colb + 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-      const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-      float a4[4], g4[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const int c2 = 8 * g + 2 * k;
-        const float H = fmaxf(__uint_as_float(v[c2]) + bb[2 * k], 0.f), Tg = sigmoid_f(__uint_as_float(v[c2 + 1]) + bb[2 * k + 1]);
-        a4[k] = H * Tg; g4[k] = 1.0f - Tg;
-      }
-      *reinterpret_cast<float4*>(stg + lane * EPI_LD + 4 * g) = make_float4(a4[0], a4[1], a4[2], a4[3]);
-      *reinterpret_cast<float4*>(stg + lane * EPI_LD + 16 + 4 * g) = make_float4(g4[0], g4[1], g4[2], g4[3]);
-    }
-    __syncwarp();
-    const int chn0 = cbase >> 1;                                          // first of the 16 output channels of this chunk
-    const int rs2 = lane >> 2, q4 = lane & 3;                             // row 8 i + rs2, channels chn0 + 4 q4 ..
-    const bool cok = cbase + 8 * q4 < p.Cout;
-    const int rows_left = p.T - e.tq - rs2;
-    const float* rrow = p.res + (long long)e.n * p.res_bs + (long long)(e.tq + rs2) * p.ldres + chn0 + 4 * q4;
-    float* orow = p.out + (long long)e.n * p.out_bs + (long long)(e.tq + rs2) * p.ldo + e.col_off + chn0 + 4 * q4;
-    float4 xin[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (cok && 8 * i < rows_left) xin[i] = ldg_f4(rrow + (8 * i) * p.ldres);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = 8 * i + rs2;
-      const float4 av = *reinterpret_cast<const float4*>(stg + r * EPI_LD + 4 * q4);
-      const float4 gv = *reinterpret_cast<const float4*>(stg + r * EPI_LD + 16 + 4 * q4);
-      if (cok && 8 * i < rows_left)
-        *reinterpret_cast<float4*>(orow + (8 * i) * p.ldo) =
-            make_float4(fmaf(xin[i].x, gv.x, av.x), fmaf(xin[i].y, gv.y, av.y), fmaf(xin[i].z, gv.z, av.z), fmaf(xin[i].w, gv.w, av.w));
-    }
-    __syncwarp();
-  }
-}
-__device__ __forceinline__ void epi_highway_scalar(const UmmaArgs& p, const EpiTile& e, float* stg, uint32_t acc, int ch_lo, int ch_hi, int lane) {
-  constexpr int LD = 33;
-#pragma unroll 1
-  for (int ch = ch_lo; ch < ch_hi; ++ch) {
-    const int cbase = e.o0 + ch * 32;
-    if (cbase >= p.Cout) break;
-    uint32_t v[32];
-    tmem_ld32(acc + (uint32_t)(ch * 32), v);
-#pragma unroll
-    for (int c = 0; c < 32; ++c) stg[lane * LD + c] = __uint_as_float(v[c]);
-    __syncwarp();
-    const int col = cbase + lane;                                         // even lane = H_c, odd lane = T_c of channel c = col / 2
-    const bool cok = col < p.Cout;
-    const float b = cok ? __ldg(e.bias + col) : 0.f;
-    const int rmax = min(32, p.T - e.tq);
-    const int chn = col >> 1;
-    float* optr = p.out + (long long)e.n * p.out_bs + (long long)e.tq * p.ldo + e.col_off + chn;
-    const float* rptr = p.res + (long long)e.n * p.res_bs + (long long)e.tq * p.ldres + chn;
-#pragma unroll 4
-    for (int r = 0; r < rmax; ++r) {
-      const float x = stg[r * LD + lane] + b;
-      const float tg = __shfl_down_sync(0xffffffffu, x, 1);
-      if (cok && !(lane & 1)) {
-        const float H = fmaxf(x, 0.f), Tg = sigmoid_f(tg);
-        const float xin = __ldg(rptr);
-        *optr = H * Tg + xin * (1.0f - Tg);
-      }
-      optr += p.ldo;
-      rptr += p.ldres;
-    }
-    __syncwarp();
-  }
-}
-
 template <int NSPLIT, int EV>
 __global__ void __launch_bounds__(NTHREADS_MAX, 2)
 conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
@@ -505,15 +422,10 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       e.shift = p.shift ? p.shift + q.ci * p.Cout : nullptr;
       e.col_off = p.col_off + q.ci * p.Cout;
       // EV: the launch's epilogue variant, compiled in (0 = any combination, decided at run time)
-      if (EV == 5) {
-        if (p.vec_epi) epi_highway_vec(p, e, stg, acc, ch_lo, ch_hi, lane);
-        else epi_highway_scalar(p, e, stg, acc, ch_lo, ch_hi, lane);
-      } else {
-        constexpr int A = EV == 0 ? 2 : ((EV == 2 || EV == 3) ? 1 : 0);
-        constexpr bool S = EV == 0 || EV == 3 || EV == 4, R = EV == 0 || EV == 4;
-        if (p.vec_epi) epi_plain_vec<A, S, R>(p, e, stg, acc, ch_lo, ch_hi, lane);
-        else epi_plain_scalar<A, S, R>(p, e, stg, acc, ch_lo, ch_hi, lane);
-      }
+      constexpr int A = EV == 0 ? 2 : ((EV == 2 || EV == 3) ? 1 : 0);
+      constexpr bool S = EV == 0 || EV == 3 || EV == 4, R = EV == 0 || EV == 4;
+      if (p.vec_epi) epi_plain_vec<A, S, R>(p, e, stg, acc, ch_lo, ch_hi, lane);
+      else epi_plain_scalar<A, S, R>(p, e, stg, acc, ch_lo, ch_hi, lane);
       // this warp has read its lanes of the accumulator: hand the buffer back to the MMA issuer
       tc_fence_before();
       __syncwarp();
@@ -863,7 +775,7 @@ int env_int(const char* name, int dflt) { const char* e = getenv(name); return e
 // Launch shapes (developer switches read once: TACO_UMMA_PERSISTENT = 0 / 1 forces, TACO_UMMA_EW, TACO_UMMA_STAGES_MAX, TACO_UMMA_CTAS):
 //  * long K (>= 24 k-blocks: the 3 x 1024 -> 256 projection, the conv banks): bound by loads and MMAs.  Persistent CTAs, one per
 //    SM, three 64 KB stages, two TMEM accumulators (the epilogue of tile i overlaps the main loop of tile i+1), 4 epilogue warps.
-//  * short K with more than two tiles per SM (the 1025-wide linear output, highway layers at full length): bound by the
+//  * short K with more than two tiles per SM (the 1025-wide linear output, the GRU input projections at full length): bound by the
 //    epilogue.  Persistent as well, but with EIGHT epilogue warps and two stages.
 //  * few tiles: one tile per CTA, eight epilogue warps, a shallow ring so that two CTAs share an SM.
 // Reads only the shape, the flags and whether each pointer is null or 16-byte aligned: no device access.
@@ -892,9 +804,8 @@ taco_gemm_plan umma_plan(const ConvUmma& c, int sms) {
   if (nctas > q.tiles) nctas = q.tiles;
   q.ctas = nctas;
   q.acc_cols = nctas < q.tiles ? 256 : 128;
-  const int chn = c.epi == EPI_HIGHWAY ? 2 : 1;
   auto al4 = [](long long v) { return (v & 3) == 0; };
-  q.vec_epi = (al4(c.ldo) && al4(c.col_off) && al4(c.out_bs) && al4(c.Cout / chn) && (c.Cout % (4 * chn) == 0) &&
+  q.vec_epi = (al4(c.ldo) && al4(c.col_off) && al4(c.out_bs) && al4(c.Cout) &&
                (c.out == nullptr || (reinterpret_cast<uintptr_t>(c.out) & 15) == 0) &&
                (c.res == nullptr || (al4(c.ldres) && al4(c.res_bs) && (reinterpret_cast<uintptr_t>(c.res) & 15) == 0)) &&
                (c.bias == nullptr || (reinterpret_cast<uintptr_t>(c.bias) & 15) == 0) &&
@@ -902,14 +813,12 @@ taco_gemm_plan umma_plan(const ConvUmma& c, int sms) {
                   ? 1 : 0;
   q.smem_bytes = (int)smem_bytes(q.stages, q.epi_warps);
   // epilogue variant: the combinations the forward uses are compiled in, anything else takes the run-time variant 0
-  if (c.epi == EPI_HIGHWAY) q.variant = 5;
-  else if (c.act == 0 && !c.scale && !c.res) q.variant = 1;
+  if (c.act == 0 && !c.scale && !c.res) q.variant = 1;
   else if (c.act == 1 && !c.scale && !c.res) q.variant = 2;
   else if (c.act == 1 && c.scale && !c.res) q.variant = 3;
   else if (c.act == 0 && c.scale && c.res) q.variant = 4;
   // refusals
-  if (c.epi == EPI_HIGHWAY && (c.bias == nullptr || c.res == nullptr)) return q;
-  if (c.out_hi != nullptr && (c.out_lo == nullptr || !q.vec_epi || c.epi != EPI_PLAIN || c.bank > 1 || c.col_off != 0 || (c.out_cp & 63) ||
+  if (c.out_hi != nullptr && (c.out_lo == nullptr || !q.vec_epi || c.bank > 1 || c.col_off != 0 || (c.out_cp & 63) ||
                               c.out_cp < c.Cout || c.out_cp > ny * BN))
     return q;
   if (c.out == nullptr && c.out_hi == nullptr) return q;
@@ -939,7 +848,7 @@ cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st, taco_gemm_plan*
   UmmaArgs p;
   p.N = c.N; p.T = c.T; p.Cp = c.Cp; p.kvalid = c.Cin > 0 && c.Cin < c.Cp ? (c.Cin + 15) & ~15 : c.Cp; p.taps = c.taps; p.bank = c.bank; p.Cout = c.Cout;
   p.bias = c.bias; p.scale = c.scale; p.shift = c.shift; p.res = c.res; p.res_bs = c.res_bs; p.ldres = c.ldres;
-  p.out = c.out; p.out_bs = c.out_bs; p.ldo = c.ldo; p.col_off = c.col_off; p.act = c.act; p.epi = c.epi;
+  p.out = c.out; p.out_bs = c.out_bs; p.ldo = c.ldo; p.col_off = c.col_off; p.act = c.act;
   p.out_hi = c.out_hi; p.out_lo = c.out_lo; p.out_cp = c.out_cp;
   p.nx = c.N * ((c.T + BM - 1) / BM);
   p.ny = (c.Cout + BN - 1) / BN;
@@ -947,14 +856,14 @@ cudaError_t launch_conv_umma(const ConvUmma& c, cudaStream_t st, taco_gemm_plan*
   p.epi_warps = q.epi_warps; p.stages = q.stages; p.acc_cols = q.acc_cols; p.vec_epi = q.vec_epi;
   dim3 grid(q.ctas, 1, 1);
   using KernelFn = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const UmmaArgs);
-  static const KernelFn kernels[2][6] = {
-      {conv_umma_kernel<3, 0>, conv_umma_kernel<3, 1>, conv_umma_kernel<3, 2>, conv_umma_kernel<3, 3>, conv_umma_kernel<3, 4>, conv_umma_kernel<3, 5>},
-      {conv_umma_kernel<1, 0>, conv_umma_kernel<1, 1>, conv_umma_kernel<1, 2>, conv_umma_kernel<1, 3>, conv_umma_kernel<1, 4>, conv_umma_kernel<1, 5>}};
+  static const KernelFn kernels[2][5] = {
+      {conv_umma_kernel<3, 0>, conv_umma_kernel<3, 1>, conv_umma_kernel<3, 2>, conv_umma_kernel<3, 3>, conv_umma_kernel<3, 4>},
+      {conv_umma_kernel<1, 0>, conv_umma_kernel<1, 1>, conv_umma_kernel<1, 2>, conv_umma_kernel<1, 3>, conv_umma_kernel<1, 4>}};
   static bool attr_done[64] = {false};
   bool& attr_set = attr_done[dev & 63];
   if (!attr_set) {
     for (int a = 0; a < 2; ++a)
-      for (int b = 0; b < 6; ++b) {
+      for (int b = 0; b < 5; ++b) {
         cudaError_t e1 = cudaFuncSetAttribute(kernels[a][b], cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e1 != cudaSuccess) return e1;
       }

@@ -15,25 +15,11 @@ void launch_gather_concat(const int32_t* ids, const int32_t* spk, const float* t
                           const float* spk_table, int S, int Es, int N, int T, float* out,
                           int* oob_flag, cudaStream_t st);
 
-// ---- conv1d-as-GEMM (conv_gemm.cu) -----------------------------------------
-// out[n,t,col_off+o] = epi( sum_{j<k, c<Cin} x[n, t+j-pl, c] * w[(j*Cin+c)*ldw + o] ),  pl=(k-1)/2,
-// rows outside [0,T) read as zero (tf 'same' padding).  k=1 is a dense layer.
-enum { EPI_PLAIN = 0, EPI_HIGHWAY = 1 };
-struct ConvGemm {
-  const float* x; int64_t x_bs; int ldx;   // x[n*x_bs + t*ldx + c]
-  int N, T, Cin, k;
-  const float* w; int ldw;                  // ldw % 4 == 0
-  const float* bias;                        // [Cout] or null
-  const float* scale; const float* shift;   // per-channel affine after the activation, or null
-  const float* res; int64_t res_bs; int ldres;  // residual (PLAIN) / carry input (HIGHWAY), or null
-  float* out; int64_t out_bs; int ldo; int col_off;
-  int Cout;                                 // GEMM columns (HIGHWAY: 2*channels, interleaved H,T)
-  int act; int epi;
-};
-void launch_conv_gemm(const ConvGemm& p, cudaStream_t st);
-
 // ---- conv1d-as-GEMM on tcgen05 tensor cores (conv_umma.cu) -------------------
-// Same operator as ConvGemm with bf16 operands staged by TMA (fp32 accumulate in TMEM).
+// out[n,t,col_off+o] = epi( sum_{j<taps, c<Cin} x[n, t+j-pl, c] * w[j, c, o] ),  pl=(taps-1)/2,
+// rows outside [0,T) read as zero (tf 'same' padding); taps=1 is a dense layer.  epi: act(. + bias), then the
+// per-channel affine scale / shift, then the residual res (each optional).  bf16 operands staged by TMA, fp32
+// accumulate in TMEM.
 // a_hi/a_lo: activations split into bf16 hi+lo, dense [N][T][Cp] (Cp % 64 == 0, zero padded);
 // b_hi/b_lo: W^T split likewise, [b_rows][Kld] with Kld = taps*Cp (K contiguous).
 // nsplit = 3: hi*hi + hi*lo + lo*hi (fp32-class accuracy); nsplit = 1: plain bf16 (lo unused).
@@ -48,9 +34,9 @@ struct ConvUmma {
   const float* bias; const float* scale; const float* shift;
   const float* res; int64_t res_bs; int ldres;
   float* out; int64_t out_bs; int ldo; int col_off;   // out may be null when only the bf16 copy below is wanted
-  int act, epi;
+  int act;
   // optional: the result also (or only) as the bf16 hi / lo operand of the GEMM that consumes it, dense [N][T][out_cp] with the
-  // channels Cout .. out_cp-1 written as zeros (out_cp % 64 == 0); plain epilogue, 16-byte aligned rows, no bank, col_off 0
+  // channels Cout .. out_cp-1 written as zeros (out_cp % 64 == 0); 16-byte aligned rows, no bank, col_off 0
   void* out_hi = nullptr; void* out_lo = nullptr; int out_cp = 0;
 };
 // The launch shape of a ConvUmma on `sms` SMs (include/taco_b200.h, taco_gemm_plan); valid == 0: the launch is refused.

@@ -36,8 +36,8 @@ struct HostVar {
   bool set = false;
 };
 
-// One GEMM-shaped weight: fp32 [taps*Cin][ldw] for the FFMA path and W^T split into bf16 hi/lo
-// ([b_rows][Kld], K contiguous) for the tcgen05 path.  A bank holds its convolutions back to back: conv ci has ci+1 taps,
+// One GEMM-shaped weight: fp32 [taps*Cin][ldw], and W^T split into bf16 hi/lo ([b_rows][Kld], K contiguous) for the
+// tcgen05 kernel, packed from the fp32 weights.  A bank holds its convolutions back to back: conv ci has ci+1 taps,
 // its fp32 rows [(ci+1)*Cin][ldw] start at row Cin*ci*(ci+1)/2 and its W^T rows are [ci*Cout, (ci+1)*Cout).
 struct GemmW {
   size_t off = 0;                      // float offset of the fp32 weights in the staging arena, until w points at the upload
@@ -94,7 +94,7 @@ struct taco_handle {
   int emb_dim = 0;
   GemmW g_pre1, g_pre2, g_mem, g_lin;
   uint16_t* dB = nullptr;              // bf16 arena: W^T hi/lo for the tensor-core path
-  int gemm_mode = 1;                   // 0 = fp32 FFMA, 1 = bf16x3 tcgen05 (fp32-class), 2 = bf16 tcgen05
+  int gemm_mode = 1;                   // 1 = bf16x3 tcgen05 (fp32-class), 2 = bf16 tcgen05
   CbhgDev enc, post;
   DecoderWeights dec[2];               // slices cut for clusters of 8 ([0]) and 16 ([1]) CTAs
   int max_clusters[2] = {0, 0};        // co-resident clusters of each size on this device
@@ -168,7 +168,7 @@ int fail(taco_handle* h, int code, const std::string& msg) {
   if (h) h->err = msg;
   return code;
 }
-// The GEMM operand split (split_bf16_kernel), the FFMA conv and the decoder read activations with 16-byte vector loads at
+// The GEMM operand split (split_bf16_kernel) and the decoder read activations with 16-byte vector loads at
 // x + n*x_bs + t*ldx + c: the stage entry points refuse pointers and strides that would misalign them.
 bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 bool rows16(const void* p, int64_t x_bs, int64_t ldx) { return al16(p) && x_bs % 4 == 0 && ldx % 4 == 0; }
@@ -278,7 +278,7 @@ size_t put_vec(Arena& A, const float* src, int n) {
 }
 
 // One highway layer (modules.py:79-89) as ONE GEMM: W_H, W_T [128][128] -> [128][256] with columns interleaved (H_c, T_c),
-// biases likewise [256] (the epilogues and highway4_kernel read the gate pair of channel c from columns 2c, 2c + 1).
+// biases likewise [256] (highway4_kernel reads the gate pair of channel c from columns 2c, 2c + 1).
 // Returns the offset of the weights.
 size_t put_highway(Arena& A, const float* wh, const float* bh, const float* wt, const float* bt, size_t& b_off) {
   const size_t w_off = A.alloc(128 * 256);
@@ -510,8 +510,9 @@ struct Bump {
 };
 
 size_t cbhg_ws_floats(int K, int P1, int P2, int64_t rows) {
-  // bank + pooled + p1 + p2 + dense + 2 highway + xproj, plus slack for alignment
-  return (size_t)rows * ((size_t)3 * K * 128 + P1 + P2 + 128 + 256 + 768 + 256) + 32768;   // + bf16 hi/lo staging (wide + narrow)
+  // bank + p1 + p2 + dense + xproj, the bf16 hi/lo staging (as wide as the bank, and 256 channels), plus the batch-norm
+  // scratch and slack for alignment
+  return (size_t)rows * ((size_t)2 * K * 128 + P1 + P2 + 128 + 768 + 256) + 32768;
 }
 
 int ensure_ws(taco_handle* h, size_t bytes) {
@@ -556,15 +557,14 @@ BfScratch take_bf(Bump& ws, int64_t rows, int maxCp) {
 // A operand [N][T][Cin] of a GEMM: fp32 x[n*x_bs + t*ldx + c], split into bf ahead of a tensor-core launch; or, presplit,
 // already in bf as the hi / lo operand (written by the producer's epilogue), and x is not read.
 struct GemmIn { const float* x; int64_t x_bs; int ldx; BfScratch bf; bool presplit = false; };
-// Epilogue: act(acc + bias), then the per-channel affine, then the residual; EPI_HIGHWAY reads res as the carry input.
+// Epilogue: act(acc + bias), then the per-channel affine, then the residual.
 // A bank's convolution ci reads bias / scale / shift at ci*Cout.
 struct GemmEpi {
   int act = TACO_ACT_NONE;
   const float* bias = nullptr; const float* scale = nullptr; const float* shift = nullptr;
   const float* res = nullptr; int64_t res_bs = 0; int ldres = 0;
-  int epi = EPI_PLAIN;
 };
-// Results: fp32 out[n*out_bs + t*ldo + col_off + c], not written when out is null; on the tensor cores, optionally also the
+// Results: fp32 out[n*out_bs + t*ldo + col_off + c], not written when out is null; optionally also the
 // hi / lo operand [N][T][copy_cp] of the GEMM that consumes the result, so that no split pass runs in between.
 struct GemmOut {
   float* out; int64_t out_bs; int ldo; int col_off = 0;
@@ -578,31 +578,17 @@ ConvUmma make_umma(const GemmW& g, int N, int T, const BfScratch& a, const GemmE
   u.b_hi = g.b_hi; u.b_lo = g.b_lo; u.b_rows = g.b_rows; u.Kld = g.Kld;
   u.taps = g.taps; u.bank = g.bank; u.Cout = g.Cout; u.nsplit = nsplit;
   u.bias = ep.bias; u.scale = ep.scale; u.shift = ep.shift; u.res = ep.res; u.res_bs = ep.res_bs; u.ldres = ep.ldres;
-  u.out = o.out; u.out_bs = o.out_bs; u.ldo = o.ldo; u.col_off = o.col_off; u.act = ep.act; u.epi = ep.epi;
+  u.out = o.out; u.out_bs = o.out_bs; u.ldo = o.ldo; u.col_off = o.col_off; u.act = ep.act;
   if (o.copy) { u.out_hi = o.copy->hi; u.out_lo = o.copy->lo; u.out_cp = o.copy_cp; }
   return u;
 }
 
-// One conv1d / dense site in the handle's gemm mode: the fp32 FFMA kernel (mode 0, one launch per bank member), or the split
-// pass unless the operand is presplit, then the tensor-core kernel (mode 1: three bf16 products, mode 2: one).  *plan (if
-// given) receives the tensor-core launch's plan.  A failed launch is also recorded as the call's sticky launch error.
+// One conv1d / dense site in the handle's gemm mode: the split pass unless the operand is presplit, then the tensor-core
+// kernel (mode 1: three bf16 products, mode 2: one).  *plan (if given) receives the launch's plan.  A failed launch is also
+// recorded as the call's sticky launch error.
 cudaError_t run_gemm(Ctx& c, const GemmW& g, int N, int T, const GemmIn& in, const GemmEpi& ep, const GemmOut& o,
                      taco_gemm_plan* plan = nullptr) {
   taco_handle* h = c.h;
-  if (h->gemm_mode == 0) {
-    for (int ci = 0; ci < g.bank; ++ci) {
-      const int m = ci * g.Cout;
-      ConvGemm p;
-      p.x = in.x; p.x_bs = in.x_bs; p.ldx = in.ldx; p.N = N; p.T = T; p.Cin = g.Cin; p.k = g.member_taps(ci);
-      p.w = g.member_w(ci); p.ldw = g.ldw;
-      p.bias = ep.bias ? ep.bias + m : nullptr; p.scale = ep.scale ? ep.scale + m : nullptr; p.shift = ep.shift ? ep.shift + m : nullptr;
-      p.res = ep.res; p.res_bs = ep.res_bs; p.ldres = ep.ldres;
-      p.out = o.out; p.out_bs = o.out_bs; p.ldo = o.ldo; p.col_off = o.col_off + m; p.Cout = g.Cout; p.act = ep.act; p.epi = ep.epi;
-      launch_conv_gemm(p, c.st);
-    }
-    h->launches += g.bank;
-    return cudaSuccess;
-  }
   if (!in.presplit) launch_split_bf16(in.x, in.x_bs, in.ldx, N, T, g.Cin, g.Cp, in.bf.hi, in.bf.lo, c.st);
   const cudaError_t e = launch_conv_umma(make_umma(g, N, T, in.bf, ep, o, h->gemm_mode == 2 ? 1 : 3), c.st, plan);
   launch_error(h, e, "conv_umma launch");
@@ -625,44 +611,40 @@ void run_bigru(Ctx& c, const CbhgDev& D, const float* xproj, const int32_t* leng
 }
 
 // reference cbhg() (models/modules.py:35-74).  x: [N,T,Cin] with batch stride x_bs; out [N,T,256] dense.
-// x_split (tensor-core path): x already as the conv bank's hi/lo operand [N][T][g_bank.Cp] (written by the producer's epilogue)
+// x_split: x already as the conv bank's hi/lo operand [N][T][g_bank.Cp] (written by the producer's epilogue)
 void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, const int32_t* lengths, int N,
               int T, int bn_mode, float* out, const BfScratch* x_split = nullptr) {
   const int K = D.K, BC = K * 128, Cin = D.Cin;
   const int64_t rows = (int64_t)N * T;
   float* bank = ws.take<float>(rows * BC);
-  float* pooled = ws.take<float>(rows * BC);
   float* p1 = ws.take<float>(rows * D.P1);
   float* p2 = ws.take<float>(rows * D.P2);
-  float* hwa = ws.take<float>(rows * 128);
-  float* hwb = ws.take<float>(rows * 128);
+  float* dense = ws.take<float>(rows * 128);
   float* xproj = ws.take<float>(rows * 768);
   float* bnv = ws.take<float>(2 * 2048);          // batch-mode scale | shift
   double* bnacc = ws.take<double>(2 * 2048);
-  BfScratch sc, sc2;                 // sc: operands as wide as the bank output; sc2: the narrow ones in between (<= 256 channels)
-  if (c.h->gemm_mode != 0) { sc = take_bf(ws, rows, BC); sc2 = take_bf(ws, rows, 256); }
+  // sc: operands as wide as the bank output; sc2: the narrow ones in between (<= 256 channels)
+  const BfScratch sc = take_bf(ws, rows, BC), sc2 = take_bf(ws, rows, 256);
   if (ws.overflow) return;
   const bool batch = bn_mode == TACO_BN_BATCH;
-  // Producer-side operand split (tensor-core path, moving statistics): a GEMM whose result is only (or also) the A operand of
-  // the next GEMM writes it as bf16 hi/lo from its own epilogue -- proj_1 -> proj_2, proj_2 -> dense -- instead of an fp32 round
-  // trip through split_bf16_kernel.  Batch statistics need the fp32 tensors (moments, in-place affine): the split passes stay.
-  const bool chain = c.h->gemm_mode != 0 && !batch;
+  // Producer-side operand split (moving statistics): a GEMM whose result is only (or also) the A operand of the next GEMM
+  // writes it as bf16 hi/lo from its own epilogue -- proj_1 -> proj_2, proj_2 -> dense -- instead of an fp32 round trip
+  // through split_bf16_kernel.  Batch statistics need the fp32 tensors (moments, in-place affine): the split passes stay.
+  const bool chain = !batch;
   // conv bank: K convolutions written side by side (tf.concat, modules.py:39-42)
   run_gemm(c, D.g_bank, N, T, {x, x_bs, Cin, x_split != nullptr ? *x_split : sc, x_split != nullptr},
            {TACO_ACT_RELU, c.W(D.bank_bias), batch ? nullptr : c.W(D.bank_scale), batch ? nullptr : c.W(D.bank_shift)},
            {bank, (int64_t)T * BC, BC});
-  // max-pool (+ batch-mode BN affine); on the tcgen05 path its output goes straight into the GEMM operand format
-  const bool fuse_split = c.h->gemm_mode != 0 && D.g_p1.Cp == BC;
+  // max-pool (+ batch-mode BN affine), written straight into proj_1's operand format (g_p1.Cp == BC)
   if (batch) {
     launch_bn_batch_stats(bank, (int64_t)T * BC, BC, 0, N, T, BC, c.W(D.bank_gamma), c.W(D.bank_beta), kBnEps,
                           bnacc, bnv, bnv + 2048, c.st);
     c.h->launches += 2;
   }
-  if (fuse_split) launch_affine_maxpool_split(bank, sc.hi, sc.lo, N, T, BC, batch ? bnv : nullptr, batch ? bnv + 2048 : nullptr, c.st);
-  else launch_affine_maxpool(bank, pooled, N, T, BC, batch ? bnv : nullptr, batch ? bnv + 2048 : nullptr, c.st);
+  launch_affine_maxpool_split(bank, sc.hi, sc.lo, N, T, BC, batch ? bnv : nullptr, batch ? bnv + 2048 : nullptr, c.st);
   c.h->launches += 1;
   // proj_1: conv k=3 + ReLU + BN
-  run_gemm(c, D.g_p1, N, T, {pooled, (int64_t)T * BC, BC, sc, fuse_split},
+  run_gemm(c, D.g_p1, N, T, {nullptr, 0, 0, sc, true},
            {TACO_ACT_RELU, c.W(D.p1_b), batch ? nullptr : c.W(D.p1_scale), batch ? nullptr : c.W(D.p1_shift)},
            {chain ? nullptr : p1, (int64_t)T * D.P1, D.P1, 0, chain ? &sc2 : nullptr, D.g_p2.Cp});   // proj_1's output feeds proj_2 only
   if (batch) {
@@ -686,31 +668,17 @@ void run_cbhg(Ctx& c, const CbhgDev& D, Bump& ws, const float* x, int64_t x_bs, 
   const float* hin = p2;
   if (D.P2 != 128) {   // modules.py:59-60
     run_gemm(c, D.g_dense, N, T, {p2, (int64_t)T * D.P2, D.P2, sc, p2_to_dense}, {TACO_ACT_NONE, c.W(D.dense_b)},
-             {hwb, (int64_t)T * 128, 128});
-    hin = hwb;
+             {dense, (int64_t)T * 128, 128});
+    hin = dense;
   }
-  // 4 highway layers (modules.py:63-64): one fused launch on the tensor-core path (the activation stays in registers, the result
-  // comes out as the hi / lo operand of the GRU input projection), four GEMM launches in gemm mode 0
-  const bool hw_fused = c.h->gemm_mode != 0;
-  if (hw_fused) {
-    const float* hb[4] = {c.W(D.hw_b[0]), c.W(D.hw_b[1]), c.W(D.hw_b[2]), c.W(D.hw_b[3])};
-    launch_error(c.h, launch_highway4(hin, nullptr, sc.hi, sc.lo, D.g_hw[0].b_hi, hb, 4, rows, c.h->gemm_mode == 2 ? 1 : 3, c.st),
-                 "highway4 launch");
-    c.h->launches += 1;
-  } else {
-    float* bufs[2] = {hwa, hwb};
-    int cur = 0;   // first output goes to hwa (hin is p2 or hwb)
-    for (int i = 0; i < 4; ++i) {
-      float* o = bufs[cur];
-      run_gemm(c, D.g_hw[i], N, T, {hin, (int64_t)T * 128, 128, sc},
-               {TACO_ACT_NONE, c.W(D.hw_b[i]), nullptr, nullptr, hin, (int64_t)T * 128, 128, EPI_HIGHWAY}, {o, (int64_t)T * 128, 128});
-      hin = o;
-      cur ^= 1;
-    }
-  }
+  // 4 highway layers (modules.py:63-64) in one launch: the activation stays in registers, the result comes out as the hi / lo
+  // operand of the GRU input projection
+  const float* hb[4] = {c.W(D.hw_b[0]), c.W(D.hw_b[1]), c.W(D.hw_b[2]), c.W(D.hw_b[3])};
+  launch_error(c.h, launch_highway4(hin, nullptr, sc.hi, sc.lo, D.g_hw[0].b_hi, hb, 4, rows, c.h->gemm_mode == 2 ? 1 : 3, c.st),
+               "highway4 launch");
+  c.h->launches += 1;
   // hoisted GRU input projection for both directions, then the recurrence
-  run_gemm(c, D.g_xproj, N, T, {hin, (int64_t)T * 128, 128, sc, hw_fused}, {TACO_ACT_NONE, c.W(D.gru_bx)},
-           {xproj, (int64_t)T * 768, 768});
+  run_gemm(c, D.g_xproj, N, T, {nullptr, 0, 0, sc, true}, {TACO_ACT_NONE, c.W(D.gru_bx)}, {xproj, (int64_t)T * 768, 768});
   run_bigru(c, D, xproj, lengths, N, T, out, (int64_t)T * 256);
 }
 
@@ -798,29 +766,26 @@ int do_encoder(taco_handle* h, Bump& ws, const int32_t* ids, const int32_t* leng
   const int E = hp.embedding_text_channels, Es = multi ? hp.embedding_id_channels : 0;
   const int64_t rows = (int64_t)N * T_in;
   float* emb = ws.take<float>(rows * (E + Es));
-  float* a1 = ws.take<float>(rows * 256);
   float* a2 = ws.take<float>(rows * 128);
-  BfScratch sc, sc2;
-  if (h->gemm_mode != 0) { sc = take_bf(ws, rows, 512); sc2 = take_bf(ws, rows, 512); }
+  const BfScratch sc = take_bf(ws, rows, 512), sc2 = take_bf(ws, rows, 512);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (encoder)");
   launch_gather_concat(ids, multi ? spk : nullptr, c.W(h->emb), hp.num_symbols, E, multi ? c.W(h->emb_id) : nullptr,
                        hp.id_num, Es, N, T_in, emb, h->d_ints, st);
   h->launches += 1;
   // encoder prenet (modules.py:5-12; dropout is the identity, SURVEY §0)
   // prenet: dense_1's output feeds dense_2 only, dense_2's feeds the conv bank (as its operand) and proj_2 (as the fp32 residual)
-  const bool chain = h->gemm_mode != 0;
   run_gemm(c, h->g_pre1, N, T_in, {emb, (int64_t)T_in * (E + Es), E + Es, sc}, {TACO_ACT_RELU, c.W(h->pre1_b)},
-           {chain ? nullptr : a1, (int64_t)T_in * 256, 256, 0, chain ? &sc2 : nullptr, h->g_pre2.Cp});
-  run_gemm(c, h->g_pre2, N, T_in, {a1, (int64_t)T_in * 256, 256, chain ? sc2 : sc, chain}, {TACO_ACT_RELU, c.W(h->pre2_b)},
-           {a2, (int64_t)T_in * 128, 128, 0, chain ? &sc : nullptr, h->enc.g_bank.Cp});
-  run_cbhg(c, h->enc, ws, a2, (int64_t)T_in * 128, lengths, N, T_in, bn_mode, memory_out, chain ? &sc : nullptr);
+           {nullptr, (int64_t)T_in * 256, 256, 0, &sc2, h->g_pre2.Cp});
+  run_gemm(c, h->g_pre2, N, T_in, {nullptr, 0, 0, sc2, true}, {TACO_ACT_RELU, c.W(h->pre2_b)},
+           {a2, (int64_t)T_in * 128, 128, 0, &sc, h->enc.g_bank.Cp});
+  run_cbhg(c, h->enc, ws, a2, (int64_t)T_in * 128, lengths, N, T_in, bn_mode, memory_out, &sc);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (encoder cbhg)");
   return check_launch(h, "encoder");
 }
 
 size_t encoder_ws_bytes(const taco_handle* h, int N, int T_in) {
   const int64_t rows = (int64_t)N * T_in;
-  return sizeof(float) * ((size_t)rows * (h->emb_dim + 256 + 128 + 512 + 512) + cbhg_ws_floats(16, 128, 128, rows)) + 65536;
+  return sizeof(float) * ((size_t)rows * (h->emb_dim + 128 + 512 + 512) + cbhg_ws_floats(16, 128, 128, rows)) + 65536;
 }
 size_t postnet_ws_bytes(const taco_handle* h, int N, int T) {
   const int64_t rows = (int64_t)N * T;
@@ -850,8 +815,7 @@ int do_decode(taco_handle* h, Bump& ws, const float* memory, int N, int T_in, co
   const int max_steps = taco_max_steps(h, teacher_force, T_tgt);
   if (max_steps <= 0) return fail(h, TACO_ERR_INVALID, "no decoder steps (T_tgt < r?)");
   float* keys = ws.take<float>((size_t)N * T_in * 256);
-  BfScratch sc;
-  if (h->gemm_mode != 0) sc = take_bf(ws, (int64_t)N * T_in, 256);
+  const BfScratch sc = take_bf(ws, (int64_t)N * T_in, 256);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (decoder)");
   // BahdanauAttention memory_layer (no bias), once per utterance (tacotron.py:68)
   run_gemm(c, h->g_mem, N, T_in, {memory, (int64_t)T_in * 256, 256, sc}, {TACO_ACT_NONE}, {keys, (int64_t)T_in * 256, 256});
@@ -912,8 +876,7 @@ int do_postnet(taco_handle* h, Bump& ws, const float* mel, int N, int T, int bn_
   Ctx c{h, st};
   const taco_hparams& hp = h->hp;
   float* post = ws.take<float>((size_t)N * T * 256);
-  BfScratch sc;
-  if (h->gemm_mode != 0) sc = take_bf(ws, (int64_t)N * T, 256);
+  const BfScratch sc = take_bf(ws, (int64_t)N * T, 256);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (postnet)");
   run_cbhg(c, h->post, ws, mel, mel_bs, nullptr, N, T, bn_mode, post);
   if (ws.overflow) return fail(h, TACO_ERR_INVALID, "workspace overflow (postnet cbhg)");
@@ -930,7 +893,7 @@ GemmW unit_gemmw(const taco_gemm_desc& d) {
 }
 // Its epilogue and outputs, with the parameters at the given device pointers
 GemmEpi unit_epi(const taco_gemm_desc& d, const float* bias, const float* scale, const float* shift) {
-  return {d.act, bias, scale, shift, d.res, d.res_bs, d.ldres, d.epi};
+  return {d.act, bias, scale, shift, d.res, d.res_bs, d.ldres};
 }
 GemmOut unit_out(const taco_gemm_desc& d, const BfScratch& copy) { return {d.out, d.out_bs, d.ldo, d.col_off, &copy, d.out_cp}; }
 
@@ -1114,7 +1077,7 @@ int taco_finalize_weights(taco_handle* h) {
     }
     CUDA_OK(h, cudaDeviceSynchronize());
     const char* gm = getenv("TACO_GEMM");
-    if (gm) h->gemm_mode = !strcmp(gm, "ffma") ? 0 : (!strcmp(gm, "bf16") ? 2 : 1);
+    if (gm) h->gemm_mode = !strcmp(gm, "bf16") ? 2 : 1;
   }
   const float* B = h->dW;
   {
@@ -1242,8 +1205,7 @@ int taco_bigru(taco_handle* h, int which, const float* x, const int32_t* lengths
   Bump ws(h->ws, h->ws_bytes);
   Ctx c{h, (cudaStream_t)stream};
   float* xproj = ws.take<float>((size_t)N * T * 768);
-  BfScratch sc;
-  if (h->gemm_mode != 0) sc = take_bf(ws, (int64_t)N * T, 128);
+  const BfScratch sc = take_bf(ws, (int64_t)N * T, 128);
   run_gemm(c, D.g_xproj, N, T, {x, (int64_t)T * 128, 128, sc}, {TACO_ACT_NONE, c.W(D.gru_bx)}, {xproj, (int64_t)T * 768, 768});
   run_bigru(c, D, xproj, lengths, N, T, out, (int64_t)T * 256);
   return check_launch(h, "bigru");
@@ -1258,32 +1220,18 @@ int taco_conv1d(taco_handle* h, const float* x, int N, int T, int Cin, const flo
   if (!al16(x) || !al16(kernel)) return fail(h, TACO_ERR_INVALID, "x and kernel must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   Ctx c{h, st};
-  GemmIn in{x, (int64_t)T * Cin, Cin, {}};
-  GemmW g;
-  if (h->gemm_mode != 0) {   // tensor-core path: pack W^T hi/lo and split x on the device, then one UMMA launch
-    g = make_gemmw(0, Cout, k, Cin, Cout);
-    const size_t nb = (size_t)g.b_rows * g.Kld, na = (size_t)N * T * g.Cp;
-    int rc = ensure_ws(h, sizeof(uint16_t) * 2 * (nb + na) + 65536);
-    if (rc) return rc;
-    Bump ws(h->ws, h->ws_bytes);
-    g.w = kernel;
-    g.b_hi = ws.take<uint16_t>(nb);
-    g.b_lo = ws.take<uint16_t>(nb);
-    in.bf = take_bf(ws, (int64_t)N * T, g.Cp);
-    pack_gemmw(g, st);
-    h->launches += 1;
-  } else {
-    g = make_gemmw(0, (Cout + 3) & ~3, k, Cin, Cout);
-    g.w = kernel;
-    if (g.ldw != Cout) {   // pad the leading dimension for 128-bit weight loads
-      int rc = ensure_ws(h, sizeof(float) * (size_t)k * Cin * g.ldw + 65536);
-      if (rc) return rc;
-      CUDA_OK(h, cudaMemsetAsync(h->ws, 0, sizeof(float) * (size_t)k * Cin * g.ldw, st));
-      CUDA_OK(h, cudaMemcpy2DAsync(h->ws, sizeof(float) * g.ldw, kernel, sizeof(float) * Cout, sizeof(float) * Cout,
-                                   (size_t)k * Cin, cudaMemcpyDeviceToDevice, st));
-      g.w = reinterpret_cast<const float*>(h->ws);
-    }
-  }
+  // pack W^T hi/lo and split x on the device, then one tensor-core launch
+  GemmW g = make_gemmw(0, Cout, k, Cin, Cout);
+  const size_t nb = (size_t)g.b_rows * g.Kld, na = (size_t)N * T * g.Cp;
+  int rc = ensure_ws(h, sizeof(uint16_t) * 2 * (nb + na) + 65536);
+  if (rc) return rc;
+  Bump ws(h->ws, h->ws_bytes);
+  g.w = kernel;
+  g.b_hi = ws.take<uint16_t>(nb);
+  g.b_lo = ws.take<uint16_t>(nb);
+  const GemmIn in{x, (int64_t)T * Cin, Cin, take_bf(ws, (int64_t)N * T, g.Cp)};
+  pack_gemmw(g, st);
+  h->launches += 1;
   run_gemm(c, g, N, T, in, {act, bias}, {out, (int64_t)T * Cout, Cout});
   return check_launch(h, "conv1d");
 }
@@ -1331,27 +1279,20 @@ int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan
   CUDA_OK(h, cudaSetDevice(h->device));
   if (plan) memset(plan, 0, sizeof(*plan));
   if (!d || d->N <= 0 || d->T <= 0 || d->Cin <= 0 || d->Cout <= 0 || d->bank < 1 || (d->bank == 1 && d->taps < 1) || !d->w_host ||
-      (d->epi != TACO_EPI_PLAIN && d->epi != TACO_EPI_HIGHWAY) || ((d->scale_host == nullptr) != (d->shift_host == nullptr)))
+      ((d->scale_host == nullptr) != (d->shift_host == nullptr)))
     return fail(h, TACO_ERR_INVALID, "bad argument");
-  const bool hw = d->epi == TACO_EPI_HIGHWAY, bank = d->bank > 1, presplit = d->x_hi != nullptr;
-  if (hw && (d->Cin != 128 || d->Cout != 256 || bank || d->taps != 1 || !d->w2_host || !d->bias_host || !d->bias2_host || !d->res ||
-             d->scale_host))
-    return fail(h, TACO_ERR_INVALID, "highway: 128 -> 256 interleaved (H, T) columns, one tap, W_T, b_H, b_T and the carry input");
+  const bool bank = d->bank > 1, presplit = d->x_hi != nullptr;
   if (presplit ? d->x_lo == nullptr : (d->x == nullptr || !rows16(d->x, d->x_bs, d->ldx)))
     return fail(h, TACO_ERR_INVALID, "x: 16-byte aligned rows with strides that are multiples of 4 floats, or both halves of a split operand");
-  const int gm = h->gemm_mode;
-  if (gm == 0 && (presplit || d->out_hi != nullptr || d->out == nullptr))
-    return fail(h, TACO_ERR_INVALID, "gemm mode 0 (FFMA) reads and writes fp32 only");
   const int nparam = bank ? d->bank * d->Cout : d->Cout;
   GemmW g = unit_gemmw(*d);
   // parameters: staged on the host as taco_finalize_weights stages them, then one copy to the device
   Arena A;
   size_t b_off = 0, sc_off = 0, sh_off = 0;
-  if (hw) g.off = put_highway(A, d->w_host, d->bias_host, d->w2_host, d->bias2_host, b_off);
-  else g.off = put_matrix(A, d->w_host, (bank ? d->bank * (d->bank + 1) / 2 : d->taps) * d->Cin, d->Cout, g.ldw);
-  if (!hw && d->bias_host) b_off = put_vec(A, d->bias_host, nparam);
+  g.off = put_matrix(A, d->w_host, (bank ? d->bank * (d->bank + 1) / 2 : d->taps) * d->Cin, d->Cout, g.ldw);
+  if (d->bias_host) b_off = put_vec(A, d->bias_host, nparam);
   if (d->scale_host) { sc_off = put_vec(A, d->scale_host, nparam); sh_off = put_vec(A, d->shift_host, nparam); }
-  const size_t nbt = gm ? (size_t)2 * g.b_rows * g.Kld : 0, na = gm && !presplit ? (size_t)2 * d->N * d->T * g.Cp : 0;
+  const size_t nbt = (size_t)2 * g.b_rows * g.Kld, na = presplit ? 0 : (size_t)2 * d->N * d->T * g.Cp;
   int rc = ensure_ws(h, sizeof(float) * A.buf.size() + sizeof(uint16_t) * (nbt + na) + 65536);
   if (rc) return rc;
   Bump ws(h->ws, h->ws_bytes);
@@ -1366,10 +1307,8 @@ int taco_gemm_unit(taco_handle* h, const taco_gemm_desc* d, taco_gemm_plan* plan
   const float* scale = d->scale_host ? dP + sc_off : nullptr;
   const float* shift = d->scale_host ? dP + sh_off : nullptr;
   g.place(dP, bt);
-  if (gm) {
-    pack_gemmw(g, st);
-    h->launches += g.bank;
-  }
+  pack_gemmw(g, st);
+  h->launches += g.bank;
   if (presplit) sc = {const_cast<void*>(d->x_hi), const_cast<void*>(d->x_lo)};
   const BfScratch copy{d->out_hi, d->out_lo};
   Ctx c{h, st};
@@ -1389,7 +1328,6 @@ int taco_highway4_unit(taco_handle* h, const float* x, int64_t rows, int layers,
       (out == nullptr && out_hi == nullptr) || ((out_hi == nullptr) != (out_lo == nullptr)))
     return fail(h, TACO_ERR_INVALID, "bad argument");
   if (!al16(x) || !al16(out) || !al16(out_hi) || !al16(out_lo)) return fail(h, TACO_ERR_INVALID, "x and the outputs must be 16-byte aligned");
-  if (h->gemm_mode == 0) return fail(h, TACO_ERR_UNSUPPORTED, "the fused highway kernel runs on the tensor cores only (gemm mode 1 or 2)");
   Arena A;
   size_t w_off[4], b_off[4];
   for (int l = 0; l < layers; ++l)
@@ -2106,7 +2044,8 @@ int taco_decoder_geometry(const taco_handle* h, int N, int* cluster_size, int* s
 }
 
 int taco_set_gemm_mode(taco_handle* h, int mode) {
-  if (!h || mode < 0 || mode > 2) return TACO_ERR_INVALID;
+  if (!h) return TACO_ERR_INVALID;
+  if (mode != 1 && mode != 2) return fail(h, TACO_ERR_INVALID, "gemm mode must be 1 (bf16x3) or 2 (bf16)");
   h->gemm_mode = mode;
   return TACO_OK;
 }

@@ -125,7 +125,7 @@ class Engine:
         return int(self.lib.taco_launch_count(self._h))
 
     def set_gemm_mode(self, mode: int):
-        """0 = fp32 FFMA, 1 = bf16x3 tcgen05 (default, fp32-class), 2 = plain bf16 tcgen05."""
+        """1 = bf16x3 tcgen05 (default, fp32-class), 2 = plain bf16 tcgen05; any other mode raises TacoError."""
         self._ck(self.lib.taco_set_gemm_mode(self._h, int(mode)))
 
     def set_decoder_clusters(self, n: int):
@@ -234,9 +234,9 @@ class Engine:
         self._ck(self.lib.taco_bn_batch_stats(self._h, _ptr(x), N, T, Cc, _ptr(gamma), _ptr(beta), _ptr(scale), _ptr(shift), self.stream))
         return scale, shift
 
-    def gemm_unit(self, N, T, Cin, Cout, w, *, x=None, x_bs=None, ldx=None, x_split=None, taps=1, bank=1, w2=None,
-                  bias=None, bias2=None, scale=None, shift=None, res=None, res_bs=None, ldres=None, act=_abi.ACT_NONE,
-                  epi=_abi.EPI_PLAIN, out=None, out_bs=None, ldo=None, col_off=0, out_split=None, out_cp=0):
+    def gemm_unit(self, N, T, Cin, Cout, w, *, x=None, x_bs=None, ldx=None, x_split=None, taps=1, bank=1, bias=None,
+                  scale=None, shift=None, res=None, res_bs=None, ldres=None, act=_abi.ACT_NONE, out=None, out_bs=None,
+                  ldo=None, col_off=0, out_split=None, out_cp=0):
         """``taco_gemm_unit`` in the current gemm mode.  ``x`` / ``res`` / ``out`` are device tensors addressed through the
         given strides (defaults: dense [N, T, C]); ``x_split`` / ``out_split`` are (hi, lo) bf16 operand tensors.  Weights
         and per-channel parameters are host arrays in the reference layouts.  Returns the plan the launch used (a dict)."""
@@ -256,12 +256,11 @@ class Engine:
         d.x, d.x_bs, d.ldx = dev(x), T * Cin if x_bs is None else x_bs, Cin if ldx is None else ldx
         d.x_hi, d.x_lo = (dev(x_split[0]), dev(x_split[1])) if x_split is not None else (None, None)
         d.N, d.T, d.Cin, d.taps, d.bank, d.Cout = N, T, Cin, taps, bank, Cout
-        d.w_host, d.w2_host, d.bias_host, d.bias2_host = host(w), host(w2), host(bias), host(bias2)
+        d.w_host, d.bias_host = host(w), host(bias)
         d.scale_host, d.shift_host = host(scale), host(shift)
-        ch = Cout // 2 if epi == _abi.EPI_HIGHWAY else Cout
-        d.res, d.res_bs, d.ldres = dev(res), T * ch if res_bs is None else res_bs, ch if ldres is None else ldres
-        d.act, d.epi = act, epi
-        width = ch * max(bank, 1)
+        d.res, d.res_bs, d.ldres = dev(res), T * Cout if res_bs is None else res_bs, Cout if ldres is None else ldres
+        d.act = act
+        width = Cout * max(bank, 1)
         d.out, d.out_bs, d.ldo, d.col_off = dev(out), T * width if out_bs is None else out_bs, width if ldo is None else ldo, col_off
         d.out_hi, d.out_lo = (dev(out_split[0]), dev(out_split[1])) if out_split is not None else (None, None)
         d.out_cp = out_cp

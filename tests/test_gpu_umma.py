@@ -15,7 +15,6 @@ on the arithmetic:
   A mode-2 run (one product per k-step) of every case must FAIL this bound (asserted): its smallest ratio on the table is
   2.2e-4, and a kernel without the hi*lo product measured 5.5e-4.
 * ``C_BF16`` for plain bf16 (mode 2): 2^-7, the worst case of one bf16 product per term (2 x 2^-9) with margin.
-* Mode 0 (fp32 FFMA kernels) runs the same table against ``C_X3``: it is the reference-precision path (measured <= 3.3e-7).
 
 Outputs are written into NaN-filled buffers wider than the written window (column offset, row pitch, batch stride and one
 extra utterance): everything outside the window must still hold the NaN pattern bit for bit.
@@ -44,15 +43,14 @@ ONE, SHORT, LONG = "one tile per CTA", "persistent short K", "persistent long K"
 
 
 class Case:
-    def __init__(self, name, N, T, Cin, Cout, taps=1, bank=1, act=0, affine=False, res=False, epi=0, layout="vec",
-                 plan=None):
+    def __init__(self, name, N, T, Cin, Cout, taps=1, bank=1, act=0, affine=False, res=False, layout="vec", plan=None):
         self.name, self.N, self.T, self.Cin, self.Cout, self.taps, self.bank = name, N, T, Cin, Cout, taps, bank
-        self.act, self.affine, self.res, self.epi, self.layout = act, affine, res, epi, layout
+        self.act, self.affine, self.res, self.layout = act, affine, res, layout
         self.plan = plan          # (kind, acc_cols, vec_epi, variant)
 
     @property
     def width(self):              # output channels written per row
-        return (self.Cout // 2 if self.epi == 1 else self.Cout) * self.bank
+        return self.Cout * self.bank
 
     def geometry(self):
         """Strides of x, res and out: wider than the data, 16-byte multiples in the vector layout, odd in the scalar one."""
@@ -60,11 +58,8 @@ class Case:
         g = {}
         g["ldx"] = self.Cin + 4
         g["x_bs"] = self.T * g["ldx"] + 4
-        if self.epi == 1:          # the carry input of a highway layer is its GEMM input
-            g["ldres"], g["res_bs"] = g["ldx"], g["x_bs"]
-        else:
-            g["ldres"] = self.width + (4 if v else 3)
-            g["res_bs"] = self.T * g["ldres"] + (4 if v else 1)
+        g["ldres"] = self.width + (4 if v else 3)
+        g["res_bs"] = self.T * g["ldres"] + (4 if v else 1)
         g["col_off"] = 4 if v else 3
         g["ldo"] = g["col_off"] + self.width + (4 if v else 2)
         g["out_bs"] = self.T * g["ldo"] + (8 if v else 5)
@@ -89,13 +84,10 @@ CASES = [
     Case("bank16_enc_n32", 32, 100, 128, 128, bank=16, act=1, affine=True, plan=(LONG, 256, 1, 3)),
     Case("bank8_post_n2", 2, 129, 80, 128, bank=8, act=1, plan=(ONE, 128, 1, 2)),
     Case("bank8_post_scalar_n3", 3, 255, 80, 128, bank=8, act=1, affine=True, layout="scalar", plan=(ONE, 128, 0, 3)),
-    Case("highway_t127", 1, 127, 128, 256, epi=1, res=True, plan=(ONE, 128, 1, 5)),
-    Case("highway_t129_scalar", 3, 129, 128, 256, epi=1, res=True, layout="scalar", plan=(ONE, 128, 0, 5)),
     # the config-3 shapes (batch 32, 1000 frames)
     Case("cfg3_final_dense_1025", 32, 1000, 256, 1025, layout="scalar", plan=(SHORT, 256, 0, 1)),
     Case("cfg3_post_proj1_3x1024_256", 32, 1000, 1024, 256, taps=3, act=1, affine=True, plan=(LONG, 256, 1, 3)),
     Case("cfg3_post_bank_8x128", 32, 1000, 80, 128, bank=8, act=1, affine=True, plan=(SHORT, 256, 1, 3)),
-    Case("cfg3_highway_256", 32, 1000, 128, 256, epi=1, res=True, plan=(SHORT, 256, 1, 5)),
 ]
 CASE_IDS = [c.name for c in CASES]
 
@@ -109,13 +101,11 @@ def plan_desc(c: Case, g=None):
     d.x, d.x_bs, d.ldx = FAKE, g["x_bs"], g["ldx"]
     d.w_host = FAKE
     d.bias_host = FAKE
-    if c.epi == 1:
-        d.w2_host = d.bias2_host = FAKE
     if c.affine:
         d.scale_host = d.shift_host = FAKE
     if c.res:
         d.res, d.res_bs, d.ldres = FAKE, g["res_bs"], g["ldres"]
-    d.act, d.epi = c.act, c.epi
+    d.act = c.act
     d.out, d.out_bs, d.ldo, d.col_off = FAKE, g["out_bs"], g["ldo"], g["col_off"]
     return d
 
@@ -156,8 +146,8 @@ def test_case_table_covers_every_plan_branch(lib):
     shapes = {(kind_of(p), p["acc_cols"]) for p in plans}
     # a short-K persistent launch has more than 2 x 148 tiles, hence always two accumulators
     assert shapes == {(ONE, 128), (SHORT, 256), (LONG, 128), (LONG, 256)}, shapes
-    assert {p["variant"] for p in plans} == set(range(6))
-    assert {(c.epi, p["vec_epi"]) for c, p in zip(CASES, plans)} == {(0, 0), (0, 1), (1, 0), (1, 1)}
+    assert {p["variant"] for p in plans} == set(range(5))
+    assert {p["vec_epi"] for p in plans} == {0, 1}
     assert {c.bank for c in CASES} == {1, 8, 16}
     assert {16, 8} <= {c.taps for c in CASES} and {1, 2, 3, 4, 5, 7} <= {c.taps for c in CASES}
     assert {4, 36, 80, 128, 1024, 2048} <= {c.Cin for c in CASES}
@@ -215,7 +205,7 @@ def test_plan_refusals(lib):
     c = Case("", 2, 50, 128, 80, act=1)
     ok = plan_desc(c)
     assert _abi.umma_plan(ok)["valid"] == 1
-    for field, value in (("N", 0), ("Cin", 0), ("out", None), ("epi", 1)):   # highway without its carry input
+    for field, value in (("N", 0), ("Cin", 0), ("out", None)):
         d = plan_desc(c)
         setattr(d, field, value)
         assert _abi.umma_plan(d)["valid"] == 0, field
@@ -277,18 +267,12 @@ class Inputs:
         N, T, Cin, Cout = c.N, c.T, c.Cin, c.Cout
         self.x = rng.standard_normal((N, T, Cin)).astype(np.float32)
         nparam = Cout * c.bank
-        if c.epi == 1:
-            self.wh = (rng.standard_normal((Cin, Cout // 2)) / np.sqrt(Cin)).astype(np.float32)
-            self.wt = (rng.standard_normal((Cin, Cout // 2)) / np.sqrt(Cin)).astype(np.float32)
-            self.bh = (0.5 * rng.standard_normal(Cout // 2)).astype(np.float32)
-            self.bt = (0.5 * rng.standard_normal(Cout // 2)).astype(np.float32)
-        else:
-            taps = [ci + 1 for ci in range(c.bank)] if c.bank > 1 else [c.taps]
-            self.ws = [(rng.standard_normal((k, Cin, Cout)) / np.sqrt(k * Cin)).astype(np.float32) for k in taps]
-            self.b = (0.5 * rng.standard_normal(nparam)).astype(np.float32)
-            self.scale = rng.uniform(-2, 2, nparam).astype(np.float32) if c.affine else None
-            self.shift = rng.standard_normal(nparam).astype(np.float32) if c.affine else None
-            self.r = rng.standard_normal((N, T, c.width)).astype(np.float32) if c.res else None
+        taps = [ci + 1 for ci in range(c.bank)] if c.bank > 1 else [c.taps]
+        self.ws = [(rng.standard_normal((k, Cin, Cout)) / np.sqrt(k * Cin)).astype(np.float32) for k in taps]
+        self.b = (0.5 * rng.standard_normal(nparam)).astype(np.float32)
+        self.scale = rng.uniform(-2, 2, nparam).astype(np.float32) if c.affine else None
+        self.shift = rng.standard_normal(nparam).astype(np.float32) if c.affine else None
+        self.r = rng.standard_normal((N, T, c.width)).astype(np.float32) if c.res else None
         self._ref = None
 
     def device(self):
@@ -296,9 +280,7 @@ class Inputs:
         xb = _filled32(c.N * g["x_bs"] + 16)
         _gather(xb, c.N, c.T, c.Cin, 0, g["ldx"], g["x_bs"]).copy_(torch.from_numpy(self.x))
         rb = None
-        if c.epi == 1:
-            rb = xb
-        elif c.res:
+        if c.res:
             rb = _filled32(c.N * g["res_bs"] + 16)
             _gather(rb, c.N, c.T, c.width, 0, g["ldres"], g["res_bs"]).copy_(torch.from_numpy(self.r))
         return xb, rb
@@ -310,35 +292,25 @@ class Inputs:
         c = self.c
         x = torch.from_numpy(self.x).double()
         ax = x.abs()
-        if c.epi == 1:
-            zero = torch.zeros(c.Cout // 2, dtype=torch.float64)
-            wh, wt = torch.from_numpy(self.wh).double(), torch.from_numpy(self.wt).double()
-            H = torch.relu(x @ wh + torch.from_numpy(self.bh).double())
-            Tg = torch.sigmoid(x @ wt + torch.from_numpy(self.bt).double())
-            ref = H * Tg + x * (1 - Tg)
-            S = (ax @ wh.abs()) + 0.25 * (ax @ wt.abs()) * (H - x).abs()
-            rnd = ref.abs() + x.abs()
-        else:
-            outs, Ss = [], []
-            for w in self.ws:
-                w = torch.from_numpy(w).double()
-                zero = torch.zeros(w.shape[2], dtype=torch.float64)
-                outs.append(O.conv1d_same(x, w, zero))
-                Ss.append(O.conv1d_same(ax, w.abs(), zero))
-            y = torch.cat(outs, -1) + torch.from_numpy(self.b).double()
-            S = torch.cat(Ss, -1)
-            y = [lambda v: v, torch.relu, torch.sigmoid, torch.tanh][c.act](y)
+        outs, Ss = [], []
+        for w in self.ws:
+            w = torch.from_numpy(w).double()
+            zero = torch.zeros(w.shape[2], dtype=torch.float64)
+            outs.append(O.conv1d_same(x, w, zero))
+            Ss.append(O.conv1d_same(ax, w.abs(), zero))
+        y = torch.cat(outs, -1) + torch.from_numpy(self.b).double()
+        S = torch.cat(Ss, -1)
+        y = [lambda v: v, torch.relu, torch.sigmoid, torch.tanh][c.act](y)
+        rnd = y.abs()
+        if c.affine:
+            sc = torch.from_numpy(self.scale).double()
+            y = y * sc + torch.from_numpy(self.shift).double()
+            S = S * sc.abs().clamp(min=1.0)
             rnd = y.abs()
-            if c.affine:
-                sc = torch.from_numpy(self.scale).double()
-                y = y * sc + torch.from_numpy(self.shift).double()
-                S = S * sc.abs().clamp(min=1.0)
-                rnd = y.abs()
-            if c.res:
-                y = y + torch.from_numpy(self.r).double()
-                rnd = rnd + y.abs()
-            ref = y
-        self._ref = (ref, S, rnd)
+        if c.res:
+            y = y + torch.from_numpy(self.r).double()
+            rnd = rnd + y.abs()
+        self._ref = (y, S, rnd)
         return self._ref
 
     def run(self, eng, out_split=None, write_out=True):
@@ -347,16 +319,11 @@ class Inputs:
         xb, rb = self.device()
         total = (c.N + 1) * g["out_bs"]
         ob = _filled32(total) if write_out else None
-        kw = dict(x=xb, x_bs=g["x_bs"], ldx=g["ldx"], taps=c.taps, bank=c.bank, act=c.act, epi=c.epi,
-                  out=ob, out_bs=g["out_bs"], ldo=g["ldo"], col_off=g["col_off"])
-        if c.epi == 1:
-            kw.update(w2=self.wt, bias=self.bh, bias2=self.bt, res=rb, res_bs=g["res_bs"], ldres=g["ldres"])
-            w = self.wh
-        else:
-            w = np.concatenate([a.reshape(-1) for a in self.ws])
-            kw.update(bias=self.b, scale=self.scale, shift=self.shift)
-            if c.res:
-                kw.update(res=rb, res_bs=g["res_bs"], ldres=g["ldres"])
+        kw = dict(x=xb, x_bs=g["x_bs"], ldx=g["ldx"], taps=c.taps, bank=c.bank, act=c.act, bias=self.b, scale=self.scale,
+                  shift=self.shift, out=ob, out_bs=g["out_bs"], ldo=g["ldo"], col_off=g["col_off"])
+        if c.res:
+            kw.update(res=rb, res_bs=g["res_bs"], ldres=g["ldres"])
+        w = np.concatenate([a.reshape(-1) for a in self.ws])
         if out_split is not None:
             kw.update(out_split=out_split[:2], out_cp=out_split[2], col_off=0, ldo=c.width, out_bs=c.T * c.width)
         plan = eng.gemm_unit(c.N, c.T, c.Cin, c.Cout, w, **kw)
@@ -386,12 +353,12 @@ def ratio(win, ref, S, rnd):
 @pytest.mark.parametrize("c", CASES, ids=CASE_IDS)
 def test_gemm_against_fp64(eng, c):
     """Mode 1 within C_X3 of the fp64 reference, with the planned launch shape and nothing written outside the window; the
-    same case in mode 2 must violate that bound (and meet C_BF16); mode 0 (fp32 FFMA kernels) meets C_X3."""
+    same case in mode 2 must violate that bound (and meet C_BF16)."""
     I = Inputs(c)
     ref, S, rnd = I.reference()
     ratios = {}
     try:
-        for mode in (1, 2, 0):
+        for mode in (1, 2):
             eng.set_gemm_mode(mode)
             plan, ob, _ = I.run(eng)
             if mode == 1:
@@ -402,11 +369,10 @@ def test_gemm_against_fp64(eng, c):
             del ob, win
     finally:
         eng.set_gemm_mode(1)
-    print("%s: worst |d| / S  mode 1 %.3e  mode 2 %.3e  mode 0 %.3e" % (c.name, ratios[1], ratios[2], ratios[0]))
+    print("%s: worst |d| / S  mode 1 %.3e  mode 2 %.3e" % (c.name, ratios[1], ratios[2]))
     assert ratios[1] <= C_X3, ratios
     assert ratios[2] > C_X3, "a one-product run passes the bf16x3 bound: the bound cannot see a dropped correction product"
     assert ratios[2] <= C_BF16, ratios
-    assert ratios[0] <= C_X3, ratios
 
 
 def _bf16_split(v):
@@ -506,7 +472,6 @@ HW4_CASES = [
                                                                   for r, l, m, o in HW4_CASES])
 def test_highway4_against_fp64(eng, rows, layers, mode, outs):
     """The fused layers against the fp64 chain (bound C_HW4 in mode 1, C_HW4_BF16 in mode 2, and mode 2 must violate C_HW4),
-    against `layers` EPI_HIGHWAY GEMMs of the same weights (within the sum of both bounds: the gate is rounded differently),
     and the bf16 copy against bf16_rne(out) / bf16_rne(out - hi).  18944 = 148 x 128 rows: one tile per CTA; 18945 and
     32000 rows make CTAs walk two tiles.  Nothing is written past `rows`."""
     want_out, want_copy = outs
@@ -521,14 +486,6 @@ def test_highway4_against_fp64(eng, rows, layers, mode, outs):
     try:
         eng.highway4_unit(xd, wh, bh, wt, bt, out=out, out_split=(hi, lo) if want_copy else None)
         torch.cuda.synchronize()
-        if want_out:
-            # the same layers as EPI_HIGHWAY GEMMs (the unfused path of the forward)
-            cur = xd
-            for l in range(layers):
-                nxt = torch.empty(rows, 128, device="cuda")
-                eng.gemm_unit(1, rows, 128, 256, wh[l], x=cur, w2=wt[l], bias=bh[l], bias2=bt[l], res=cur, epi=1, out=nxt)
-                cur = nxt
-            torch.cuda.synchronize()
     finally:
         eng.set_gemm_mode(1)
     c_mode = C_HW4 if mode == 1 else C_HW4_BF16
@@ -544,8 +501,6 @@ def test_highway4_against_fp64(eng, rows, layers, mode, outs):
         assert bool((d <= tol).all()), r
         if mode == 2:
             assert r > C_HW4, "a one-product run passes the bf16x3 bound"
-        unf = cur.cpu()
-        assert bool(((got.double() - unf.double()).abs() <= 2 * tol).all())
     if want_copy:
         hic, loc = hi.view(torch.int16).cpu(), lo.view(torch.int16).cpu()
         assert bool((hic[rows * 128:] == NAN16).all()) and bool((loc[rows * 128:] == NAN16).all())
